@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the SSD3D hot path: volumes/sec for forward + decode + NMS (= ``LSSD3D.predict_step``).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): SSD3D-MobileNet inference on synthetic 2-channel 128^3 cube-lesion
 volumes (generate_artificial_dataset.py distribution), batch 8 per GPU, bf16 activations, random-init
@@ -10,8 +10,11 @@ runs the same per-GPU batch (independent volumes, no data-path collective): weak
 
 The single JSON line printed by rank 0 carries
   value        whole-job volumes/s with the input batches already resident in HBM (device-timed, max over ranks).
-               The K steps are repeated R times inside ONE event pair so that the timed region is >= 50 ms
-               (``repeats``, ``timed_region_ms``); ms_per_step = region / (K*R)
+               Exactly K steps inside ONE event pair, taken from the middle of one pipelined pass: W warm-up
+               batches fill the pipeline before it, the batches still in flight after it drain outside it
+               (``timed_steps``, ``timed_region_ms``); ms_per_step = region / K.  Nothing stretches the region:
+               at about 0.18 ms per step (B200, 1000 W power limit) a small K gives a window of a few ms and
+               a number that carries clock and scheduler noise; K of a few hundred (>= 50 ms) gives a stable one
   e2e          the same through the public streaming API (LSSD3D.predict_batches, the analogue of the
                reference's Trainer.predict loop) from PINNED HOST buffers: H2D of every batch and D2H of its
                detections inside the timed region.  Headline: bf16 host batches (the stem rounds fp32 inputs
@@ -27,6 +30,11 @@ The single JSON line printed by rank 0 carries
 ``--impl reference`` times the UNMODIFIED reference (``oracle/_ref``, staged by ``oracle/make_ref.py``;
 ``kind: "reference"``) -- LSSD3D.forward + detect_objects on the host CPU, best thread count of a sweep --
 or, where the staged files are missing, the oracle port (``kind: "port"``); rank 0 only.
+
+``--dump-outputs DIR`` writes what the last timed step handed back (rank 0's detections for its batch of 8
+volumes, concatenated in volume order) as float32 ``.npy`` files: ``boxes`` (n, 6), ``labels`` (n,), ``scores``
+(n,) and ``counts`` (8,), the number of detections per volume.  Inputs and weights are seeded, so two builds
+run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -308,14 +316,12 @@ def train_leg(dev, rank, world, steps, warmup, barrier, max_over_ranks):
         barrier()
         return max_over_ranks(e0.elapsed_time(e1), dev), host_ms, last
 
-    probe, _, _ = region(max(steps // 4, 3))
-    reps = max(1, int(math.ceil(MIN_REGION_MS / max(probe * steps / max(steps // 4, 3), 1e-3))))
     ops.LAUNCHES[0] = 0
-    ms, host_ms, last = region(steps * reps)
-    launches = ops.LAUNCHES[0] / float(steps * reps)
+    ms, host_ms, last = region(steps)
+    launches = ops.LAUNCHES[0] / float(steps)
     out = {"metric": "SSD3D training volumes/sec (fwd + IoU matching + MultiBox loss + bwd + all-reduce + Adam)",
-           "volumes_per_s": world * TRAIN_BATCH * steps * reps / (ms / 1000.0), "ms_per_step": ms / (steps * reps),
-           "host_ms_per_step": host_ms / (steps * reps), "steps": steps, "repeats": reps, "timed_region_ms": ms,
+           "volumes_per_s": world * TRAIN_BATCH * steps / (ms / 1000.0), "ms_per_step": ms / steps,
+           "host_ms_per_step": host_ms / steps, "steps": steps, "timed_region_ms": ms,
            "launches_per_step": launches, "n_gpus": world, "scaling": "weak", "dtype": "bf16 activations, fp32 "
            "gradients / optimizer", "loss": [float(v) for v in last.cpu()],
            "skipped_steps": model.fit_skipped_steps(),
@@ -387,6 +393,15 @@ def train_roofline(dev):
             "timing": "%d back-to-back launches between one CUDA event pair, three rotating (z, g) pairs = 680 MB" % launches}
 
 
+def dump_outputs(out_dir, boxes, labels, scores):
+    """Per-volume detections of one step (lists of device tensors) -> out_dir/{boxes,labels,scores,counts}.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"boxes": torch.cat(boxes).reshape(-1, 6), "labels": torch.cat(labels), "scores": torch.cat(scores),
+              "counts": torch.tensor([b.shape[0] for b in boxes])}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(np.float32))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -398,7 +413,11 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip every secondary measurement")
     ap.add_argument("--eager", action="store_true",
                     help="launch every kernel individually (no CUDA graph): for ncu launch lists, not for numbers")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the detections of the last timed step to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     from mslesions3d_b200.parallel import rank_world, max_over_ranks
@@ -459,58 +478,63 @@ def main():
         sampler.window(t0, time.time())
         return max_over_ranks(e0.elapsed_time(e1), dev)    # the job is as slow as its slowest rank
 
-    d2h_bytes = [0]
+    depth = int(model.pipeline_depth)
 
-    def run_resident(steps):
-        """`steps` device-resident batches through LSSD3D.predict_batches (results stay on the device)."""
-        batches = ({"img": dev_bf16[i % N_ROTATE]} for i in range(steps))
-        if args.eager:
+    def run_stream(src, warmup, steps, to_host=False):
+        """Batches rotating over src through ONE pass of LSSD3D.predict_batches (one predict_step per batch on the
+        device-resident path with --eager).  The CUDA event pair opens when the result of the warmup-th batch is
+        handed back and closes at the result of the `steps`-th batch after it, with depth - 1 more batches still
+        queued behind it: both ends see the same batches in flight, so the region holds exactly `steps` steps of a
+        full pipeline; its fill and drain are outside.  -> (ms max over ranks, results of the last timed step)."""
+        barrier()
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        batches = ({"img": src[i % N_ROTATE]} for i in range(warmup + steps + depth - 1))
+        if args.eager and not to_host:
             model.use_cuda_graph = False
-            with torch.no_grad():
-                for b in batches:
-                    model.predict_step(b, 0)
-            return
+            results = (model.predict_step(b, 0) for b in batches)
+        else:
+            results = model.predict_batches(batches, to_host=to_host)
         with torch.no_grad():
-            for _ in model.predict_batches(batches):
+            for i, out in enumerate(results):
+                assert out[0][0].is_cuda != to_host
+                if i == warmup - 1:
+                    t0 = time.time()
+                    e0.record()
+                elif i == warmup + steps - 1:
+                    e1.record()
+                    t1, last = time.time(), out
+        barrier()
+        sampler.window(t0, t1)
+        return max_over_ranks(e0.elapsed_time(e1), dev), last    # the job is as slow as its slowest rank
+
+    def capture(src, to_host=False):
+        """Build (capture) the inference plan of every pipeline slot: one-off setup, not a step."""
+        with torch.no_grad():
+            for _ in model.predict_batches(({"img": src[i % N_ROTATE]} for i in range(depth)), to_host=to_host):
                 pass
 
-    def run_e2e(steps, host):
-        """`steps` batches through the public streaming API (LSSD3D.predict_batches): every batch is copied
-        from pinned host memory inside the timed region and its detections are read back to the host."""
-        batches = ({"img": host[i % N_ROTATE]} for i in range(steps))
-        with torch.no_grad():
-            for b, l, s in model.predict_batches(batches, to_host=True):
-                assert not b[0].is_cuda
-        # per step: padded boxes/labels/scores (top_k rows per volume) + the count/status/flag words
-        d2h_bytes[0] = BATCH * TOP_K * (24 + 4 + 8 + 8) + 4 * (BATCH + 2)
-
-    def repeats_for(ms_probe, probe_steps):
-        return max(1, int(math.ceil(MIN_REGION_MS / max(ms_probe * args.steps / probe_steps, 1e-3))))
-
     # ---- resident-input throughput (value) --------------------------------------------------------
-    # Build (capture) the inference plan of every pipeline slot first: that is one-off setup, not a step.
-    depth = int(model.pipeline_depth)
-    run_resident(depth)
-    run_resident(args.warmup)
-    probe = timed(lambda: run_resident(args.steps))
-    reps = repeats_for(probe, args.steps)
+    if not args.eager:
+        capture(dev_bf16)
     ops.LAUNCHES[0] = 0
-    ms = timed(lambda: run_resident(args.steps * reps))
-    launches = ops.LAUNCHES[0]
-    n_timed = args.steps * reps
+    ms, last = run_stream(dev_bf16, args.warmup, args.steps)
+    launches = round(ops.LAUNCHES[0] * args.steps / (args.warmup + args.steps + depth - 1))   # same every step
+    n_timed = args.steps
     value = world * BATCH * n_timed / (ms / 1000.0)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)
+    del last
 
     # ---- end to end from pinned host memory --------------------------------------------------------
+    # every batch is copied from pinned host memory inside the timed region and its detections are read back
+    # to the host; per step: padded boxes/labels/scores (top_k rows per volume) + the count/status/flag words
+    d2h_bytes = BATCH * TOP_K * (24 + 4 + 8 + 8) + 4 * (BATCH + 2)
     e2e = {}
     for name, host in (("bf16", host_bf16), ("fp32", host_f32)):
-        run_e2e(depth, host)
-        run_e2e(args.warmup, host)
-        probe = timed(lambda: run_e2e(args.steps, host))
-        r_e = repeats_for(probe, args.steps)
-        ms_e = timed(lambda: run_e2e(args.steps * r_e, host))
-        e2e[name] = {"value": world * BATCH * args.steps * r_e / (ms_e / 1000.0), "ms_per_step": ms_e / (args.steps * r_e),
-                     "h2d_bytes_per_step": host[0].numel() * host[0].element_size(), "repeats": r_e,
-                     "timed_region_ms": ms_e}
+        capture(host, to_host=True)
+        ms_e, _ = run_stream(host, args.warmup, args.steps, to_host=True)
+        e2e[name] = {"value": world * BATCH * args.steps / (ms_e / 1000.0), "ms_per_step": ms_e / args.steps,
+                     "h2d_bytes_per_step": host[0].numel() * host[0].element_size(), "timed_region_ms": ms_e}
     # bare copy loop: what the host fabric gives `world` ranks copying at once, no compute
     stage = torch.empty_like(dev_bf16[0])
     copy_stream = torch.cuda.Stream(device=dev)
@@ -627,7 +651,7 @@ def main():
             model._plans.clear()
             del dev_bf16
             torch.cuda.empty_cache()
-            extras["train"] = train_leg(dev, rank, world, min(args.steps, 50), args.warmup, barrier, max_over_ranks)
+            extras["train"] = train_leg(dev, rank, world, args.steps, args.warmup, barrier, max_over_ranks)
         except Exception as exc:      # noqa: BLE001
             if world > 1:
                 raise
@@ -651,20 +675,20 @@ def main():
             "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": ms / n_timed, "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "bf16", "data": "synthetic",
-            "repeats": reps, "timed_steps": n_timed, "timed_region_ms": ms,
+            "timed_steps": n_timed, "timed_region_ms": ms,
             "config": {"workload": WORKLOAD, "global_batch": BATCH * world, "parallelism": "dp%d" % world,
                        "l2": "inputs rotate over %d resident batches (%d MB) > 126 MB L2" %
                              (N_ROTATE, N_ROTATE * in_bytes // 2 ** 20),
                        "min_score": MIN_SCORE, "max_overlap": MAX_OVERLAP, "top_k": TOP_K, "priors": 9344,
-                       "timed_region": "the %d steps are repeated %d x inside one CUDA event pair (>= %d ms)"
-                                       % (args.steps, reps, int(MIN_REGION_MS)),
+                       "timed_region": "%d steps inside one CUDA event pair, in the middle of one pipelined pass (after "
+                                       "%d warm-up batches, before the drain)" % (args.steps, args.warmup),
                        "pipeline": "%d batches in flight (LSSD3D.predict_batches: one captured plan per slot, own "
                                    "stream each; a step = one batch through stem + graph replay + result read-back)" % depth},
             "e2e": {"value": e2e["bf16"]["value"], "unit": UNIT, "h2d_bytes_per_step": in_bytes,
-                    "d2h_bytes_per_step": d2h_bytes[0], "ms_per_step": e2e["bf16"]["ms_per_step"],
+                    "d2h_bytes_per_step": d2h_bytes, "ms_per_step": e2e["bf16"]["ms_per_step"],
                     "host_format": "bf16 pinned batches (bit-identical detections: the stem rounds fp32 inputs to bf16 "
                                    "on load)",
-                    "repeats": e2e["bf16"]["repeats"], "timed_region_ms": e2e["bf16"]["timed_region_ms"],
+                    "timed_region_ms": e2e["bf16"]["timed_region_ms"],
                     "fp32_host": {"value": e2e["fp32"]["value"], "ms_per_step": e2e["fp32"]["ms_per_step"],
                                   "h2d_bytes_per_step": e2e["fp32"]["h2d_bytes_per_step"],
                                   "note": "the fp32 batches the reference's loader yields (datasets.py:403)"},

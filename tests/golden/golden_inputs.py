@@ -56,6 +56,14 @@ def checksum(t: torch.Tensor) -> float:
     return float(t.double().sum())
 
 
+def checksum_matches(t: torch.Tensor, gold: float) -> bool:
+    """``checksum(t) == gold`` up to the rounding of the float64 sum itself: the order in which torch adds on the
+    CPU (vector width, thread count) moves the last bits from one machine to another.  1e-13 of the sum of
+    magnitudes is far above that rounding and far below what a drifted random stream or input recipe changes."""
+    t = t.double()
+    return abs(float(t.sum()) - gold) <= 1e-13 * max(1.0, float(t.abs().sum()))
+
+
 def forward_inputs(case):
     """(state_dict, image) for a FORWARD case."""
     sd = O.random_state_dict(case["channels"], case.get("aspect_ratios"), case.get("n_classes", 2),

@@ -45,11 +45,14 @@ def test_library_is_sm100a_tcgen05_code():
     import shutil
     import subprocess
     from mslesions3d_b200 import _lib
-    if not shutil.which("cuobjdump"):
-        pytest.skip("cuobjdump not on PATH")
-    elf = subprocess.run(["cuobjdump", "-lelf", _lib.LIB_PATH], capture_output=True, text=True).stdout
+    # the toolkit under CUDA_HOME (where the build looks for nvcc), whether or not its bin directory is on PATH
+    cuda_bin = os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin")
+    cuobjdump = shutil.which("cuobjdump", path=cuda_bin) or shutil.which("cuobjdump")
+    if not cuobjdump:
+        pytest.skip("cuobjdump not found")
+    elf = subprocess.run([cuobjdump, "-lelf", _lib.LIB_PATH], capture_output=True, text=True).stdout
     assert "sm_100a" in elf and "sm_90" not in elf and "sm_80" not in elf
-    sass = subprocess.run(["cuobjdump", "-sass", _lib.LIB_PATH], capture_output=True, text=True).stdout
+    sass = subprocess.run([cuobjdump, "-sass", _lib.LIB_PATH], capture_output=True, text=True).stdout
     for mnemonic in ("UTCHMMA", "UTMALDG", "LDTM"):
         assert mnemonic in sass, "%s missing from the GEMM SASS" % mnemonic
 

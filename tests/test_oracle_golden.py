@@ -41,8 +41,8 @@ def test_prior_known_answers():
 def test_forward_matches_reference(name):
     case, gold = GI.FORWARD_CASES[name], load_golden("forward.pt")[name]
     sd, x = GI.forward_inputs(case)
-    assert GI.checksum(x) == gold["x_sum"], "synthetic input drifted from the golden run"
-    assert GI.checksum(torch.cat([v.flatten().float() for v in sd.values()])) == gold["w_sum"]
+    assert GI.checksum_matches(x, gold["x_sum"]), "synthetic input drifted from the golden run"
+    assert GI.checksum_matches(torch.cat([v.flatten().float() for v in sd.values()]), gold["w_sum"])
     assert set(sd.keys()) == set(gold["keys"])
     with torch.no_grad():
         locs, scores = O.forward(sd, x, case.get("aspect_ratios"), case.get("n_classes", 2))
@@ -68,7 +68,7 @@ def test_detect_matches_reference(name):
     case, gold = GI.DETECT_CASES[name], load_golden("detect.pt")[name]
     priors = O.prior_boxes(case["size"], in_channels=case["channels"])
     locs, scores = GI.detect_inputs(case, priors.shape[0])
-    assert GI.checksum(torch.cat([locs.flatten(), scores.flatten()])) == gold["in_sum"]
+    assert GI.checksum_matches(torch.cat([locs.flatten(), scores.flatten()]), gold["in_sum"])
     b, l, s, idx = O.detect_objects(locs, scores, priors, case["min_score"], case["max_overlap"], case["top_k"],
                                     return_indices=True)
     for i in range(case["batch"]):
@@ -88,7 +88,7 @@ def test_detect_long_lists_match_reference(name):
     assert priors.shape[0] == gold["n_priors"] > 16384 and 10 * case["top_k"] > 8192
     assert torch.equal(priors, O.prior_boxes(case["size"], case["aspect_ratios"], in_channels=case["channels"]))
     locs, scores = GI.detect_long_inputs(case, priors.shape[0])
-    assert GI.checksum(torch.cat([locs.flatten(), scores.flatten()])) == gold["in_sum"]
+    assert GI.checksum_matches(torch.cat([locs.flatten(), scores.flatten()]), gold["in_sum"])
     b, l, s, idx = O.detect_objects(locs, scores, priors, case["min_score"], case["max_overlap"], case["top_k"],
                                     return_indices=True)
     for i in range(case["batch"]):
@@ -125,7 +125,7 @@ def test_bf16_emulation_is_close_to_fp32():
 def test_map_matches_reference(name):
     case, gold = GI.MAP_CASES[name], load_golden("map.pt")[name]
     db, dl, ds, tb, tl, td = GI.map_inputs(case)
-    assert GI.checksum(torch.cat([torch.cat(db).flatten(), torch.cat(ds)])) == gold["in_sum"]
+    assert GI.checksum_matches(torch.cat([torch.cat(db).flatten(), torch.cat(ds)]), gold["in_sum"])
     o = O.calculate_map(db, dl, ds, tb, tl, td, case["min_overlap"])
     d = gold["detail"]
     assert o["mAP"] == d["mAP"] == gold["simple"][1]
@@ -145,7 +145,7 @@ def test_train_step_matches_reference(name):
     """Train-mode forward + MultiBox loss + autograd backward of the oracle vs the unmodified reference."""
     case, gold = GI.TRAIN_CASES[name], load_golden("train.pt")[name]
     sd, x, boxes, labels = GI.train_inputs(case)
-    assert GI.checksum(x) == gold["x_sum"]
+    assert GI.checksum_matches(x, gold["x_sum"])
     pri = O.prior_boxes(case["size"], in_channels=case["channels"])
     r = O.train_step_grads(sd, x, boxes, labels, pri, case["threshold"])
     torch.testing.assert_close(r["conf"], gold["conf"], rtol=1e-5, atol=1e-5)
