@@ -492,6 +492,52 @@ int ssd3d_gt_boxes_from_instances(const void* seg, int seg_dtype, int N, int D, 
                                   float* boxes, int64_t* labels, int32_t* counts, int32_t* n_components,
                                   void* workspace, int64_t workspace_bytes, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Training from a device-resident data set: sampling and augmentation inside the captured training step.
+ *
+ * ssd3d_augment_batch builds one training batch in one launch.  Slot b takes subject
+ * order[(step * N * world + rank * N + b) mod S] (DistributedSampler's split; the last batch wraps around, so
+ * every batch holds N volumes).  Its draws come from Philox4x32-10, key = seed, counter = (rank * N + b, draw
+ * counter low, draw counter high, call), with u01(u) = (u >> 8) * 2^-24, Bernoulli(p) = u01 < p and
+ * randint(lo, hi) = lo + ((u * (hi - lo)) >> 32) as ssd3d_generate_volumes:
+ *   call 0 {positive crop, box, rot90, k}, call 1 {offset d, h, w}, call 2 {flip d, h, w}, call 3 {scale, shift}.
+ * Applied in this order, to the image and the mask alike:
+ *   1. crop to (d, h, w): with probability pos_ratio, if the subject has a lesion box, one of its boxes
+ *      (uniform) and per axis an offset uniform over the windows that contain the box -- or, on an axis where the
+ *      box is longer than the window, its centre voxel (lo + hi) / 2; otherwise uniform over [0, src - out].
+ *   2. np.rot90(x, k, axes = (rot_axis0, rot_axis1)) with probability rot90_prob, k uniform in {1, 2, 3}; the
+ *      two output extents must be equal.
+ *   3. np.flip of each spatial axis with probability flip_prob.
+ *   4. (image only) y = bf16_rn(fp32_rn(fp32_rn(x * fp32_rn(1 + f)) + o)), f = scale * (2 u01 - 1),
+ *      o = shift * (2 u01 - 1), per volume and shared by its channels (MONAI's non-channel-wise default).
+ * Bounding boxes of the mask follow from it through ssd3d_gt_boxes_from_segmentation (utils.py:438-513).
+ *   src (S, C, Ds, Hs, Ws) fp32 (src_is_bf16 = 0) or bf16; masks (S, Ds, Hs, Ws) uint8; order (S) int32
+ *   state (8 int64) = {seed, draw counter, step in the epoch, rank, world size, 0 (kernel scratch), -, -}: the
+ *         launch advances the draw counter and the step by one, so a captured graph draws a new batch per replay
+ *   boxes (B, 6) int32 lesion boxes in voxel indices [lo d, lo h, lo w, hi d, hi h, hi w] (inclusive), subject s
+ *         owning rows [box_offsets[s], box_offsets[s + 1])
+ *   out (N, C, d, h, w) bf16, out_mask (N, d, h, w) uint8, record (N, 16) int32 = {subject, offset d, h, w, k,
+ *         flip d, h, w, positive crop, box (-1: none), f (fp32 bits), o (fp32 bits), step, draw counter low,
+ *         global slot, boxes of the subject}.
+ * d, h, w <= Ds, Hs, Ws; w % 16 == 0 (16-byte stores); probabilities in [0, 1].
+ *
+ * ssd3d_gt_pack turns the per-image output of ssd3d_gt_boxes_from_segmentation (boxes (N, max_boxes, 6), labels
+ * (N, max_boxes), counts, n_components) into the packed ground truth of the training step: gt_boxes
+ * (N * per_volume, 6), gt_labels (N * per_volume) int64 and offsets (N + 1) int32 (the ssd3d_match_priors input),
+ * without a host sync.  A batch in which a volume has more boxes than per_volume, or more components than
+ * max_boxes (its list was truncated), overflows: it is packed as a batch without ground truth -- no positive
+ * prior, so the MultiBox gradient is non-finite and ssd3d_adam_step_dev skips and counts the step -- and
+ * status (2 int32) = {overflow of this batch, overflowing batches so far} records it (status[1] zeroed once by
+ * the caller).  N <= 8192. */
+int ssd3d_augment_batch(const void* src, int src_is_bf16, const uint8_t* masks, int S, int C, int Ds, int Hs, int Ws,
+                        const int32_t* order, int64_t* state, const int32_t* boxes, const int32_t* box_offsets, int N,
+                        int d, int h, int w, float pos_ratio, float flip_prob, float rot90_prob, int rot_axis0,
+                        int rot_axis1, float scale, float shift, void* out, uint8_t* out_mask, int32_t* record,
+                        void* stream);
+int ssd3d_gt_pack(const float* boxes, const int64_t* labels, const int32_t* counts, const int32_t* n_components,
+                  int N, int max_boxes, int per_volume, float* gt_boxes, int64_t* gt_labels, int32_t* offsets,
+                  int32_t* status, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

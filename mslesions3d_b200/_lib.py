@@ -121,6 +121,10 @@ SIGNATURES = {
                                             P]),
     "ssd3d_adam_step_dev": (c_int, [P, P, P, P, c_int64, c_int64, c_float, c_float, c_int, c_float, c_float, c_float,
                                     c_float, c_float, P, P, P]),
+    # ---- training batches from a device-resident data set ----
+    "ssd3d_augment_batch": (c_int, [P, c_int, P, c_int, c_int, c_int, c_int, c_int, P, P, P, P, c_int, c_int, c_int,
+                                    c_int, c_float, c_float, c_float, c_int, c_int, c_float, c_float, P, P, P, P]),
+    "ssd3d_gt_pack": (c_int, [P, P, P, P, c_int, c_int, c_int, P, P, P, P, P]),
 }
 
 _lib = None

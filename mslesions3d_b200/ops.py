@@ -1043,6 +1043,18 @@ def gt_boxes_from_segmentation(seg: torch.Tensor, n_classes: int = 0, max_boxes:
         seg = seg[:, 0]
     if seg.dim() != 4:
         raise RuntimeError("expected (N, D, H, W) or (N, 1, D, H, W) segmentations")
+    boxes, labels, meta = gt_boxes_padded(seg, n_classes, max_boxes)
+    n = boxes.shape[0]
+    counts, comps = meta.cpu().tolist()
+    if max(comps) > max_boxes:
+        raise RuntimeError("segmentation has %d connected components, max_boxes=%d" % (max(comps), max_boxes))
+    return [boxes[i, :counts[i]] for i in range(n)], [labels[i, :counts[i]] for i in range(n)]
+
+
+def gt_boxes_padded(seg: torch.Tensor, n_classes: int = 0, max_boxes: int = 1024, out=None, workspace=None):
+    """``gt_boxes_from_segmentation`` without the host read: -> (boxes (N, max_boxes, 6), labels (N, max_boxes),
+    meta (2, N) int32 = [counts, n_components]); rows [0, counts[i]) are valid, and only if n_components[i] <=
+    max_boxes.  ``out`` / ``workspace`` (from an earlier call) make it capturable in a CUDA graph."""
     if seg.dtype == torch.uint8:
         dt = 0
     else:
@@ -1050,20 +1062,21 @@ def gt_boxes_from_segmentation(seg: torch.Tensor, n_classes: int = 0, max_boxes:
     seg = seg.contiguous()
     n, d, h, w = seg.shape
     dev = seg.device
-    boxes = torch.empty((n, max_boxes, 6), dtype=torch.float32, device=dev)
-    labels = torch.empty((n, max_boxes), dtype=torch.int64, device=dev)
-    meta = torch.empty((2, n), dtype=torch.int32, device=dev)
     lib = _lib.load()
-    ws = torch.empty((lib.ssd3d_gt_boxes_workspace_bytes(n, d, h, w, max_boxes),), dtype=torch.uint8, device=dev)
+    if out is None:
+        out = (torch.empty((n, max_boxes, 6), dtype=torch.float32, device=dev),
+               torch.empty((n, max_boxes), dtype=torch.int64, device=dev),
+               torch.empty((2, n), dtype=torch.int32, device=dev))
+    boxes, labels, meta = out
+    if workspace is None:
+        workspace = torch.empty((lib.ssd3d_gt_boxes_workspace_bytes(n, d, h, w, max_boxes),), dtype=torch.uint8,
+                                device=dev)
     rc = lib.ssd3d_gt_boxes_from_segmentation(seg.data_ptr(), dt, n, d, h, w, int(n_classes), int(max_boxes),
                                               boxes.data_ptr(), labels.data_ptr(), meta[0].data_ptr(),
-                                              meta[1].data_ptr(), ws.data_ptr(), ws.numel(), _stream())
+                                              meta[1].data_ptr(), workspace.data_ptr(), workspace.numel(), _stream())
     _lib.check(rc, "ssd3d_gt_boxes_from_segmentation")
     LAUNCHES[0] += 6
-    counts, comps = meta.cpu().tolist()
-    if max(comps) > max_boxes:
-        raise RuntimeError("segmentation has %d connected components, max_boxes=%d" % (max(comps), max_boxes))
-    return [boxes[i, :counts[i]] for i in range(n)], [labels[i, :counts[i]] for i in range(n)]
+    return boxes, labels, meta
 
 
 def gt_boxes_from_instances(seg: torch.Tensor, thresholds, max_boxes: int = 1024):
@@ -1134,3 +1147,63 @@ def generate_volumes(n: int, channels: int, image_size, first_idx: int = 0, seed
     _lib.check(rc, "ssd3d_generate_volumes")
     LAUNCHES[0] += 2
     return raw, mask, cubes, n_cubes
+
+
+# ----------------------------------------------------------------------------------------------
+# training batches from a device-resident data set (data.py, training.fit_epoch)
+# ----------------------------------------------------------------------------------------------
+def augment_batch(src: torch.Tensor, masks: torch.Tensor, order: torch.Tensor, state: torch.Tensor,
+                  boxes: torch.Tensor, box_offsets: torch.Tensor, batch_size: int, out_size, pos_ratio: float = 0.0,
+                  flip_prob: float = 0.0, rot90_prob: float = 0.0, rot90_axes=(0, 1), scale: float = 0.0,
+                  shift: float = 0.0, out=None):
+    """One augmented training batch (see ``ssd3d_augment_batch`` in the header): src (S, C, Ds, Hs, Ws) fp32 / bf16,
+    masks (S, Ds, Hs, Ws) uint8, order (S) int32, state (8) int64 (advanced by the call), boxes (B, 6) int32 voxel
+    boxes, box_offsets (S + 1) int32 -> (images (N, C, d, h, w) bf16, masks (N, d, h, w) uint8, record (N, 16)
+    int32).  ``out``: the three output tensors to write (static buffers of a captured step)."""
+    _need_cuda(src, masks, order, state, boxes, box_offsets)
+    if src.dim() != 5 or masks.dim() != 4 or src.dtype not in (torch.float32, BF16) or masks.dtype != torch.uint8:
+        raise RuntimeError("expected src (S, C, D, H, W) fp32/bf16 and masks (S, D, H, W) uint8")
+    for t, dt in ((order, torch.int32), (state, torch.int64), (boxes, torch.int32), (box_offsets, torch.int32)):
+        if t.dtype != dt or not t.is_contiguous():
+            raise RuntimeError("order / boxes / box_offsets must be contiguous int32 and state int64")
+    s, c, ds, hs, ws = src.shape
+    d, h, w = (int(v) for v in out_size)
+    n = int(batch_size)
+    if out is None:
+        out = (torch.empty((n, c, d, h, w), dtype=BF16, device=src.device),
+               torch.empty((n, d, h, w), dtype=torch.uint8, device=src.device),
+               torch.empty((n, 16), dtype=torch.int32, device=src.device))
+    img, msk, rec = out
+    rc = _lib.load().ssd3d_augment_batch(src.data_ptr(), int(src.dtype == BF16), masks.data_ptr(), s, c, ds, hs, ws,
+                                         order.data_ptr(), state.data_ptr(), boxes.data_ptr(), box_offsets.data_ptr(),
+                                         n, d, h, w, float(pos_ratio), float(flip_prob), float(rot90_prob),
+                                         int(rot90_axes[0]), int(rot90_axes[1]), float(scale), float(shift),
+                                         img.data_ptr(), msk.data_ptr(), rec.data_ptr(), _stream())
+    _lib.check(rc, "ssd3d_augment_batch")
+    LAUNCHES[0] += 1
+    return img, msk, rec
+
+
+def gt_pack(boxes: torch.Tensor, labels: torch.Tensor, meta: torch.Tensor, per_volume: int, out=None,
+            status: Optional[torch.Tensor] = None):
+    """The output of ``gt_boxes_padded`` -> the packed ground truth of a training step, no host sync:
+    (gt_boxes (N * per_volume, 6), gt_labels (N * per_volume) int64, offsets (N + 1) int32, status (2) int32 =
+    [overflow of this batch, overflowing batches so far]).  An overflowing batch is packed without ground truth."""
+    _need_cuda(boxes, labels, meta)
+    n, max_boxes = int(boxes.shape[0]), int(boxes.shape[1])
+    dev = boxes.device
+    if out is None:
+        out = (torch.zeros((n * per_volume, 6), dtype=torch.float32, device=dev),
+               torch.zeros((n * per_volume,), dtype=torch.int64, device=dev),
+               torch.zeros((n + 1,), dtype=torch.int32, device=dev))
+    if status is None:
+        status = torch.zeros((2,), dtype=torch.int32, device=dev)
+    gb, gl, offs = out
+    if gb.shape[0] < n * per_volume or gl.shape[0] < n * per_volume or offs.shape[0] != n + 1:
+        raise RuntimeError("gt_pack: output buffers smaller than N * per_volume rows")
+    rc = _lib.load().ssd3d_gt_pack(boxes.data_ptr(), labels.data_ptr(), meta[0].data_ptr(), meta[1].data_ptr(), n,
+                                   max_boxes, int(per_volume), gb.data_ptr(), gl.data_ptr(), offs.data_ptr(),
+                                   status.data_ptr(), _stream())
+    _lib.check(rc, "ssd3d_gt_pack")
+    LAUNCHES[0] += 1
+    return gb, gl, offs, status

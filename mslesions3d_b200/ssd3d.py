@@ -842,6 +842,29 @@ class LSSD3D(_LightningBase):
             raise RuntimeError("fit_step needs train() mode")
         return training.fit_step(self, batch, world_size, allreduce)
 
+    def fit_epoch(self, dataset, batch_size: int, augment=None, epoch: int = 0, world_size: int = None,
+                  allreduce=None, max_boxes_per_volume: int = 64):
+        """One epoch over a ``data.DeviceDataset``, every step ONE CUDA-graph replay: sample the batch (this rank's
+        share of ``data.epoch_order``), augment it (``data.Augment``; default: none, which needs a data set of
+        ``input_size`` volumes) into bf16 images, extract and pack the ground truth of the augmented masks, then
+        forward, loss, backward, (all-reduce) and Adam as ``fit_step``.  ceil(S / (batch_size * world_size)) steps;
+        the last batch wraps around to the start of the order.  No host copy or sync inside the epoch.
+        Returns (losses (steps, 2) [conf, loc], subjects (steps, batch_size) int32) as device tensors.
+        A step in which a volume has more than ``max_boxes_per_volume`` boxes (a crop can split a lesion) is
+        skipped like a non-finite one; the epoch then raises at its end."""
+        from . import training
+        import torch.distributed as dist
+        dist_on = dist.is_available() and dist.is_initialized()
+        if world_size is None:
+            world_size = dist.get_world_size() if dist_on else 1
+        if allreduce is None and world_size > 1:
+            allreduce = dist.all_reduce
+        if not self.training:
+            raise RuntimeError("fit_epoch needs train() mode")
+        rank = dist.get_rank() if dist_on and world_size > 1 else 0
+        return training.fit_epoch(self, dataset, batch_size, augment, epoch, world_size, allreduce, rank,
+                                  max_boxes_per_volume)
+
     def fit_skipped_steps(self) -> int:
         """Number of fit_step calls whose gradient was NaN / Inf (e.g. a batch without one positive prior: the
         reference raises "Loss is NaN", ssd3d.py:938-940) and whose update was therefore skipped on the device.

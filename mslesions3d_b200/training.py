@@ -529,6 +529,7 @@ class _TrainPlan:
         self.n_kernels = 0
         self.graph = None
         self.optimizer_in_graph = False
+        self.extra_state = []       # device state besides the model's that the warm-up steps change (restored)
 
     def load(self, images, gt_boxes, gt_labels):
         self.image.copy_(images, non_blocking=True)
@@ -556,6 +557,7 @@ class _TrainPlan:
                 self.gt_labels[:total].copy_(torch.cat(labels).long(), non_blocking=True)
 
     def _run(self, model, with_optimizer: bool):
+        self._prepare(model)
         eng = model.train_engine()
         lf = model.loss_fn
         t0, t1 = (lf.threshold, lf.threshold) if lf.thresholding_mode == "hard" else lf.threshold
@@ -573,6 +575,9 @@ class _TrainPlan:
             _optimizer_step(model, self.flat, self.world_size, self.allreduce)
         self.loss = out
 
+    def _prepare(self, model):
+        """Work of the step before the forward pass (nothing: the host stages the batch, ``load``)."""
+
     def capture(self, model):
         """Warm up (lazy module loading, workspaces, the NCCL communicator) and record.  The warm-up steps run
         for real, so everything they touch -- BatchNorm buffers, parameters, Adam moments and counters -- is
@@ -580,7 +585,8 @@ class _TrainPlan:
         flat = self.flat
         in_graph = os.environ.get("SSD3D_TRAIN_OPT_IN_GRAPH", "1") != "0"
         buffers = {k: v.clone() for k, v in model.named_buffers()}
-        saved = [t.clone() for t in (flat.param, flat.exp_avg, flat.exp_avg_sq, flat.status)]
+        state = (flat.param, flat.exp_avg, flat.exp_avg_sq, flat.status, *self.extra_state)
+        saved = [t.clone() for t in state]
         side = torch.cuda.Stream(device=model.device)
         side.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(side), torch.no_grad():
@@ -593,7 +599,7 @@ class _TrainPlan:
             with torch.no_grad():
                 for k, v in model.named_buffers():
                     v.copy_(buffers[k])
-                for t, v in zip((flat.param, flat.exp_avg, flat.exp_avg_sq, flat.status), saved):
+                for t, v in zip(state, saved):
                     t.copy_(v)
                 model.train_engine().packed.refresh()
             torch.cuda.synchronize()
@@ -692,3 +698,107 @@ def fit_step(model, batch, world_size: int = 1, allreduce=None):
         _optimizer_step(model, flat, world_size, allreduce)
         model.invalidate_packed()
     return out
+
+
+class _EpochPlan(_TrainPlan):
+    """The fused step fed from a ``DeviceDataset``: the captured graph also samples and augments the batch straight
+    into the static image buffer (``ssd3d_augment_batch``), extracts the ground truth of the augmented masks
+    (``ssd3d_gt_boxes_from_segmentation``) and packs it into the static GT buffers (``ssd3d_gt_pack``).  The draw
+    state advances inside the graph, so every replay is the next step of the epoch with no host copy or sync."""
+
+    def __init__(self, model, dataset, augment, n: int, per_volume: int, world_size: int, allreduce):
+        dev = model.device
+        d, h, w = (int(v) for v in model.input_size)
+        c = dataset.channels
+        super().__init__(model, torch.empty((n, c, d, h, w), dtype=torch.bfloat16, device="meta"), n * per_volume,
+                         world_size, allreduce)
+        self.dataset, self.augment, self.per_volume = dataset, augment, per_volume
+        self.mask = torch.empty((n, d, h, w), dtype=torch.uint8, device=dev)
+        self.record = torch.empty((n, 16), dtype=torch.int32, device=dev)
+        self.order = torch.zeros((len(dataset),), dtype=torch.int32, device=dev)
+        # {seed, draw counter, step in epoch, rank, world size, kernel scratch, -, -}
+        self.state = torch.zeros((8,), dtype=torch.int64, device=dev)
+        self.pack_status = torch.zeros((2,), dtype=torch.int32, device=dev)
+        self.gt_out = (torch.empty((n, per_volume, 6), dtype=torch.float32, device=dev),
+                       torch.empty((n, per_volume), dtype=torch.int64, device=dev),
+                       torch.empty((2, n), dtype=torch.int32, device=dev))
+        lib = _lib.load()
+        self.gt_ws = torch.empty((lib.ssd3d_gt_boxes_workspace_bytes(n, d, h, w, per_volume),), dtype=torch.uint8,
+                                 device=dev)
+        self.extra_state = [self.state, self.pack_status]
+
+    def _prepare(self, model):
+        a, ds = self.augment, self.dataset
+        ops.augment_batch(ds.images, ds.masks, self.order, self.state, ds.boxes, ds.box_offsets, self.n,
+                          model.input_size, a.pos_ratio, a.flip_prob, a.rot90_prob, a.rot90_axes, a.scale, a.shift,
+                          out=(self.image, self.mask, self.record))
+        boxes, labels, meta = ops.gt_boxes_padded(self.mask, ds.n_classes, self.per_volume, out=self.gt_out,
+                                                  workspace=self.gt_ws)
+        ops.gt_pack(boxes, labels, meta, self.per_volume, out=(self.gt_boxes, self.gt_labels, self.offsets),
+                    status=self.pack_status)
+
+    def start_epoch(self, epoch: int, steps: int, rank: int):
+        """Host writes of one epoch, before its first step: the order, the draw state, the overflow count."""
+        from .data import epoch_order
+        seed = int(self.augment.seed)
+        self.order.copy_(epoch_order(len(self.dataset), epoch, seed))
+        seed = seed - (1 << 64) if seed >= (1 << 63) else seed
+        # draws are a pure function of (seed, epoch, step, slot): the counter of step t of epoch e is e * steps + t
+        self.state.copy_(torch.tensor([seed, int(epoch) * steps, 0, rank, self.world_size, 0, 0, 0],
+                                      dtype=torch.int64))
+        self.pack_status.zero_()
+
+
+def fit_epoch(model, dataset, batch_size: int, augment=None, epoch: int = 0, world_size: int = 1, allreduce=None,
+              rank: int = 0, max_boxes_per_volume: int = 64):
+    """One epoch of fused steps over a ``DeviceDataset``; see ``LSSD3D.fit_epoch``."""
+    from .data import Augment
+    if augment is None:
+        augment = Augment()
+    if not model.use_cuda_graph:
+        raise RuntimeError("fit_epoch runs every step as a CUDA-graph replay; it needs model.use_cuda_graph")
+    if dataset.images.device != model.device:
+        raise RuntimeError("the data set lives on %s, the model on %s" % (dataset.images.device, model.device))
+    if dataset.channels != model.input_channels:
+        raise ValueError("the data set has %d channels, the model expects %d" % (dataset.channels,
+                                                                                 model.input_channels))
+    augment.validate(model.input_size, dataset.shape)
+    n, per_volume = int(batch_size), int(max_boxes_per_volume)
+    if n < 1 or per_volume < 1:
+        raise ValueError("batch_size and max_boxes_per_volume must be >= 1")
+    eng = model.train_engine()
+    eng.flatten()
+    eng.collective_mode = "none" if allreduce is None else ("nccl all_reduce of the flat gradient, captured in the "
+                                                            "step's CUDA graph")
+    steps = -(-len(dataset) // (n * world_size))
+    key = ("epoch", id(dataset), augment, n, per_volume, tuple(model.input_size), int(world_size), int(rank),
+           allreduce)
+    plan = eng.plans.get(key)
+    if plan is None or plan.dataset is not dataset:
+        plan = _EpochPlan(model, dataset, augment, n, per_volume, world_size, allreduce)
+        plan.start_epoch(epoch, steps, rank)
+        model.invalidate_packed()
+        plan.capture(model)
+        eng.plans.pop(key, None)
+        if len(eng.plans) >= 4:
+            eng.plans.clear()
+        eng.plans[key] = plan
+    plan.start_epoch(epoch, steps, rank)
+    dev = model.device
+    losses = torch.empty((steps, 2), dtype=torch.float32, device=dev)
+    subjects = torch.empty((steps, n), dtype=torch.int32, device=dev)
+    with torch.no_grad():
+        for i in range(steps):
+            plan.graph.replay()
+            ops.LAUNCHES[0] += plan.n_kernels
+            if not plan.optimizer_in_graph:
+                _optimizer_step(model, plan.flat, world_size, allreduce)
+            losses[i].copy_(plan.loss)
+            subjects[i].copy_(plan.record[:, 0])
+        model.invalidate_packed()
+    overflows = int(plan.pack_status[1].item())         # the one host read of the epoch
+    if overflows:
+        raise RuntimeError("%d of %d steps had more ground-truth boxes in a volume than max_boxes_per_volume=%d (or "
+                           "more connected components than that); their updates were skipped -- raise "
+                           "max_boxes_per_volume" % (overflows, steps, per_volume))
+    return losses, subjects
