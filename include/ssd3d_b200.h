@@ -265,19 +265,10 @@ int ssd3d_stem_conv_affine_simt(const void* x, int x_is_bf16, const void* w, con
 /* The same stem contract on the banded-B tcgen05 kernel (csrc/conv_stem_tz.cu): the W taps live in a Toeplitz B
  * operand, the A operand is the raw TMA'd input row (no per-voxel tap gather), 512 voxels per accumulator, epilogue
  * straight to global memory.  bf16 volumes, Cin <= 2, W % 8 == 0 (ssd3d_stem_tz_supported);
- * ssd3d_stem_conv_affine / .._bn_relu pick it by themselves when it applies (SSD3D_STEM_TZ=0 turns that off). */
+ * ssd3d_stem_conv_affine / .._bn_relu pick it by themselves when it applies and W % 64 == 0. */
 int ssd3d_stem_conv_affine_tz(const void* x, int x_is_bf16, const void* w, const float* scale, const float* shift,
                               void* y, int N, int Cin, int D, int H, int W, int stride_d, int relu, void* stream);
 int ssd3d_stem_tz_supported(int x_is_bf16, int Cin, int W);
-/* Stem + the depthwise conv of the first Block in ONE kernel (csrc/conv_stem_dw.cu; mobilenet.py:28-30 followed by
- * mobilenet.py:38,44 in eval mode): the stem activation (32 channels at half resolution, the largest tensor of the
- * network) stays in shared memory.  x as for the stem (bf16 only), w_stem (32, KPAD) bf16, w_dw (27, 32) bf16,
- * scale/shift = the two folded BatchNorms, y (N, Dd, Hd, Wd, 32) bf16 with Dd = ((D-1)/sd+1 - 1)/2 + 1 etc.
- * ssd3d_stem_dw_fused_supported: bf16 volumes, Cin <= 2, W = 128, even stem map along D and H. */
-int ssd3d_stem_dw_fused(const void* x, int x_is_bf16, const void* w_stem, const float* scale0, const float* shift0,
-                        const void* w_dw, const float* scale1, const float* shift1, void* y, int N, int Cin, int D,
-                        int H, int W, int stride_d, void* stream);
-int ssd3d_stem_dw_fused_supported(int x_is_bf16, int Cin, int D, int H, int W, int stride_d);
 /* The gather-based tcgen05 stem kernel (csrc/conv_stem_tc.cu) addressed explicitly: the kernel ssd3d_stem_conv_affine
  * uses for fp32 volumes and Cin > 2; SSD3D_ERR_UNSUPPORTED when ssd3d_stem_tc_supported says no. */
 int ssd3d_stem_conv_affine_tc(const void* x, int x_is_bf16, const void* w, const float* scale, const float* shift,

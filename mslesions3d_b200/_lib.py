@@ -69,8 +69,6 @@ SIGNATURES = {
     "ssd3d_stem_conv_affine_simt": (c_int, [P, c_int, P, P, P, P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P]),
     "ssd3d_stem_conv_affine_tz": (c_int, [P, c_int, P, P, P, P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P]),
     "ssd3d_stem_tz_supported": (c_int, [c_int, c_int, c_int]),
-    "ssd3d_stem_dw_fused": (c_int, [P, c_int, P, P, P, P, P, P, P, c_int, c_int, c_int, c_int, c_int, c_int, P]),
-    "ssd3d_stem_dw_fused_supported": (c_int, [c_int, c_int, c_int, c_int, c_int, c_int]),
     "ssd3d_stem_conv_affine_tc": (c_int, [P, c_int, P, P, P, P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P]),
     "ssd3d_dwconv3d_affine": (c_int, [P, P, P, P, P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P]),
     "ssd3d_dwconv3d_affine_direct": (c_int, [P, P, P, P, P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, P]),

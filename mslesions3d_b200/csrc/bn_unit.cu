@@ -677,7 +677,7 @@ cudaError_t launch_bn_cluster(const BnUnitParams& p, int K, cudaStream_t st) {
   cfg.stream = st;
   cudaLaunchAttribute attr[2];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
   attr[1].id = cudaLaunchAttributeClusterDimension;
   attr[1].val.clusterDim.x = (unsigned)K;
   attr[1].val.clusterDim.y = 1;
@@ -1031,15 +1031,11 @@ static int bn_launch_result(cudaError_t e) {
   return (int)e;
 }
 
-static const bool g_bn_cluster = [] { const char* e = getenv("SSD3D_BN_CLUSTER"); return !(e && e[0] == '0'); }();
-// SSD3D_BN_TILE=0: the two-barrier bn_unit_kernel for the larger maps (A/B measurements)
-static const bool g_bn_tile = [] { const char* e = getenv("SSD3D_BN_TILE"); return !(e && e[0] == '0'); }();
-
 extern "C" int ssd3d_bn_unit_supported(int64_t M, int C) {
   long long rpc;
   int R;
   if (M <= 0) return 0;
-  if (g_bn_cluster && bn_cluster_plan(M, C, &rpc, &R) > 0) return 1;
+  if (bn_cluster_plan(M, C, &rpc, &R) > 0) return 1;
   return bn_unit_plan(M, C, &rpc) > 0 ? 1 : 0;
 }
 
@@ -1056,7 +1052,7 @@ extern "C" int ssd3d_bn_unit_fwd(const void* z, int64_t M, int C, const float* g
   if (!z || !scale || !shift || !mean || !invstd || !workspace || !sync_words || M <= 0) return SSD3D_ERR_ARG;
   BnUnitParams p{};
   int R = 0;
-  const int K = g_bn_cluster ? bn_cluster_plan(M, C, &p.rows_per_cta, &R) : -1;
+  const int K = bn_cluster_plan(M, C, &p.rows_per_cta, &R);
   const int G = K > 0 ? 0 : bn_unit_plan(M, C, &p.rows_per_cta);
   if (G < 0 || workspace_bytes < (int64_t)G * 2 * C * 4) return SSD3D_ERR_ARG;
   p.z = static_cast<const bf16*>(z);
@@ -1073,14 +1069,12 @@ extern "C" int ssd3d_bn_unit_fwd(const void* z, int64_t M, int C, const float* g
     const cudaError_t e = launch_bn_cluster_r<0>(p, K, R, static_cast<cudaStream_t>(stream));
     return bn_launch_result(e);
   }
-  if (g_bn_tile) {
-    BnTileParams q{};
-    q.u = p;
-    const int GT = bn_tile_plan(M, C, &q);
-    if (GT > 0 && workspace_bytes >= (int64_t)GT * 128 * 4) {
-      const cudaError_t e = launch_bn_tile<0>(q, GT, static_cast<cudaStream_t>(stream));
-      return bn_launch_result(e);
-    }
+  BnTileParams q{};
+  q.u = p;
+  const int GT = bn_tile_plan(M, C, &q);
+  if (GT > 0 && workspace_bytes >= (int64_t)GT * 128 * 4) {
+    const cudaError_t e = launch_bn_tile<0>(q, GT, static_cast<cudaStream_t>(stream));
+    return bn_launch_result(e);
   }
   const cudaError_t e = launch_bn_unit<0>(p, G, static_cast<cudaStream_t>(stream));
   return bn_launch_result(e);
@@ -1095,7 +1089,7 @@ extern "C" int ssd3d_bn_unit_bwd(const void* z, const void* grad_a, int64_t M, i
     return SSD3D_ERR_ARG;
   BnUnitParams p{};
   int R = 0;
-  const int K = g_bn_cluster ? bn_cluster_plan(M, C, &p.rows_per_cta, &R) : -1;
+  const int K = bn_cluster_plan(M, C, &p.rows_per_cta, &R);
   const int G = K > 0 ? 0 : bn_unit_plan(M, C, &p.rows_per_cta);
   if (G < 0 || workspace_bytes < (int64_t)G * 2 * C * 4) return SSD3D_ERR_ARG;
   p.z = static_cast<const bf16*>(z);
@@ -1112,14 +1106,12 @@ extern "C" int ssd3d_bn_unit_bwd(const void* z, const void* grad_a, int64_t M, i
     const cudaError_t e = launch_bn_cluster_r<1>(p, K, R, static_cast<cudaStream_t>(stream));
     return bn_launch_result(e);
   }
-  if (g_bn_tile) {
-    BnTileParams q{};
-    q.u = p;
-    const int GT = bn_tile_plan(M, C, &q);
-    if (GT > 0 && workspace_bytes >= (int64_t)GT * 128 * 4) {
-      const cudaError_t e = launch_bn_tile<1>(q, GT, static_cast<cudaStream_t>(stream));
-      return bn_launch_result(e);
-    }
+  BnTileParams q{};
+  q.u = p;
+  const int GT = bn_tile_plan(M, C, &q);
+  if (GT > 0 && workspace_bytes >= (int64_t)GT * 128 * 4) {
+    const cudaError_t e = launch_bn_tile<1>(q, GT, static_cast<cudaStream_t>(stream));
+    return bn_launch_result(e);
   }
   const cudaError_t e = launch_bn_unit<1>(p, G, static_cast<cudaStream_t>(stream));
   return bn_launch_result(e);

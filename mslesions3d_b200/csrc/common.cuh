@@ -14,7 +14,6 @@
     if (e__ != cudaSuccess) return (int)e__;         \
   } while (0)
 
-#include <cstdlib>
 #include <utility>
 
 namespace ssd3d {
@@ -29,29 +28,14 @@ namespace ssd3d {
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 
-inline bool pdl_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("SSD3D_PDL");
-    v = (e && e[0] == '0') ? 0 : 1;
-  }
-  return v != 0;
-}
-
-// SMs a persistent kernel spreads over: all of them minus SSD3D_RESERVE_SMS (default 0).  Persistent CTAs hold
-// their SM for the whole kernel, so leaving a few SMs free lets the latency-bound kernels of OTHER in-flight
-// batches (sort / NMS / small heads: a handful of CTAs) start immediately instead of waiting for a slot.
+// SMs a persistent kernel spreads over: the device's SM count, read once.
 inline int persistent_sms() {
   static int n = 0;
   if (n == 0) {
     int dev = 0, sms = 0;
     cudaGetDevice(&dev);
     if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sms <= 0) sms = 148;
-    const char* e = getenv("SSD3D_RESERVE_SMS");
-    int r = e ? atoi(e) : 0;
-    if (r < 0) r = 0;
-    if (r > sms / 2) r = sms / 2;
-    n = sms - r;
+    n = sms;
   }
   return n;
 }
@@ -66,7 +50,7 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
   cfg.stream = st;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);

@@ -274,16 +274,9 @@ extern "C" int ssd3d_dwconv3d_affine(const void* x, const void* w, const float* 
   if (!x || !w || !scale || !shift || !y || N <= 0 || D <= 0 || H <= 0 || W <= 0) return SSD3D_ERR_ARG;
   if (C <= 0 || (C & 7)) return SSD3D_ERR_ARG;
   if (stride != 1 && stride != 2) return SSD3D_ERR_ARG;
-  static int use_tma = -1;
-  if (use_tma < 0) {
-    const char* e = getenv("SSD3D_DW_TMA");
-    use_tma = (e && e[0] == '0') ? 0 : 1;
-  }
-  if (use_tma) {
-    const int rc = ssd3d_dwconv3d_tma(x, w, scale, shift, y, N, C, D, H, W, stride, SSD3D_FLOOR(relu),
-                                      static_cast<cudaStream_t>(stream));
-    if (rc != SSD3D_ERR_UNSUPPORTED) return rc;
-  }
+  const int rc = ssd3d_dwconv3d_tma(x, w, scale, shift, y, N, C, D, H, W, stride, SSD3D_FLOOR(relu),
+                                    static_cast<cudaStream_t>(stream));
+  if (rc != SSD3D_ERR_UNSUPPORTED) return rc;
   return dwconv3d_direct(x, w, scale, shift, y, N, C, D, H, W, stride, relu, stream);
 }
 

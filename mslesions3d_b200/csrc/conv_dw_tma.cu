@@ -554,20 +554,13 @@ using namespace ssd3d;
 int ssd3d_dwconv3d_tma(const void* x, const void* w, const float* scale, const float* shift, void* y, int N, int C,
                        int D, int H, int W, int stride, float floor, cudaStream_t st) {
   const int Do = (D - 1) / stride + 1, Ho = (H - 1) / stride + 1, Wo = (W - 1) / stride + 1;
-  static int min_w = 0;
-  if (min_w == 0) {
-    const char* e = getenv("SSD3D_DW_TMA_MIN_W");
-    min_w = e ? atoi(e) : 8;
-    if (min_w < 8) min_w = 8;
-  }
-  if (C % DW_CB || Wo < min_w || Ho < 4 || Do < 4) return SSD3D_ERR_UNSUPPORTED;
+  if (C % DW_CB || Wo < 8 || Ho < 4 || Do < 4) return SSD3D_ERR_UNSUPPORTED;
   if ((reinterpret_cast<uintptr_t>(x) & 15) != 0) return SSD3D_ERR_UNSUPPORTED;
   DwTmaParams p{};
   p.N = N; p.C = C; p.D = D; p.H = H; p.W = W; p.Do = Do; p.Ho = Ho; p.Wo = Wo;
   p.w = static_cast<const __nv_bfloat16*>(w);
   p.scale = scale; p.shift = shift; p.y = static_cast<__nv_bfloat16*>(y); p.floor = floor;
-  static const bool deint = [] { const char* e = getenv("SSD3D_DW_S2_DEINTERLEAVE"); return !(e && e[0] == '0'); }();
-  if (stride == 2) return deint ? launch_dw_tma_s2(x, p, st) : launch_dw_tma<2, 2, 4, 4, 8>(x, p, st);
+  if (stride == 2) return launch_dw_tma_s2(x, p, st);
   return launch_dw_tma<1, 4, 4, 8, 8>(x, p, st);
 }
 

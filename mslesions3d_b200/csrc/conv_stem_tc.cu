@@ -736,15 +736,9 @@ extern "C" int ssd3d_stem_tz_supported(int x_is_bf16, int Cin, int W);
 // Which tcgen05 stem kernel ssd3d_stem_conv_affine picks: the banded-B kernel (conv_stem_tz.cu) when its 32-voxel row
 // slots are all full (W a multiple of 64: 43-44 us against 45.5 us for the gather kernel at the benchmark shape; both
 // sit on the mixed read/write HBM floor), the gather kernel otherwise (Wo = 48 wastes a third of the second slot:
-// 37-41 vs 37.3 us).  SSD3D_STEM_TZ=0 never, =1 whenever the kernel applies and Wo >= 24.
+// 37-41 vs 37.3 us).
 static bool stem_tz_wanted(int x_is_bf16, int Cin, int W) {
-  static int mode = -1;
-  if (mode < 0) {
-    const char* e = getenv("SSD3D_STEM_TZ");
-    mode = !e ? 2 : (e[0] == '0' ? 0 : 1);
-  }
-  if (mode == 0 || !ssd3d_stem_tz_supported(x_is_bf16, Cin, W)) return false;
-  return mode == 1 ? ((W - 1) / 2 + 1 >= 24) : (W % 64 == 0);
+  return ssd3d_stem_tz_supported(x_is_bf16, Cin, W) && W % 64 == 0;
 }
 
 extern "C" int ssd3d_stem_conv_affine_tc(const void* x, int x_is_bf16, const void* w, const float* scale,

@@ -270,16 +270,9 @@ extern "C" int ssd3d_pwconv_affine(const void* x, const void* w, const float* sc
   if (!x || !w || !scale || !shift || !y || M <= 0) return SSD3D_ERR_ARG;
   if (Cin <= 0 || (Cin % 32) || Cout <= 0 || (Cout % 16)) return SSD3D_ERR_ARG;
   {
-    static int use_persistent = -1;
-    if (use_persistent < 0) {
-      const char* e = getenv("SSD3D_PW_PERSISTENT");
-      use_persistent = (e && e[0] == '0') ? 0 : 1;
-    }
-    if (use_persistent) {
-      const int rc = ssd3d_pwconv_persistent(x, w, scale, shift, y, M, Cin, Cout, SSD3D_FLOOR(relu), nan_flag,
-                                             static_cast<cudaStream_t>(stream));
-      if (rc != SSD3D_ERR_UNSUPPORTED) return rc;
-    }
+    const int rc = ssd3d_pwconv_persistent(x, w, scale, shift, y, M, Cin, Cout, SSD3D_FLOOR(relu), nan_flag,
+                                           static_cast<cudaStream_t>(stream));
+    if (rc != SSD3D_ERR_UNSUPPORTED) return rc;
   }
   const int BK = (Cin % 64 == 0) ? 64 : 32;
   const long long m_tiles = (M + 127) / 128;

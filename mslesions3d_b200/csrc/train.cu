@@ -3,9 +3,10 @@
 //   * train-mode BatchNorm: per-channel batch statistics of a raw conv output (two-stage, deterministic),
 //     running-stat update, normalise + ReLU; and its backward (ReLU mask recomputed from the saved raw
 //     output, dgamma / dbeta reductions, dz)
-//   * weight gradients of the pointwise, head (3x3x3) and stem (3x3x3, NCDHW input) convolutions as ONE
-//     split-M implicit GEMM   dW[n][k] = sum_m dz[m][n] * im2col(x)[m][k]   on mma.sync bf16 tensor cores
-//     (operands are channels-last, i.e. M-major: fragments come from ldmatrix.trans), fixed-order reduction
+//   * weight gradients of the pointwise and stem (3x3x3, NCDHW input) convolutions as ONE split-M implicit GEMM
+//     dW[n][k] = sum_m dz[m][n] * im2col(x)[m][k]   on mma.sync bf16 tensor cores (operands are channels-last,
+//     i.e. M-major: fragments come from ldmatrix.trans), fixed-order reduction; the head (3x3x3) weight gradient
+//     in an activation-stationary form of the same contraction
 //   * data gradient of the head convs (transposed 3x3x3 conv, 16 -> C channels) as an mma.sync implicit GEMM
 //   * depthwise 3x3x3 data and weight gradients (HBM-bound CUDA-core kernels, 16-byte channel vectors)
 //   * packing of d(loss)/d(locs, scores) into the head's (voxel, 16) bf16 gradient rows
@@ -301,179 +302,6 @@ __global__ void __launch_bounds__(256) bn_relu_bwd_apply_kernel(const bf16* __re
 }
 
 // ------------------------------------------------------------------------------------------------
-// The same two "apply" passes with the cross-block finalize folded in (one launch less per BatchNorm pass, and the
-// single-CTA finalize kernels -- pure latency on the critical chain: 28 launches x ~7 us per step -- are gone):
-// EVERY CTA first sums the column partials of all C channels itself -- fp64, fixed order: lane l of a channel adds
-// blocks l, l+L, ..., the lanes are combined in order, so all CTAs (and all runs) get bit-identical values -- keeps
-// the per-channel constants in shared memory, and CTA 0 also writes them out (BN state for the backward pass,
-// running statistics / the parameter gradients).  colreduce_plan_fused keeps B*C small enough for that prologue
-// to cost ~2 us.
-// ------------------------------------------------------------------------------------------------
-constexpr int FIN_MAX_C = 512;
-
-// -> fin[c][0] = sum_b partial[b][c], fin[c][1] = sum_b partial[b][C + c]   (doubles, all C channels)
-__device__ __forceinline__ void cta_colpartials_sum(const float* __restrict__ partial, int B, int C,
-                                                    double (*red)[2], double (*fin)[2]) {
-  const int L = (C >= 256) ? 1 : 256 / C;              // block lanes per channel
-  for (int it = threadIdx.x; it < C * L; it += 256) {
-    const int c = it % C, l = it / C;
-    double ls = 0.0, lq = 0.0;
-    int b = l;
-    for (; b + 7 * L < B; b += 8 * L) {                // 16 independent loads in flight, then the ordered adds
-      float a0[8], a1[8];
-#pragma unroll
-      for (int u = 0; u < 8; ++u) {
-        a0[u] = partial[(size_t)(b + u * L) * 2 * C + c];
-        a1[u] = partial[(size_t)(b + u * L) * 2 * C + C + c];
-      }
-#pragma unroll
-      for (int u = 0; u < 8; ++u) { ls += (double)a0[u]; lq += (double)a1[u]; }
-    }
-    for (; b < B; b += L) {
-      ls += (double)partial[(size_t)b * 2 * C + c];
-      lq += (double)partial[(size_t)b * 2 * C + C + c];
-    }
-    red[it][0] = ls;
-    red[it][1] = lq;
-  }
-  __syncthreads();
-  for (int c = threadIdx.x; c < C; c += 256) {
-    double s = 0.0, q = 0.0;
-    for (int l = 0; l < L; ++l) { s += red[l * C + c][0]; q += red[l * C + c][1]; }
-    fin[c][0] = s;
-    fin[c][1] = q;
-  }
-  __syncthreads();
-}
-
-__global__ void __launch_bounds__(256) bn_apply_relu_fin_kernel(const bf16* __restrict__ z,
-                                                                const float* __restrict__ partial, int B, int C,
-                                                                long long M, const float* __restrict__ gamma,
-                                                                const float* __restrict__ beta, float eps,
-                                                                float momentum, float* __restrict__ running_mean,
-                                                                float* __restrict__ running_var,
-                                                                long long* __restrict__ num_batches_tracked,
-                                                                float* __restrict__ scale_out,
-                                                                float* __restrict__ shift_out,
-                                                                float* __restrict__ mean_out,
-                                                                float* __restrict__ invstd_out, bf16* __restrict__ a,
-                                                                long long total_vec, int* nan_flag) {
-  __shared__ double red[FIN_MAX_C][2];
-  __shared__ double fin[FIN_MAX_C][2];
-  __shared__ float s_scale[FIN_MAX_C], s_shift[FIN_MAX_C];
-  pdl_wait();
-  pdl_launch_dependents();
-  cta_colpartials_sum(partial, B, C, red, fin);
-  for (int c = threadIdx.x; c < C; c += 256) {
-    const double mu = fin[c][0] / (double)M;
-    double var = fin[c][1] / (double)M - mu * mu;
-    if (var < 0.0) var = 0.0;
-    const float istd = (float)(1.0 / sqrt(var + (double)eps));
-    const float ga = gamma ? gamma[c] : 1.f, be = beta ? beta[c] : 0.f;
-    const float sc = ga * istd;
-    const float sh = be - (float)mu * sc;
-    s_scale[c] = sc;
-    s_shift[c] = sh;
-    if (blockIdx.x == 0) {
-      scale_out[c] = sc;
-      shift_out[c] = sh;
-      mean_out[c] = (float)mu;
-      invstd_out[c] = istd;
-      if (running_mean && running_var) {
-        const double unbiased = (M > 1) ? var * (double)M / (double)(M - 1) : var;
-        running_mean[c] = (float)((1.0 - (double)momentum) * (double)running_mean[c] + (double)momentum * mu);
-        running_var[c] = (float)((1.0 - (double)momentum) * (double)running_var[c] + (double)momentum * unbiased);
-      }
-    }
-  }
-  if (num_batches_tracked && blockIdx.x == 0 && threadIdx.x == 0) *num_batches_tracked += 1;
-  __syncthreads();
-  if (!a) return;
-  const int CV = C >> 3;
-  bool bad = false;
-  const long long stride = (long long)gridDim.x * blockDim.x;
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total_vec; i += 2 * stride) {
-    const long long i1 = i + stride;
-    const uint4 z0 = ld_nc16(z + i * 8);
-    uint4 z1 = make_uint4(0u, 0u, 0u, 0u);
-    if (i1 < total_vec) z1 = ld_nc16(z + i1 * 8);
-#pragma unroll
-    for (int k = 0; k < 2; ++k) {
-      const long long idx = k ? i1 : i;
-      if (idx >= total_vec) break;
-      const int c0 = (int)(idx % CV) << 3;
-      float zf[8], o[8];
-      unpack8f(k ? z1 : z0, zf);
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        o[j] = relu_nan(__fadd_rn(__fmul_rn(zf[j], s_scale[c0 + j]), s_shift[c0 + j]));
-        bad |= (o[j] != o[j]);
-      }
-      *reinterpret_cast<uint4*>(a + idx * 8) = pack8f(o);
-    }
-  }
-  if (bad && nan_flag) atomicOr(nan_flag, SSD3D_NAN_BACKBONE);
-}
-
-__global__ void __launch_bounds__(256) bn_relu_bwd_apply_fin_kernel(const bf16* __restrict__ z, const bf16* g,
-                                                                    const float* __restrict__ partial, int B, int C,
-                                                                    const float* __restrict__ scale,
-                                                                    const float* __restrict__ shift,
-                                                                    const float* __restrict__ mean,
-                                                                    const float* __restrict__ invstd,
-                                                                    float* __restrict__ dgamma,
-                                                                    float* __restrict__ dbeta, float inv_m, bf16* dz,
-                                                                    long long total_vec) {
-  __shared__ double red[FIN_MAX_C][2];
-  __shared__ double fin[FIN_MAX_C][2];
-  __shared__ float s_sc[FIN_MAX_C], s_sh[FIN_MAX_C], s_ka[FIN_MAX_C], s_kb[FIN_MAX_C];
-  pdl_wait();
-  pdl_launch_dependents();
-  cta_colpartials_sum(partial, B, C, red, fin);
-  for (int c = threadIdx.x; c < C; c += 256) {
-    const float db = (float)fin[c][0], dg = (float)fin[c][1];
-    if (blockIdx.x == 0) { dbeta[c] = db; dgamma[c] = dg; }
-    // dz = sc*(dy - dbeta/M - xhat*dgamma/M) with xhat = (z - mu)*invstd, regrouped as sc*dy + A + z*B
-    const float sc = scale[c], is = invstd[c], mu = mean[c];
-    const float t = sc * is * dg * inv_m;
-    s_sc[c] = sc;
-    s_sh[c] = shift[c];
-    s_kb[c] = -t;
-    s_ka[c] = fmaf(mu, t, -(sc * db * inv_m));
-  }
-  __syncthreads();
-  const int CV = C >> 3;
-  const long long stride = (long long)gridDim.x * blockDim.x;
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total_vec; i += 2 * stride) {
-    const long long i1 = i + stride;
-    const bool two = i1 < total_vec;
-    const uint4 z0 = ld_nc16(z + i * 8);
-    const uint4 g0 = *reinterpret_cast<const uint4*>(g + i * 8);
-    uint4 z1 = make_uint4(0u, 0u, 0u, 0u), g1 = make_uint4(0u, 0u, 0u, 0u);
-    if (two) {
-      z1 = ld_nc16(z + i1 * 8);
-      g1 = *reinterpret_cast<const uint4*>(g + i1 * 8);
-    }
-#pragma unroll
-    for (int k = 0; k < 2; ++k) {
-      if (k && !two) break;
-      const long long idx = k ? i1 : i;
-      const int c0 = (int)(idx % CV) << 3;
-      float zf[8], gf[8], o[8];
-      unpack8f(k ? z1 : z0, zf);
-      unpack8f(k ? g1 : g0, gf);
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        const float pre = __fadd_rn(__fmul_rn(zf[j], s_sc[c0 + j]), s_sh[c0 + j]);
-        const float dy = (pre > 0.f) ? gf[j] : 0.f;
-        o[j] = fmaf(zf[j], s_kb[c0 + j], fmaf(s_sc[c0 + j], dy, s_ka[c0 + j]));
-      }
-      *reinterpret_cast<uint4*>(dz + idx * 8) = pack8f(o);
-    }
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
 // mma.sync helpers (bf16 x bf16 -> fp32, m16n8k16)
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ void ldsm_x4(uint32_t addr, uint32_t (&r)[4]) {
@@ -495,7 +323,6 @@ __device__ __forceinline__ void mma_bf16(float (&d)[4], const uint32_t (&a)[4], 
 // ------------------------------------------------------------------------------------------------
 // Weight gradient as a split-M implicit GEMM:  dW[n][k] = sum_m dz[m][n] * X[m][k]
 //   MODE 0 pointwise : X[m][k] = x[m*C + k], zero for k >= C                        (K = Cin rounded up to 64)
-//   MODE 1 head 3^3  : k = tap*C + c, X = x[voxel(m) + (tap offsets - 1)][c], zero outside the map
 //   MODE 2 stem 3^3  : k = ci*27 + tap, X = bf16(x_ncdhw[n][ci][sd*do+kd-1][2*ho+kh-1][2*wo+kw-1])
 // CTA: 128 threads, output tile NT (n) x 64 (k), rows [split*rows_per_split, ...) in chunks of 64.
 // Both operands sit in smem as [m][n] / [m][k] (M-major); A (= dz^T) and B fragments are ldmatrix.trans.
@@ -507,8 +334,8 @@ struct WgradParams {
   int K;                      // padded to a multiple of 64
   const void* x;
   int x_is_bf16;              // stem only
-  int C;                      // pointwise: Cin (row pitch); head: channels
-  int N, D, H, W;             // head: feature map; stem: input volume
+  int C;                      // pointwise: Cin (row pitch)
+  int N, D, H, W;             // stem: input volume
   int Do, Ho, Wo, sd, Cin;    // stem
   long long rows_per_split;
   int n_pad;                  // rows of one partial slab (multiple of NT)
@@ -538,14 +365,8 @@ __global__ void __launch_bounds__(128) wgrad_kernel(const WgradParams p) {
   // ---- per-thread constants of the X gather ----
   const int xcc = tid % XCH;          // 16-byte chunk (8 k values) inside the KT-wide k tile
   const int xrow0 = tid / XCH;        // rows xrow0 + XRS*i, i < XPT
-  int tap_d = 0, tap_h = 0, tap_w = 0, cbase = 0;       // MODE 1
   int e_off[8];                                          // MODE 2: per element (ci, tap) -> offset, or -1
   int e_kd[8], e_kh[8], e_kw[8];
-  if (MODE == 1) {
-    const int tap = k0 / p.C;
-    cbase = k0 - tap * p.C + xcc * 8;
-    tap_d = tap / 9 - 1; tap_h = (tap / 3) % 3 - 1; tap_w = tap % 3 - 1;
-  }
   if (MODE == 2) {
 #pragma unroll
     for (int e = 0; e < 8; ++e) {
@@ -573,13 +394,6 @@ __global__ void __launch_bounds__(128) wgrad_kernel(const WgradParams p) {
       if (m >= m_end) continue;
       if (MODE == 0) {
         if (k0 + xcc * 8 < p.C) xr[i] = ld_nc16(static_cast<const bf16*>(p.x) + m * p.C + k0 + xcc * 8);
-      } else if (MODE == 1) {
-        long long t = m;
-        const int w = (int)(t % p.W) + tap_w; t /= p.W;
-        const int h = (int)(t % p.H) + tap_h; t /= p.H;
-        const int d = (int)(t % p.D) + tap_d; t /= p.D;
-        if ((unsigned)w < (unsigned)p.W && (unsigned)h < (unsigned)p.H && (unsigned)d < (unsigned)p.D)
-          xr[i] = ld_nc16(static_cast<const bf16*>(p.x) + ((((long long)t * p.D + d) * p.H + h) * p.W + w) * p.C + cbase);
       } else {
         long long t = m;
         const int wo = (int)(t % p.Wo); t /= p.Wo;
@@ -642,23 +456,6 @@ __global__ void __launch_bounds__(128) wgrad_kernel(const WgradParams p) {
       }
     }
   }
-  if (MODE == 1) {
-    // head: the slab is laid out like the conv weight itself, [n][c][tap], so that the final sum is a plain
-    // contiguous reduction (k = tap*C + c: this CTA's 64 k values share one tap)
-    const int tap = k0 / p.C, cb = k0 - tap * p.C + warp * 8 * NB;
-    float* out = p.partial + ((size_t)blockIdx.z * p.n_pad + n0) * p.K;
-#pragma unroll
-    for (int a = 0; a < NT / 16; ++a)
-#pragma unroll
-      for (int b = 0; b < NB; ++b) {
-        const int n = a * 16 + (lane >> 2), c = cb + b * 8 + (lane & 3) * 2;
-        out[((size_t)n * p.C + c) * 27 + tap] = acc[a][b][0];
-        out[((size_t)n * p.C + c + 1) * 27 + tap] = acc[a][b][1];
-        out[((size_t)(n + 8) * p.C + c) * 27 + tap] = acc[a][b][2];
-        out[((size_t)(n + 8) * p.C + c + 1) * 27 + tap] = acc[a][b][3];
-      }
-    return;
-  }
   float* out = p.partial + ((size_t)blockIdx.z * p.n_pad + n0) * p.K + k0 + warp * 8 * NB;
 #pragma unroll
   for (int a = 0; a < NT / 16; ++a)
@@ -676,7 +473,8 @@ __global__ void __launch_bounds__(128) wgrad_kernel(const WgradParams p) {
 // is loaded ONCE and contracted against G[u][j*16 + n] = dO[u - off(kd, j)][n], the 9 (kh, kw) shifts of the
 // 16-column gradient rows (32 bytes each, zero outside the map, L1/L2 resident), instead of gathering the 27
 // shifted activation tiles.  CTA = (64-channel tile, kd, voxel split); cp.async double buffering; warp w owns
-// channels 16w..16w+15 x 144 columns (72 accumulator registers).  Slab layout [split][16][C][27] as before.
+// channels 16w..16w+15 x 144 columns (72 accumulator registers).  Slab layout [split][16][C][27], the layout of
+// the conv weight rows, so that the final sum is a plain contiguous reduction.
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ void cp_async16(uint32_t dst, const void* src, bool valid) {
   const int sz = valid ? 16 : 0;
@@ -1512,17 +1310,6 @@ static int colreduce_plan(long long M, int C, int* threads, long long* rows_per_
 
 extern "C" int64_t ssd3d_bn_workspace_bytes(int C) { return (int64_t)COLRED_MAX_BLOCKS * 2 * C * 4; }
 
-// the apply kernels finalize in every CTA (see above): keep blocks x channels bounded so that this costs ~2 us
-// MEASURED (B200, C3 step): 1.82 ms with the fused finalize against 1.59 ms with the separate single-CTA finalize
-// kernels -- every one of the ~1000 apply CTAs re-reads B x 2C partials from L2 (up to 150 KB each) and the
-// reduction runs with fewer blocks -- so it is OFF by default (SSD3D_BN_FUSED_FINALIZE=1 switches it on).
-static const bool g_bn_fused_finalize = [] { const char* e = getenv("SSD3D_BN_FUSED_FINALIZE"); return e && e[0] == '1'; }();
-static int colreduce_cap_fused(int C, int cap) {
-  int b = 18944 / (C > 0 ? C : 1);
-  if (b < 16) b = 16;
-  return b < cap ? b : cap;
-}
-
 extern "C" int ssd3d_bn_train_fwd(const void* z, int64_t M, int C, const float* gamma, const float* beta, float eps,
                                   float momentum, float* running_mean, float* running_var,
                                   int64_t* num_batches_tracked, float* scale, float* shift, float* mean, float* invstd,
@@ -1530,23 +1317,13 @@ extern "C" int ssd3d_bn_train_fwd(const void* z, int64_t M, int C, const float* 
   if (!z || !scale || !shift || !mean || !invstd || !workspace || M <= 0) return SSD3D_ERR_ARG;
   int threads;
   long long rpb;
-  const bool fused = g_bn_fused_finalize && C <= FIN_MAX_C;
-  const int B = colreduce_plan(M, C, &threads, &rpb, fused ? colreduce_cap_fused(C, COLRED_MAX_BLOCKS) : COLRED_MAX_BLOCKS);
+  const int B = colreduce_plan(M, C, &threads, &rpb);
   if (B < 0 || workspace_bytes < (int64_t)B * 2 * C * 4) return SSD3D_ERR_ARG;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   float* partial = static_cast<float*>(workspace);
   const bf16* zp = static_cast<const bf16*>(z);
   SSD3D_LAUNCH_PDL(colreduce_kernel<0>, dim3(B), dim3(threads), 0, st, zp, (const bf16*)nullptr, (const float*)nullptr,
                    (const float*)nullptr, (const float*)nullptr, (const float*)nullptr, (long long)M, C, rpb, partial);
-  if (fused) {
-    const long long total_vec = (long long)M * (C / 8);
-    const int grid = a ? grid_for((total_vec + 1) / 2, 256, 148 * 8) : 1;
-    SSD3D_LAUNCH_PDL(bn_apply_relu_fin_kernel, dim3(grid), dim3(256), 0, st, zp, (const float*)partial, B, C, (long long)M,
-                     gamma, beta, eps, momentum, running_mean, running_var,
-                     reinterpret_cast<long long*>(num_batches_tracked), scale, shift, mean, invstd,
-                     static_cast<bf16*>(a), total_vec, nan_flag);
-    return SSD3D_OK;
-  }
   SSD3D_LAUNCH_PDL(bn_finalize_fwd_kernel, dim3((C + 31) / 32), dim3(1024), 0, st, (const float*)partial, B, C,
                    (long long)M, gamma, beta, eps, momentum, running_mean, running_var, scale, shift, mean, invstd,
                    reinterpret_cast<long long*>(num_batches_tracked));
@@ -1567,8 +1344,7 @@ extern "C" int ssd3d_bn_relu_bwd(const void* z, const void* grad_a, int64_t M, i
   long long rpb;
   // the backward reduction holds 84 registers: three CTAs per SM are resident, so at most 3 x 148 blocks (a fourth
   // quarter of the grid would run as a second, mostly empty wave)
-  const bool fused = g_bn_fused_finalize && C <= FIN_MAX_C;
-  const int B = colreduce_plan(M, C, &threads, &rpb, fused ? colreduce_cap_fused(C, 444) : 444);
+  const int B = colreduce_plan(M, C, &threads, &rpb, 444);
   if (B < 0 || workspace_bytes < (int64_t)B * 2 * C * 4) return SSD3D_ERR_ARG;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   float* partial = static_cast<float*>(workspace);
@@ -1576,13 +1352,6 @@ extern "C" int ssd3d_bn_relu_bwd(const void* z, const void* grad_a, int64_t M, i
   const bf16* gp = static_cast<const bf16*>(grad_a);
   SSD3D_LAUNCH_PDL(colreduce_kernel<1>, dim3(B), dim3(threads), 0, st, zp, gp, scale, shift, mean, invstd, (long long)M,
                    C, rpb, partial);
-  if (fused) {
-    const long long total_vec = (long long)M * (C / 8);
-    SSD3D_LAUNCH_PDL(bn_relu_bwd_apply_fin_kernel, dim3(grid_for((total_vec + 1) / 2, 256, 148 * 8)), dim3(256), 0, st, zp,
-                     gp, (const float*)partial, B, C, scale, shift, mean, invstd, dgamma, dbeta,
-                     (float)(1.0 / (double)M), static_cast<bf16*>(dz), total_vec);
-    return SSD3D_OK;
-  }
   SSD3D_LAUNCH_PDL(bn_finalize_bwd_kernel, dim3((C + 31) / 32), dim3(1024), 0, st, (const float*)partial, B, C, dgamma,
                    dbeta);
   const long long total_vec = (long long)M * (C / 8);
@@ -1638,8 +1407,6 @@ int head_wgrad_tc_launch(const void* dO16, const void* x, int N, int C, int D, i
 int head_dgrad_tc_launch(const void* dO, const void* w, const void* addend, void* dx, int N, int C, int D, int H, int W,
                          int groups, cudaStream_t st);
 }
-// SSD3D_WGRAD_TC=0 keeps the mma.sync kernel (A/B measurements, and the shapes the tcgen05 tiling does not take)
-static const bool g_wgrad_tc = [] { const char* e = getenv("SSD3D_WGRAD_TC"); return !(e && e[0] == '0'); }();
 
 extern "C" int ssd3d_pwconv_wgrad(const void* dz, const void* x, int64_t M, int Cin, int Cout, float* dw,
                                   void* workspace, int64_t workspace_bytes, void* stream) {
@@ -1647,7 +1414,7 @@ extern "C" int ssd3d_pwconv_wgrad(const void* dz, const void* x, int64_t M, int 
   if (Cin <= 0 || (Cin % 32) || Cout <= 0 || (Cout % 64)) return SSD3D_ERR_ARG;
   if (workspace_bytes < ssd3d_wgrad_workspace_bytes(M, Cout, Cin)) return SSD3D_ERR_ARG;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (g_wgrad_tc && workspace_bytes >= wgrad_tc_workspace_bytes(M, Cin, Cout)) {
+  if (workspace_bytes >= wgrad_tc_workspace_bytes(M, Cin, Cout)) {
     const int S = wgrad_tc_launch(dz, x, M, Cin, Cout, dw, static_cast<float*>(workspace), st);
     if (S == 1) return SSD3D_OK;
     if (S > 1)
@@ -1694,42 +1461,26 @@ extern "C" int ssd3d_head_wgrad(const void* dO, const void* x, int N, int C, int
   const long long M = (long long)N * D * H * W;
   if (workspace_bytes < ssd3d_wgrad_workspace_bytes(M, 16, 27 * C)) return SSD3D_ERR_ARG;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  static const bool use_g = [] { const char* e = getenv("SSD3D_HEAD_WGRAD_G"); return !(e && e[0] == '0'); }();
   const int groups = (n_loc + n_cls + 15) / 16;      // 16 output columns per pass (dO is (groups, M, 16))
   for (int g = 0; g < groups; ++g) {
     const bf16* dOg = static_cast<const bf16*>(dO) + (size_t)g * M * 16;
-    if (g_wgrad_tc) {
-      const int rc = head_wgrad_tc_launch(dOg, x, N, C, D, H, W, g, n_loc, n_cls, dw_loc, dw_cls,
-                                          static_cast<float*>(workspace), workspace_bytes, st);
-      if (rc == 0) continue;
-      if (rc < -1) return SSD3D_ERR_ARG;    // -1: no 64-voxel box fits this map -> mma.sync kernel below
-    }
-    if (use_g) {
-      HeadWgradParams q{};
-      q.dO = dOg; q.x = static_cast<const bf16*>(x);
-      q.N = N; q.D = D; q.H = H; q.W = W; q.C = C; q.M = M;
-      const long long chunks = (M + 63) / 64;
-      const int S0 = head_wgrad_splits(M, C);
-      q.chunks_per_split = (int)((chunks + S0 - 1) / S0);
-      const int S = (int)((chunks + q.chunks_per_split - 1) / q.chunks_per_split);
-      q.partial = static_cast<float*>(workspace);
-      const size_t smem = (size_t)2 * 64 * (HW_XP + HW_GP) * 2;
-      cudaError_t e = cudaFuncSetAttribute(head_wgrad_g_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-      if (e != cudaSuccess) return (int)e;
-      SSD3D_LAUNCH_PDL(head_wgrad_g_kernel, dim3((unsigned)(C / 64), 3u, (unsigned)S), dim3(128), smem, st, q);
-      if (const int rc_s = head_wgrad_scatter(q.partial, S, C, g, n_loc, n_cls, dw_loc, dw_cls, st)) return rc_s;
-      continue;
-    }
-    WgradParams p{};
-    p.dz = dOg; p.ldz = 16; p.M = M;
-    p.K = 27 * C;
-    p.x = x; p.C = C; p.N = N; p.D = D; p.H = H; p.W = W; p.n_pad = 16;
-    p.partial = static_cast<float*>(workspace);
-    int S = 0;
-    const int rc = run_wgrad<16, 1, 64>(p, 16, st, &S);
-    if (rc) return rc;
-    // slabs are [16][C][27] = the layout of the conv weight rows of this group
-    if (const int rc_s = head_wgrad_scatter((const float*)p.partial, S, C, g, n_loc, n_cls, dw_loc, dw_cls, st)) return rc_s;
+    const int rc = head_wgrad_tc_launch(dOg, x, N, C, D, H, W, g, n_loc, n_cls, dw_loc, dw_cls,
+                                        static_cast<float*>(workspace), workspace_bytes, st);
+    if (rc == 0) continue;
+    if (rc < -1) return SSD3D_ERR_ARG;    // -1: no 64-voxel box fits this map -> mma.sync kernel below
+    HeadWgradParams q{};
+    q.dO = dOg; q.x = static_cast<const bf16*>(x);
+    q.N = N; q.D = D; q.H = H; q.W = W; q.C = C; q.M = M;
+    const long long chunks = (M + 63) / 64;
+    const int S0 = head_wgrad_splits(M, C);
+    q.chunks_per_split = (int)((chunks + S0 - 1) / S0);
+    const int S = (int)((chunks + q.chunks_per_split - 1) / q.chunks_per_split);
+    q.partial = static_cast<float*>(workspace);
+    const size_t smem = (size_t)2 * 64 * (HW_XP + HW_GP) * 2;
+    cudaError_t e = cudaFuncSetAttribute(head_wgrad_g_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return (int)e;
+    SSD3D_LAUNCH_PDL(head_wgrad_g_kernel, dim3((unsigned)(C / 64), 3u, (unsigned)S), dim3(128), smem, st, q);
+    if (const int rc_s = head_wgrad_scatter(q.partial, S, C, g, n_loc, n_cls, dw_loc, dw_cls, st)) return rc_s;
   }
   return SSD3D_OK;
 }
@@ -1776,8 +1527,7 @@ extern "C" int ssd3d_stem_wgrad(const void* dz, const void* x, int x_is_bf16, in
   const int K = (27 * Cin <= 32) ? 32 : (27 * Cin + 63) / 64 * 64;     // one 32-wide k tile for Cin = 1
   if (workspace_bytes < ssd3d_wgrad_workspace_bytes(M, 32, 27 * Cin)) return SSD3D_ERR_ARG;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  static const bool use_tiles = [] { const char* e = getenv("SSD3D_STEM_WGRAD_TILES"); return !(e && e[0] == '0'); }();
-  if (use_tiles && M >= 128 * 148) {
+  if (M >= 128 * 148) {
     // halo tiles through TMA + im2col in shared memory (the forward stem's gather), one slab per persistent CTA
     const int kp = (27 * Cin <= 64) ? 64 : 128;
     const int max_slabs = (int)std::min<long long>(workspace_bytes / (32ll * kp * 4), 4096);
@@ -1838,11 +1588,9 @@ extern "C" int ssd3d_head_dgrad(const void* dO, const void* w, const void* adden
   if (C <= 0 || (C % 64) || n_cols <= 0 || n_cols > 256) return SSD3D_ERR_UNSUPPORTED;
   const long long M = (long long)N * D * H * W;
   const int groups = (n_cols + 15) / 16;
-  if (g_wgrad_tc) {
-    const int rc = head_dgrad_tc_launch(dO, w, addend, dx, N, C, D, H, W, groups, static_cast<cudaStream_t>(stream));
-    if (rc == 0) return SSD3D_OK;
-    if (rc < -1) return SSD3D_ERR_ARG;      // -1: no 128-voxel box fits this map -> mma.sync kernel below
-  }
+  const int rc = head_dgrad_tc_launch(dO, w, addend, dx, N, C, D, H, W, groups, static_cast<cudaStream_t>(stream));
+  if (rc == 0) return SSD3D_OK;
+  if (rc < -1) return SSD3D_ERR_ARG;      // -1: no 128-voxel box fits this map -> mma.sync kernel below
   const size_t smem = (size_t)(27 * 16 * 72 + 2 * 64 * 24) * 2;
   cudaError_t e = cudaFuncSetAttribute(head_dgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
@@ -1872,7 +1620,7 @@ extern "C" int ssd3d_dwconv3d_dgrad(const void* dz, const void* w, void* dx, int
   if (stride == 1) {
     SSD3D_LAUNCH_PDL(dw_dgrad_kernel<1>, dim3(blocks), dim3(256), 0, st, gp, wp, static_cast<bf16*>(dx), N, C, D, H, W,
                      Do, Ho, Wo, total);
-  } else if (C <= 256 && !(getenv("SSD3D_DW_DGRAD_BLOCK") && getenv("SSD3D_DW_DGRAD_BLOCK")[0] == '0')) {
+  } else if (C <= 256) {
     const int Md = (D + 1) / 2, Mh = (H + 1) / 2, Mw = (W + 1) / 2;
     const long long tot = (long long)N * Md * Mh * Mw * (C / 8);
     SSD3D_LAUNCH_PDL(dw_dgrad_s2_block_kernel, dim3((unsigned)((tot + 255) / 256)), dim3(256), (size_t)27 * C * 4, st, gp,
@@ -1894,9 +1642,8 @@ static int dw_wgrad_plan(long long Mo, int C, int* threads, int* G, long long* v
   *threads = CV * 3 * (*G);
   // voxels per voxel lane: the loop over them is serial (one L2 round trip + ~350 instructions each, 1-2 warps per
   // scheduler), so small maps get as few as 2 -- ~1.5 CTAs per SM -- and pay with more slabs; large ones 8
-  static const int vpl_env = [] { const char* e = getenv("SSD3D_DW_WGRAD_VPL"); return e ? atoi(e) : 0; }();
-  long long vpl = vpl_env > 0 ? vpl_env : Mo / ((long long)(*G) * 222);
-  if (vpl_env <= 0) vpl = vpl < 2 ? 2 : (vpl > 8 ? 8 : vpl);
+  long long vpl = Mo / ((long long)(*G) * 222);
+  vpl = vpl < 2 ? 2 : (vpl > 8 ? 8 : vpl);
   long long B = (Mo + (*G) * vpl - 1) / ((*G) * vpl);       // >= vpl voxels per voxel lane
   if (B > 592) B = 592;
   if (B < 1) B = 1;

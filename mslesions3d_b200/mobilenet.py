@@ -15,8 +15,6 @@ stand-alone there too, mobilenet.py:34-49) each module is one autograd node over
 """
 from __future__ import annotations
 
-import os
-
 import torch
 import torch.nn as nn
 
@@ -35,21 +33,6 @@ config_mobilenet = [32,
 MOBILENET_CONFIGS = {
     "mobilenet": config_mobilenet
 }
-
-
-# fused depthwise -> pointwise Block kernel (csrc/conv_dwpw.cu) for the shapes it is built for.  FUSE_DWPW is a bit
-# mask over the depthwise channel count of the block (1: 32 ch = f1, 2: 64 ch = f2, 4: 128 ch = f3); 0 runs the two
-# stand-alone kernels everywhere.  Measured on B200 at the benchmark size (profiles/r02_block_fused.md): alone,
-# every fused block beats its two kernels (f1 41 vs 47, f2 16.5 vs 20.6, f3 18.8 vs 22.8 us) and f1 keeps 33.6 MB
-# per step out of HBM -- so eager calls and the lone ``predict_step`` (latency) fuse all three -- but in the
-# 6-deep ``predict_batches`` pipeline (throughput) the fused CTAs own their SM (200 KB of shared memory) while the
-# stand-alone pointwise GEMMs they replace run underneath other batches' kernels: there the plans are captured
-# unfused (LSSD3D.fuse_blocks_pipeline).  SSD3D_FUSE_DWPW / SSD3D_FUSE_DWPW_PIPELINE override the two masks.
-FUSE_DWPW = [int(os.environ.get("SSD3D_FUSE_DWPW", "7"))]
-
-
-def _fuse_bit(cin: int) -> int:
-    return {32: 1, 64: 2, 128: 4}.get(int(cin), 0)
 
 
 def _versions(*tensors):
@@ -126,14 +109,13 @@ class Block(nn.Module):
             self._packed_key = key
         return self._packed
 
-    def pointwise_only(self, x):
-        """conv2 + bn2 + ReLU on an activation that already went through conv1 + bn1 + ReLU (the fused stem +
-        depthwise kernel of the inference plan produced it)."""
-        _, _, _, wp, s2, b2 = self._pack()
-        flag = self.nan_flag if self.nan_flag is not None else torch.zeros((1,), dtype=torch.int32, device=x.device)
-        return ops.pwconv_bn_relu(x, wp, s2, b2, flag)
-
-    def forward(self, x):
+    def forward(self, x, fuse: bool = True):
+        """``fuse``: run the shapes the fused depthwise -> pointwise kernel (csrc/conv_dwpw.cu) is built for as that one
+        kernel.  Measured on B200 at the benchmark size (profiles/r02_block_fused.md): alone, every fused block beats
+        its two kernels (f1 41 vs 47, f2 16.5 vs 20.6, f3 18.8 vs 22.8 us) and f1 keeps 33.6 MB per step out of HBM,
+        so eager calls and the lone ``predict_step`` (latency) fuse.  In the 6-deep ``predict_batches`` pipeline
+        (throughput) the fused CTAs own their SM (200 KB of shared memory) while the stand-alone pointwise GEMMs they
+        replace run underneath other batches' kernels: there the plans pass False."""
         s = _stride3(self.conv1.stride)
         if s[0] != s[1] or s[1] != s[2] or s[0] not in (1, 2):
             raise NotImplementedError("depthwise kernel is built for isotropic stride 1 or 2 (mobilenet.py:13-20)")
@@ -143,8 +125,7 @@ class Block(nn.Module):
         wd, s1, b1, wp, s2, b2 = self._pack()
         own_flag = self.nan_flag is None
         flag = torch.zeros((1,), dtype=torch.int32, device=x.device) if own_flag else self.nan_flag
-        if (int(FUSE_DWPW[0]) & _fuse_bit(x.shape[1])) and x.is_cuda and x.dim() == 5 and \
-                ops.block_fused_supported(x, wp.shape[0], s[0]):
+        if fuse and x.is_cuda and x.dim() == 5 and ops.block_fused_supported(x, wp.shape[0], s[0]):
             # the three large blocks: depthwise tile -> shared memory -> tcgen05 pointwise GEMM, one kernel
             out = ops.block_dwpw_bn_relu(x, wd, s1, b1, wp, s2, b2, s[0], flag)
         else:

@@ -6,8 +6,6 @@ from __future__ import annotations
 
 from typing import List, Optional, Sequence, Tuple
 
-import os
-
 import numpy as np
 import torch
 
@@ -91,32 +89,6 @@ def stem_conv_bn_relu(x: torch.Tensor, w_packed: torch.Tensor, scale: torch.Tens
     rc = fn(x.data_ptr(), int(x.dtype == BF16), w_packed.data_ptr(), scale.data_ptr(), shift.data_ptr(), y.data_ptr(),
             n, cin, d, h, w, stride_d, _stream())
     _lib.check(rc, "ssd3d_stem_conv_bn_relu")
-    LAUNCHES[0] += 1
-    return y
-
-
-def stem_dw_fused_supported(x: torch.Tensor, stride_d: int) -> bool:
-    """True when stem + first depthwise conv can run as one kernel on ``x`` (N, Cin, D, H, W)."""
-    if x.dim() != 5 or not x.is_cuda:
-        return False
-    n, cin, d, h, w = x.shape
-    return bool(_lib.load().ssd3d_stem_dw_fused_supported(int(x.dtype == BF16), cin, d, h, w, stride_d))
-
-
-def stem_dw_bn_relu(x: torch.Tensor, w_stem: torch.Tensor, scale0: torch.Tensor, shift0: torch.Tensor,
-                    w_dw: torch.Tensor, scale1: torch.Tensor, shift1: torch.Tensor, stride_d: int,
-                    out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """Stem conv_bn (mobilenet.py:28-30) + depthwise 3x3x3 stride 2 + BN + ReLU of the first Block
-    (mobilenet.py:38,44) in one kernel: x (N,Cin,D,H,128) bf16 -> (N,32,Dd,Hd,32) channels-last bf16."""
-    _need_cuda(x, w_stem, scale0, shift0, w_dw, scale1, shift1)
-    x = x.contiguous()
-    n, cin, d, h, w = x.shape
-    ds, hs, ws = conv_out(d, stride_d), conv_out(h, 2), conv_out(w, 2)
-    y = out if out is not None else _alloc_ndhwc(n, 32, conv_out(ds, 2), conv_out(hs, 2), conv_out(ws, 2), x.device)
-    rc = _lib.load().ssd3d_stem_dw_fused(x.data_ptr(), int(x.dtype == BF16), w_stem.data_ptr(), scale0.data_ptr(),
-                                         shift0.data_ptr(), w_dw.data_ptr(), scale1.data_ptr(), shift1.data_ptr(),
-                                         y.data_ptr(), n, cin, d, h, w, stride_d, _stream())
-    _lib.check(rc, "ssd3d_stem_dw_fused")
     LAUNCHES[0] += 1
     return y
 
@@ -696,11 +668,6 @@ def _sync_words(device) -> torch.Tensor:
     return cur
 
 
-def _bn_unit_enabled() -> bool:
-    """SSD3D_BN_UNIT=0 selects the three-launch BatchNorm passes of train.cu (kept for A/B measurements)."""
-    return os.environ.get("SSD3D_BN_UNIT", "1") != "0"
-
-
 def stem_conv_raw(x: torch.Tensor, w_packed: torch.Tensor, stride_d: int) -> torch.Tensor:
     """Raw stem conv output (no BN, no ReLU), channels-last bf16."""
     _need_cuda(x, w_packed)
@@ -762,6 +729,16 @@ class BNState:
 def bn_train_relu(z: torch.Tensor, bn: torch.nn.BatchNorm3d, nan_flag: Optional[torch.Tensor] = None):
     """Training-mode BatchNorm3d + ReLU on a raw conv output (channels-last bf16) -> (a, BNState); updates the
     module's running statistics and num_batches_tracked like nn.BatchNorm3d does."""
+    return _bn_train_relu(z, bn, nan_flag, single_launch=True)
+
+
+def _bn_train_relu_passes(z: torch.Tensor, bn: torch.nn.BatchNorm3d, nan_flag: Optional[torch.Tensor] = None):
+    """``bn_train_relu`` on the three-launch passes of train.cu: what it falls back to when ``bn_unit`` does not take
+    the shape or the driver refuses its launch, and the reference the single launch is tested against."""
+    return _bn_train_relu(z, bn, nan_flag, single_launch=False)
+
+
+def _bn_train_relu(z, bn, nan_flag, single_launch: bool):
     _need_cuda(z, nan_flag)
     n, c, d, h, w = z.shape
     m = n * d * h * w
@@ -781,7 +758,7 @@ def bn_train_relu(z: torch.Tensor, bn: torch.nn.BatchNorm3d, nan_flag: Optional[
             st.scale.data_ptr(), st.shift.data_ptr(), st.mean.data_ptr(), st.invstd.data_ptr(),
             a.data_ptr(), _ptr(nan_flag), ws.data_ptr(), ws.numel())
     rc = _lib.SSD3D_ERR_UNSUPPORTED
-    if _bn_unit_enabled() and lib.ssd3d_bn_unit_supported(m, c):
+    if single_launch and lib.ssd3d_bn_unit_supported(m, c):
         rc = lib.ssd3d_bn_unit_fwd(*args, _sync_words(z.device).data_ptr(), _stream())
         if rc != _lib.SSD3D_ERR_UNSUPPORTED:     # unsupported = the driver refused the launch: three-launch path
             _lib.check(rc, "ssd3d_bn_unit_fwd")
@@ -801,6 +778,16 @@ def bn_train_relu(z: torch.Tensor, bn: torch.nn.BatchNorm3d, nan_flag: Optional[
 
 def bn_relu_backward(z: torch.Tensor, grad_a: torch.Tensor, st: BNState, dgamma: torch.Tensor, dbeta: torch.Tensor):
     """-> dz, written over grad_a (both channels-last bf16); dgamma / dbeta (C) fp32 are filled."""
+    return _bn_relu_backward(z, grad_a, st, dgamma, dbeta, single_launch=True)
+
+
+def _bn_relu_backward_passes(z: torch.Tensor, grad_a: torch.Tensor, st: BNState, dgamma: torch.Tensor,
+                             dbeta: torch.Tensor):
+    """``bn_relu_backward`` on the three-launch passes of train.cu (see ``_bn_train_relu_passes``)."""
+    return _bn_relu_backward(z, grad_a, st, dgamma, dbeta, single_launch=False)
+
+
+def _bn_relu_backward(z, grad_a, st, dgamma, dbeta, single_launch: bool):
     n, c, d, h, w = z.shape
     lib = _lib.load()
     ws = _workspace(lib.ssd3d_bn_workspace_bytes(c), z.device)
@@ -808,7 +795,7 @@ def bn_relu_backward(z: torch.Tensor, grad_a: torch.Tensor, st: BNState, dgamma:
     args = (z.data_ptr(), grad_a.data_ptr(), m, c, st.scale.data_ptr(), st.shift.data_ptr(), st.mean.data_ptr(),
             st.invstd.data_ptr(), dgamma.data_ptr(), dbeta.data_ptr(), grad_a.data_ptr(), ws.data_ptr(), ws.numel())
     rc = _lib.SSD3D_ERR_UNSUPPORTED
-    if _bn_unit_enabled() and lib.ssd3d_bn_unit_supported(m, c):
+    if single_launch and lib.ssd3d_bn_unit_supported(m, c):
         rc = lib.ssd3d_bn_unit_bwd(*args, _sync_words(z.device).data_ptr(), _stream())
         if rc != _lib.SSD3D_ERR_UNSUPPORTED:
             _lib.check(rc, "ssd3d_bn_unit_bwd")
@@ -854,7 +841,7 @@ def stem_unit_backward(z: torch.Tensor, grad_a: torch.Tensor, st: BNState, dgamm
     m = n * do * ho * wo
     _, cin, d, h, w = x.shape
     lib = _lib.load()
-    if not (_bn_unit_enabled() and lib.ssd3d_bn_unit_supported(m, c)) or m < 128 * 148 or cin > 4:
+    if not lib.ssd3d_bn_unit_supported(m, c) or m < 128 * 148 or cin > 4:
         return False
     if not lib.ssd3d_stem_tc_supported(int(x.dtype == BF16), cin, w):
         return False

@@ -19,7 +19,6 @@ from __future__ import annotations
 
 import inspect
 import operator
-import os
 from typing import Dict, List, Optional
 
 import numpy as np
@@ -135,15 +134,19 @@ class MobileNetBase(nn.Module):
                 f.nan_flag = flag
         return prev
 
-    def forward(self, image, check_nan: bool = True, stem_out=None):
+    def forward(self, image, check_nan: bool = True, stem_out=None, fuse: bool = True):
         """``stem_out``: the already-computed output of features[0] (the captured inference plan runs the
-        stem eagerly on the caller's tensor and replays the rest from a static buffer)."""
+        stem eagerly on the caller's tensor and replays the rest from a static buffer).  ``fuse``: see
+        ``Block.forward``."""
         flag = self.nan_flag(image.device if stem_out is None else stem_out.device)
         out = image
         wanted = list(self.aspect_ratios.keys())
         out_features = {}
         for i, feat in enumerate(self.features):
-            out = stem_out if (i == 0 and stem_out is not None) else feat(out)
+            if i == 0:
+                out = feat(out) if stem_out is None else stem_out
+            else:
+                out = feat(out, fuse=fuse)
             if i in wanted:
                 out_features[i] = out
         if check_nan and int(flag.item()) & _lib.NAN_BACKBONE:
@@ -243,6 +246,9 @@ class PredictionConvolutions(nn.Module):
             ops.head_conv(feat, w, b, locs, classes_scores, bpl, self.n_classes, prior_offset, nan_flag)
 
 
+TAIL_FROM = 3   # first backbone layer of a captured inference plan on the high-priority stream
+
+
 class _InferencePlan:
     """forward + detect_objects for one input signature, captured once into a CUDA graph.
 
@@ -252,9 +258,9 @@ class _InferencePlan:
     whose per-image counts, the detect status word and the NaN flag are packed in one int32 vector that is
     read back with a single device->host copy."""
 
-    def __init__(self, model: "LSSD3D", shape, dtype, min_score, max_overlap, top_k, fuse_mask=None):
+    def __init__(self, model: "LSSD3D", shape, dtype, min_score, max_overlap, top_k, fuse_blocks: bool):
         dev = model.device
-        self.fuse_mask = fuse_mask          # which Blocks run as the fused depthwise->pointwise kernel (None: default)
+        self.fuse_blocks = fuse_blocks      # Blocks run as the fused depthwise->pointwise kernel where it applies
         n = shape[0]
         self.key = None
         self.inp = torch.empty(shape, dtype=dtype, device=dev)
@@ -268,14 +274,6 @@ class _InferencePlan:
         self.cloned = torch.cuda.Event()     # results of the latest launch were copied out of the static buffers
         self.copied = torch.cuda.Event()     # the latest host batch has arrived in the static input buffer
         self.stem = model.base.features[0]
-        # stem + depthwise conv of the first Block as ONE eager kernel (csrc/conv_stem_dw.cu; opt-in, see
-        # LSSD3D.fuse_stem_dw): the static buffer the graph reads then holds the depthwise output and the graph
-        # starts at the first Block's pointwise conv
-        blk1 = self.blk1 = model.base.features[1] if len(model.base.features) > 1 else None
-        sd3 = tuple(int(v) for v in self.stem[0].stride)
-        self.front_fused = bool(getattr(model, "fuse_stem_dw", 0)) and blk1 is not None and \
-            tuple(int(v) for v in blk1.conv1.stride) == (2, 2, 2) and blk1.conv1.in_channels == 32 and \
-            ops.stem_dw_fused_supported(self.inp, sd3[0])
         self.flag = torch.zeros((1,), dtype=torch.int32, device=dev)   # this plan's own NaN word: plans may overlap
         self.stream = torch.cuda.Stream(device=dev)                     # compute stream of the streaming API
         # Later stages run at higher stream priority (recorded into the graph's kernel nodes): when two batches
@@ -283,7 +281,6 @@ class _InferencePlan:
         # takes SM slots as soon as CTAs of the younger batch's big layers retire, instead of queueing behind them.
         self.head_streams = [torch.cuda.Stream(device=dev, priority=-1) for _ in model.aspect_ratios]
         self.tail_stream = torch.cuda.Stream(device=dev, priority=-1)
-        self.tail_from = model.tail_from   # backbone layers >= this index run on the high-priority stream
         side = torch.cuda.Stream(device=dev)
         side.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(side), torch.no_grad():
@@ -301,27 +298,17 @@ class _InferencePlan:
         self.graph = graph
 
     def _front(self, image: torch.Tensor, out):
-        """features[0] (or, fused, features[0] + the depthwise half of features[1]) on ``image``.  It runs outside
-        the graph so that a device-resident batch is consumed in place (no staging copy of the largest tensor of
-        the step); a host batch goes through the static input buffer."""
-        if not self.front_fused:
-            return self.stem(image, out=out)
-        w0, sc0, sh0 = self.stem._pack()
-        wd, sc1, sh1 = self.blk1._pack()[:3]
-        return ops.stem_dw_bn_relu(image, w0, sc0, sh0, wd, sc1, sh1, int(self.stem[0].stride[0]), out=out)
+        """features[0] on ``image``.  It runs outside the graph so that a device-resident batch is consumed in place
+        (no staging copy of the largest tensor of the step); a host batch goes through the static input buffer."""
+        return self.stem(image, out=out)
 
     def _run(self, model: "LSSD3D"):
-        from . import mobilenet
         dev = self.inp.device
         model.base.nan_flag(dev)
         prev_flag = model.base.use_nan_flag(self.flag)
-        prev_mask = mobilenet.FUSE_DWPW[0]
-        if self.fuse_mask is not None:
-            mobilenet.FUSE_DWPW[0] = int(self.fuse_mask)
         try:
             self._run_with_flag(model, self.flag)
         finally:
-            mobilenet.FUSE_DWPW[0] = prev_mask
             model.base.use_nan_flag(prev_flag)
 
     def _run_with_flag(self, model: "LSSD3D", flag: torch.Tensor):
@@ -342,14 +329,12 @@ class _InferencePlan:
         cur = main
         tail = self.tail_stream
         for i, feat in enumerate(base.features):
-            if i == self.tail_from and cur is main:
+            if i == TAIL_FROM and cur is main:
                 tail.wait_stream(main)
                 cur = tail
             with torch.cuda.stream(cur):
-                if i == 1 and self.front_fused:
-                    out = feat.pointwise_only(out)       # its depthwise half ran with the stem
-                elif i > 0:
-                    out = feat(out)
+                if i > 0:
+                    out = feat(out, fuse=self.fuse_blocks)
                 if i in keys:
                     j = keys.index(i)
                     keep_alive.append(out)
@@ -530,13 +515,7 @@ class LSSD3D(_LightningBase):
         self.loss_fn = MultiBoxLoss(self.priors_cxcycz, threshold=threshold, alpha=alpha)
         self.defer_nan_check = False
         self.use_cuda_graph = True     # predict_step replays a captured forward+detect graph
-        self.pipeline_depth = int(os.environ.get("SSD3D_PIPELINE_DEPTH", "6"))   # batches in flight in predict_batches
-        self.tail_from = int(os.environ.get("SSD3D_TAIL_FROM", "3"))   # first backbone layer on the high-priority stream
-        # fused Block kernels in the streaming pipeline (see mobilenet.FUSE_DWPW): off, measured slower there
-        self.fuse_blocks_pipeline = int(os.environ.get("SSD3D_FUSE_DWPW_PIPELINE", "0"))
-        # stem + first depthwise conv as one kernel in the captured plans (csrc/conv_stem_dw.cu).  Opt-in: measured
-        # at the benchmark shape it equals the two stand-alone kernels (77 vs 76 us alone), see DESIGN.md section 6
-        self.fuse_stem_dw = int(os.environ.get("SSD3D_FUSE_STEM_DW", "0"))
+        self.pipeline_depth = 6        # batches in flight in predict_batches
         self._plans = {}
 
     # ------------------------------------------------------------------------------------------
@@ -618,8 +597,7 @@ class LSSD3D(_LightningBase):
         24-byte read per prior) while ``priors_cxcycz`` is still the constructor's tensor; the tensor itself once a
         caller has replaced or edited it (it is a public attribute of the reference's class)."""
         pri = self._priors_on(dev)
-        if (os.environ.get("SSD3D_ANALYTIC_PRIORS", "1") == "0" or pri is not self.__dict__.get("_priors_origin")
-                or pri._version != self.__dict__.get("_priors_version")):
+        if pri is not self.__dict__.get("_priors_origin") or pri._version != self.__dict__.get("_priors_version"):
             return pri
         tbl = self.__dict__.get("_prior_table")
         if tbl is None or tbl.dev.device != dev:
@@ -718,19 +696,19 @@ class LSSD3D(_LightningBase):
             eng.packed.refresh()     # values were copied into the flat buffer in place
         return out
 
-    def _plan_for(self, image: torch.Tensor, slot: int = 0, fuse_mask=None) -> _InferencePlan:
+    def _plan_for(self, image: torch.Tensor, slot: int = 0, fuse_blocks: bool = True) -> _InferencePlan:
         if self.training:
             raise RuntimeError("predict_step needs eval() mode (BatchNorm running statistics)")
         dtype = image.dtype if image.dtype in (torch.float32, torch.bfloat16) else torch.float32
         key = (tuple(image.shape), dtype, str(self.device), float(self.min_score), float(self.max_overlap),
-               int(self.top_k), slot, fuse_mask, int(self.fuse_stem_dw))
+               int(self.top_k), slot, fuse_blocks)
         ver = self._state_version()
         plan = self._plans.get(key)
         if plan is None or plan.key != ver:
             if len(self._plans) > 24:
                 self._plans.clear()
             plan = _InferencePlan(self, tuple(image.shape), dtype, self.min_score, self.max_overlap, self.top_k,
-                                  fuse_mask)
+                                  fuse_blocks)
             plan.key = ver
             self._plans[key] = plan
         return plan
@@ -773,7 +751,7 @@ class LSSD3D(_LightningBase):
             image = batch["img"]
             if len(inflight) == depth:
                 yield inflight.pop(0).results(self, post_stream, to_host, caller)
-            plan = self._plan_for(image, slot, self.fuse_blocks_pipeline)
+            plan = self._plan_for(image, slot, fuse_blocks=False)
             if image.dtype != plan.inp.dtype:
                 image = image.to(plan.inp.dtype)
             plan.launch(image, copy_stream, own_stream=True, caller_stream=caller)

@@ -19,7 +19,6 @@ PyTorch is plumbing (memory, streams, autograd hand-off, NCCL); every arithmetic
 from __future__ import annotations
 
 import math
-import os
 from typing import Dict, List, Optional
 
 import torch
@@ -28,6 +27,10 @@ import torch.nn as nn
 
 from . import _lib, ops
 from .mobilenet import Block, ConvBN, _stride3
+
+
+SIDE_STREAMS = 3                 # side streams of a training step (TrainEngine._side_streams)
+HEAVY_LEAF_BYTES = 32 * 2 ** 20  # weight-gradient leaves that read this much or more stay on the main stream
 
 
 class _Grads:
@@ -228,17 +231,13 @@ class TrainEngine:
         self.record = None
         self.collective_mode = "none"
 
-    def _wgrad_side_stream(self, main):
-        """Second stream of the backward pass (weight gradients), on ``main``'s device."""
-        return self._side_streams(main)[0]
-
     def _side_streams(self, main):
-        """The side streams of the step: the weight-gradient leaves are dealt round-robin over them (each is a few
-        small launches -- tens of CTAs -- so independent leaves run next to each other instead of queueing behind
-        one another); every stream has its own scratch slot.  SSD3D_TRAIN_SIDE_STREAMS sets the count."""
-        n = max(1, int(os.environ.get("SSD3D_TRAIN_SIDE_STREAMS", "3")))
-        if self._side is None or self._side[0].device != main.device or len(self._side) != n:
-            self._side = [torch.cuda.Stream(device=main.device) for _ in range(n)]
+        """The side streams of the step, on ``main``'s device: the weight-gradient leaves are dealt round-robin over
+        them (each is a few small launches -- tens of CTAs -- so independent leaves run next to each other instead
+        of queueing behind one another); every stream has its own scratch slot.  The forward pass issues the heads
+        on the first one."""
+        if self._side is None or self._side[0].device != main.device:
+            self._side = [torch.cuda.Stream(device=main.device) for _ in range(SIDE_STREAMS)]
         return self._side
 
     # ------------------------------------------------------------------------------------------
@@ -290,7 +289,7 @@ class TrainEngine:
         head_w = ([(packed.views["head%d.w" % j], packed.views["head%d.b" % j]) for j in range(len(keys))]
                   if packed else pc._pack())
         main = torch.cuda.current_stream()
-        side = self._wgrad_side_stream(main) if os.environ.get("SSD3D_TRAIN_WGRAD_STREAM", "1") != "0" else None
+        side = self._side_streams(main)[0]
         for i, feat in enumerate(m.base.features):
             if isinstance(feat, ConvBN):
                 conv, bn = feat[0], feat[1]
@@ -320,21 +319,16 @@ class TrainEngine:
                 j = keys.index(i)
                 if tuple(x.shape[2:]) != dims_of(x, counts_at[i], pc.n_boxes[i]):
                     raise RuntimeError("feature map %d has an unexpected shape %r" % (i, tuple(x.shape)))
-                if side is not None:
-                    side.wait_stream(main)
-                    ops._WS_SLOT[0] = "ws_side"
-                    try:
-                        with torch.cuda.stream(side):
-                            ops.head_conv(x, head_w[j][0], head_w[j][1], locs, scores, pc.n_boxes[i], pc.n_classes,
-                                          offs[j], flag)
-                    finally:
-                        ops._WS_SLOT[0] = "ws"
-                else:
-                    ops.head_conv(x, head_w[j][0], head_w[j][1], locs, scores, pc.n_boxes[i], pc.n_classes, offs[j],
-                                  flag)
+                side.wait_stream(main)
+                ops._WS_SLOT[0] = "ws_side"
+                try:
+                    with torch.cuda.stream(side):
+                        ops.head_conv(x, head_w[j][0], head_w[j][1], locs, scores, pc.n_boxes[i], pc.n_classes,
+                                      offs[j], flag)
+                finally:
+                    ops._WS_SLOT[0] = "ws"
                 tape["heads"].append(dict(j=j, layer=i, feat=x, w=head_w[j][0], off=offs[j], bpl=pc.n_boxes[i]))
-        if side is not None:
-            main.wait_stream(side)
+        main.wait_stream(side)
         self.tape = tape
         return locs, scores
 
@@ -372,8 +366,7 @@ class TrainEngine:
         # gradient tensors the side stream reads are kept alive until the join (the allocator would hand their
         # memory to a later main-stream tensor otherwise); the side stream has its own scratch slot.
         main = torch.cuda.current_stream()
-        sides = self._side_streams(main) if os.environ.get("SSD3D_TRAIN_WGRAD_STREAM", "1") != "0" else None
-        side = sides[0] if sides else None
+        sides = self._side_streams(main)
         keep = []
         n_leaf = [0]
 
@@ -381,10 +374,8 @@ class TrainEngine:
         # around them, so overlapping buys nothing, and their persistent CTAs (180 registers, ~200 KB of shared
         # memory) would keep the all-resident BatchNorm grids of the main chain (csrc/bn_unit.cu) waiting for SMs.
         # They run in order on the main stream.
-        heavy_bytes = float(os.environ.get("SSD3D_TRAIN_HEAVY_LEAF_MB", "32")) * 2 ** 20
-
         def leaf(fn, *tensors, nbytes=0):
-            if side is None or nbytes >= heavy_bytes:
+            if nbytes >= HEAVY_LEAF_BYTES:
                 fn()
                 return
             k = n_leaf[0] % len(sides)
@@ -453,7 +444,7 @@ class TrainEngine:
                     r["g"] = snap(g)
                 # first layer: nothing upstream needs dz, so (outside the tests' recording mode) it is never written --
                 # the weight-gradient kernel applies the BatchNorm + ReLU backward to the rows it loads
-                fused = (r is None and os.environ.get("SSD3D_STEM_BWD_FUSED", "1") != "0" and
+                fused = (r is None and
                          ops.stem_unit_backward(u["z"], g, u["st"], grads[p + ".1.weight"], grads[p + ".1.bias"],
                                                 u["x"], u["stride"], grads[p + ".0.weight"]))
                 if not fused:
@@ -462,9 +453,8 @@ class TrainEngine:
                         r["dz"] = snap(dz)
                     ops.stem_wgrad(dz, u["x"], u["stride"], grads[p + ".0.weight"])
                 g = None
-        if sides is not None:
-            for st in sides:
-                main.wait_stream(st)
+        for st in sides:
+            main.wait_stream(st)
         del keep
 
 
@@ -583,7 +573,6 @@ class _TrainPlan:
         for real, so everything they touch -- BatchNorm buffers, parameters, Adam moments and counters -- is
         restored afterwards."""
         flat = self.flat
-        in_graph = os.environ.get("SSD3D_TRAIN_OPT_IN_GRAPH", "1") != "0"
         buffers = {k: v.clone() for k, v in model.named_buffers()}
         state = (flat.param, flat.exp_avg, flat.exp_avg_sq, flat.status, *self.extra_state)
         saved = [t.clone() for t in state]
@@ -591,7 +580,7 @@ class _TrainPlan:
         side.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(side), torch.no_grad():
             for _ in range(2):
-                self._run(model, in_graph)
+                self._run(model, True)
         torch.cuda.current_stream().wait_stream(side)
         torch.cuda.synchronize()
 
@@ -613,10 +602,10 @@ class _TrainPlan:
         try:
             # thread_local: the NCCL watchdog thread may query events of earlier collectives while we capture
             with torch.no_grad(), torch.cuda.graph(graph, stream=cap, capture_error_mode="thread_local"):
-                self._run(model, in_graph)
-            self.optimizer_in_graph = in_graph
+                self._run(model, True)
+            self.optimizer_in_graph = True
         except Exception:
-            if not (in_graph and self.allreduce is not None):
+            if self.allreduce is None:
                 raise
             # a collective that cannot be captured (a custom ``allreduce`` callable): optimizer outside the graph
             torch.cuda.synchronize()

@@ -50,7 +50,6 @@ def main():
         model.load_state_dict(sd)
         model = model.to(dev).train()
         model.use_cuda_graph = False
-        os.environ["SSD3D_TRAIN_WGRAD_STREAM"] = "0"       # one stream: serialised launches, clean per-kernel times
         x, b, l = synthetic.make_batch(16, 1, (96, 96, 96), with_boxes=True)
         batch = {"img": torch.from_numpy(x).to(dev), "boxes": [torch.from_numpy(v).to(dev) for v in b],
                  "labels": [torch.from_numpy(v).to(dev) for v in l]}

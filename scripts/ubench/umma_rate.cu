@@ -1,6 +1,6 @@
 // Micro-benchmark: issue rate / execution time of tcgen05.mma kind::f16 (bf16, M=128, K=16) with both operands in
 // shared memory, as a function of N and of the operand layout (no swizzle with the overlapping LBO = 16 B trick of
-// conv_stem_tz.cu / conv_stem_dw.cu, plain no-swizzle, 128B swizzle).  One CTA per SM, one issuing thread,
+// conv_stem_tz.cu, plain no-swizzle, 128B swizzle).  One CTA per SM, one issuing thread,
 // `reps` UMMAs into the same accumulator, one commit; cycles from clock64.
 //   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -I mslesions3d_b200/csrc scripts/ubench/umma_rate.cu -o gpurun_out/umma_rate
 #include "common.cuh"

@@ -90,44 +90,6 @@ def test_stem_conv(cin, size, sd, dtype, batch):
         assert_bf16_close(got, want, "stem %s" % (kernel or "auto"))
 
 
-@pytest.mark.parametrize("cin,size,sd,batch", [
-    (2, (16, 28, 128), 2, 2),      # one 7-row tile, runs of 2-3 steps per CTA
-    (1, (24, 64, 128), 1, 1),      # stride 1 along D, three row tiles (7, 7, 2 rows)
-    (2, (128, 128, 128), 2, 1),    # the benchmark volume
-    (2, (36, 60, 128), 2, 3),      # ragged last row tile, runs crossing image / tile boundaries
-])
-def test_stem_dw_fused(cin, size, sd, batch):
-    """stem conv_bn + first depthwise conv in one kernel vs torch fp32 on bf16-rounded tensors (the stem activation
-    is rounded to bf16 like the stand-alone path stores it) and vs the two stand-alone kernels."""
-    ops = _ops()
-    g = torch.Generator().manual_seed(7 * cin + size[0])
-    x = bf16r(torch.randn((batch, cin) + size, generator=g))
-    w0 = torch.randn((32, cin, 3, 3, 3), generator=g) * 0.2
-    sc0, sh0 = rand_bn(32, g)
-    w1 = torch.randn((32, 1, 3, 3, 3), generator=g) * 0.3
-    sc1, sh1 = rand_bn(32, g)
-    xg = x.cuda().to(torch.bfloat16)
-    assert ops.stem_dw_fused_supported(xg, sd)
-    mid = F.conv3d(x, bf16r(w0), None, (sd, 2, 2), 1)
-    mid = bf16r(F.relu(mid * sc0.view(1, -1, 1, 1, 1) + sh0.view(1, -1, 1, 1, 1)))
-    want = F.conv3d(mid, bf16r(w1), None, 2, 1, 1, 32)
-    want = bf16r(F.relu(want * sc1.view(1, -1, 1, 1, 1) + sh1.view(1, -1, 1, 1, 1)))
-    ws, wd = ops.pack_stem_weight(w0.cuda()), ops.pack_dw_weight(w1.cuda())
-    got = ops.stem_dw_bn_relu(xg, ws, sc0.cuda(), sh0.cuda(), wd, sc1.cuda(), sh1.cuda(), sd)
-    assert got.shape == want.shape and got.is_contiguous(memory_format=torch.channels_last_3d)
-    # the two stand-alone kernels: the banded-B stem accumulates in the same order as the fused kernel and the
-    # depthwise kernels apply their taps in the same (kd, kh, kw) order with fp32 FMAs -> bit-identical
-    mid_g = ops.stem_conv_bn_relu(xg, ws, sc0.cuda(), sh0.cuda(), sd, kernel="tz")
-    two = ops.dwconv3d_bn_relu(mid_g, wd, sc1.cuda(), sh1.cuda(), 2)
-    assert torch.equal(got, two), "fused vs stand-alone kernels: %d elements differ, max %.4g" % (
-        int((got != two).sum()), float((got.float() - two.float()).abs().max()))
-    # vs torch fp32: a stem value that rounds the other way (rare) moves a depthwise sum by up to weight * ulp
-    diff = (got.float().cpu() - want).abs()
-    tol = 2.0 ** -7 * want.abs().clamp_min(2.0 ** -6)
-    assert float((diff > tol).float().mean()) < 0.01, "%.2f%% beyond one bf16 ulp" % (100 * float((diff > tol).float().mean()))
-    assert float(diff.max()) < 0.06, "fused stem+dw: max diff %.4g" % float(diff.max())
-
-
 @pytest.mark.parametrize("c,size,stride,batch", [
     (32, (16, 16, 16), 2, 2),
     (32, (9, 11, 13), 2, 1),

@@ -105,7 +105,7 @@ def test_bn_train_relu_forward_backward(n, c, size):
                                       (3, 128, (7, 5, 3)), (16, 256, (12, 12, 12)),
                                       # more than 32768 rows: the grid-barrier kernel, C/8 = 32, 64, 128
                                       (1, 256, (34, 33, 31)), (1, 512, (33, 32, 32)), (2, 1024, (17, 32, 32))])
-def test_bn_single_launch_matches_three_launch_path(n, c, size, monkeypatch):
+def test_bn_single_launch_matches_three_launch_passes(n, c, size):
     """csrc/bn_unit.cu (one launch, grid barriers) against the three-launch passes of train.cu on the same inputs:
     same statistics to fp32 rounding, same activations / gradients to 1 bf16 ulp; repeated launches (the barrier
     words are reused) are bit-identical; the launch counter shows which path ran."""
@@ -115,7 +115,8 @@ def test_bn_single_launch_matches_three_launch_path(n, c, size, monkeypatch):
     ga = to_cl(bf16r(torch.randn((n, c) + size, generator=g)))
     res = {}
     for mode in ("0", "1", "1"):
-        monkeypatch.setenv("SSD3D_BN_UNIT", mode)
+        fwd, bwd = (ops.bn_train_relu, ops.bn_relu_backward) if mode == "1" else \
+            (ops._bn_train_relu_passes, ops._bn_relu_backward_passes)
         bn = torch.nn.BatchNorm3d(c)
         with torch.no_grad():
             bn.weight.copy_(0.5 + torch.rand(c, generator=torch.Generator().manual_seed(c)))
@@ -123,10 +124,10 @@ def test_bn_single_launch_matches_three_launch_path(n, c, size, monkeypatch):
         bn = bn.cuda().train()
         flag = torch.zeros(1, dtype=torch.int32, device="cuda")
         before = ops.LAUNCHES[0]
-        a, st = ops.bn_train_relu(z, bn, flag)
+        a, st = fwd(z, bn, flag)
         assert ops.LAUNCHES[0] - before == (1 if mode == "1" else 3)
         dgamma, dbeta = torch.empty(c, device="cuda"), torch.empty(c, device="cuda")
-        dz = ops.bn_relu_backward(z, ga.clone(), st, dgamma, dbeta)
+        dz = bwd(z, ga.clone(), st, dgamma, dbeta)
         torch.cuda.synchronize()
         cur = dict(a=a, dz=dz, dgamma=dgamma, dbeta=dbeta, scale=st.scale, shift=st.shift, mean=st.mean,
                    invstd=st.invstd, rm=bn.running_mean.clone(), rv=bn.running_var.clone(), flag=int(flag),
