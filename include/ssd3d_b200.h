@@ -529,6 +529,36 @@ int ssd3d_gt_pack(const float* boxes, const int64_t* labels, const int32_t* coun
                   int N, int max_boxes, int per_volume, float* gt_boxes, int64_t* gt_labels, int32_t* offsets,
                   int32_t* status, void* stream);
 
+/* ------------------------------------------------------------------------------------------------
+ * Sliding-window inference over scans larger than the network input.
+ *
+ * ssd3d_window_gather copies the windows of S scans src (S, C, D, H, W) (fp32 with src_is_bf16 = 0, else bf16)
+ * into out (S*T, C, d, h, w) bf16, NCDHW, scan-major.  Per spatial axis a (extent S_a, window w_a, stride s_a >= 1)
+ * there are n_a = ceil((S_a - w_a) / s_a) + 1 windows starting at o_i = min(i * s_a, S_a - w_a); window
+ * t = (i_d * n_h + i_h) * n_w + i_w, T = n_d * n_h * n_w.  fp32 is rounded to nearest even (bit-equal to
+ * torch.Tensor.to(torch.bfloat16) for every non-NaN value).  d <= D, h <= H, w <= W; w % 8 == 0 and w <= 8192
+ * (16-byte stores of whole rows), else SSD3D_ERR_UNSUPPORTED.  No host sync: graph-capturable.
+ *
+ * ssd3d_merge_windows merges per-window detections -- the padded outputs of ssd3d_detect_objects over the S*T
+ * windows: win_boxes (S*T, K, 6), win_scores (S*T, K), win_labels (S*T, K) int64, win_count (S*T) -- into
+ * per-scan detections with the same padded outputs (out_* (S, top_k[, 6]), out_count (S)).  Candidate
+ * j = t * K + r is entry r < win_count[t] of window t; entries with label outside [1, n_classes) (label 0 is
+ * the "nothing found" placeholder) or score <= min_score are skipped.  Its box is mapped into the scan's
+ * fractional coordinates, coordinates k and k + 3 on spatial axis k:
+ *   x' = fp32_rn(fp32_rn(x * scale_k) + win_offset[t * 3 + k]),  scale_k = fp32(w_k / S_k), offset = fp32(o_k / S_k)
+ * (win_offset (T, 3) fp32 on the device).  Then exactly ssd3d_detect_objects' stages 2-4 with P = T * K and
+ * "prior" j: per (scan, class) sort by {score descending, j ascending}, truncation to 10 * top_k, greedy NMS
+ * at max_overlap, class merge, top-k and the placeholder for a scan with nothing left; out_cand receives j
+ * (-1 for a placeholder).  Same limits as ssd3d_detect_objects (status bit 0, SSD3D_ERR_UNSUPPORTED). */
+int ssd3d_window_gather(const void* src, int src_is_bf16, int S, int C, int D, int H, int W, int d, int h, int w,
+                        int stride_d, int stride_h, int stride_w, void* out, void* stream);
+int64_t ssd3d_merge_windows_workspace_bytes(int n_scans, int n_windows, int K, int n_classes, int top_k);
+int ssd3d_merge_windows(const float* win_boxes, const float* win_scores, const int64_t* win_labels,
+                        const int32_t* win_count, int n_scans, int n_windows, int K, const float* win_offset,
+                        float scale_d, float scale_h, float scale_w, int n_classes, float min_score, float max_overlap,
+                        int top_k, float* out_boxes, float* out_scores, int64_t* out_labels, int64_t* out_cand,
+                        int32_t* out_count, void* workspace, int64_t workspace_bytes, int32_t* status, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -123,6 +123,12 @@ SIGNATURES = {
     "ssd3d_augment_batch": (c_int, [P, c_int, P, c_int, c_int, c_int, c_int, c_int, P, P, P, P, c_int, c_int, c_int,
                                     c_int, c_float, c_float, c_float, c_int, c_int, c_float, c_float, P, P, P, P]),
     "ssd3d_gt_pack": (c_int, [P, P, P, P, c_int, c_int, c_int, P, P, P, P, P]),
+    # ---- sliding-window inference ----
+    "ssd3d_window_gather": (c_int, [P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,
+                                    c_int, P, P]),
+    "ssd3d_merge_windows_workspace_bytes": (c_int64, [c_int, c_int, c_int, c_int, c_int]),
+    "ssd3d_merge_windows": (c_int, [P, P, P, P, c_int, c_int, c_int, P, c_float, c_float, c_float, c_int, c_float,
+                                    c_float, c_int, P, P, P, P, P, P, c_int64, P, P]),
 }
 
 _lib = None

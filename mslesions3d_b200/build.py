@@ -26,7 +26,8 @@ COMMON_FLAGS = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "-Xcomp
                 "--expt-relaxed-constexpr", "--expt-extended-lambda"]
 # integer-exact kernels: never let the compiler contract a*b+c (boxes.cuh already uses *_rn intrinsics)
 PER_FILE_FLAGS = {"detect.cu": ["-fmad=false"], "match_loss.cu": ["-fmad=false"], "box_ops.cu": ["-fmad=false"],
-                  "metrics.cu": ["-fmad=false"], "augment.cu": ["-fmad=false"]}
+                  "metrics.cu": ["-fmad=false"], "augment.cu": ["-fmad=false"],
+                  "windows.cu": ["-fmad=false"]}
 
 
 def _nvcc() -> str:

@@ -7,7 +7,7 @@
 //   3. nms_mask      : IoU > max_overlap bit matrix (64-bit words) over the sorted candidates
 //   4. nms_select    : greedy scan of the bit matrix (ssd3d.py:414-426), per-image merge of the classes,
 //                      final top-k cut (ssd3d.py:449-453), placeholder for empty images (ssd3d.py:437-440)
-#include "boxes.cuh"
+#include "detect.cuh"
 
 namespace ssd3d {
 
@@ -1095,13 +1095,7 @@ static inline long long nms_stage_words(int words, long long n_max) {
   return want < budget ? want : (budget > 0 ? budget : 0);
 }
 
-struct DetectLayout {
-  int S, nmax, words;
-  long long off_count, off_nkeep, off_keptcnt, off_boxes, off_cand, off_cand2, cand2_stride, off_sboxes, off_sscores, off_sprior, off_mask,
-      off_keptpos, off_keptscore, total;
-};
-
-static DetectLayout detect_layout(int N, long long P, int C, int top_k) {
+DetectLayout detect_layout(int N, long long P, int C, int top_k) {
   DetectLayout L;
   L.S = N * (C - 1);
   long long nm = 10ll * (long long)top_k;
@@ -1377,17 +1371,14 @@ extern "C" int ssd3d_decode_filter_analytic(const float* locs, const float* scor
                             stream);
 }
 
-static int detect_objects_impl(const float* locs, const float* scores, PriorSrc priors, int N, int64_t P,
-                               int n_classes, float min_score, float max_overlap, int top_k, float* out_boxes,
-                               float* out_scores, int64_t* out_labels, int64_t* out_prior, int32_t* out_count,
-                               void* workspace, int64_t workspace_bytes, int32_t* status, void* stream) {
-  if (!locs || !scores || (!priors.ptr && !priors.tbl) || !out_boxes || !out_scores || !out_labels || !out_prior || !out_count || !workspace)
-    return SSD3D_ERR_ARG;
-  if (N <= 0 || P <= 0 || n_classes < 2 || top_k <= 0 || P > 0x7fffffffll) return SSD3D_ERR_ARG;
-  const DetectLayout L = detect_layout(N, P, n_classes, top_k);
-  if (workspace_bytes < L.total) return SSD3D_ERR_ARG;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  uint8_t* ws = static_cast<uint8_t*>(workspace);
+namespace ssd3d {
+// Stages 2-4 of detect_objects on the per-(image, class) candidate lists that a stage-1 kernel left in the workspace
+// (count, cand and the boxes they index, laid out by detect_layout): sort -> 10*top_k truncation -> bit-matrix NMS ->
+// per-image class merge, top-k and placeholder.  ssd3d_detect_objects and ssd3d_merge_windows share it.
+int detect_select(const DetectLayout& L, uint8_t* ws, int N, long long P, int n_classes, float max_overlap, int top_k,
+                  float* out_boxes, float* out_scores, int64_t* out_labels, int64_t* out_prior, int32_t* out_count,
+                  int32_t* status, cudaStream_t st) {
+  cudaError_t e = cudaSuccess;
   int* count = reinterpret_cast<int*>(ws + L.off_count);
   int* nkeep = reinterpret_cast<int*>(ws + L.off_nkeep);
   int* keptcnt = reinterpret_cast<int*>(ws + L.off_keptcnt);
@@ -1399,18 +1390,6 @@ static int detect_objects_impl(const float* locs, const float* scores, PriorSrc 
   unsigned long long* mask = reinterpret_cast<unsigned long long*>(ws + L.off_mask);
   int* keptpos = reinterpret_cast<int*>(ws + L.off_keptpos);
   float* keptscore = reinterpret_cast<float*>(ws + L.off_keptscore);
-
-  cudaError_t e = cudaMemsetAsync(count, 0, (size_t)(L.off_boxes - L.off_count), st);
-  if (e != cudaSuccess) return (int)e;
-  if (status) {
-    e = cudaMemsetAsync(status, 0, 4, st);
-    if (e != cudaSuccess) return (int)e;
-  }
-  {
-    dim3 grid((unsigned)((P + 255) / 256), (unsigned)N);
-    SSD3D_LAUNCH_PDL(decode_filter_kernel, grid, dim3(256), 0, st, locs, scores, priors, (long long)P, n_classes, min_score, boxes,
-                     cand, count);
-  }
   {
     int cap = 1;
     while (cap < P && cap < SSD3D_SORT_MAX) cap <<= 1;
@@ -1468,6 +1447,37 @@ static int detect_objects_impl(const float* locs, const float* scores, PriorSrc 
                      reinterpret_cast<long long*>(out_labels), reinterpret_cast<long long*>(out_prior), out_count);
   }
   return SSD3D_OK;
+}
+}  // namespace ssd3d
+
+static int detect_objects_impl(const float* locs, const float* scores, PriorSrc priors, int N, int64_t P,
+                               int n_classes, float min_score, float max_overlap, int top_k, float* out_boxes,
+                               float* out_scores, int64_t* out_labels, int64_t* out_prior, int32_t* out_count,
+                               void* workspace, int64_t workspace_bytes, int32_t* status, void* stream) {
+  if (!locs || !scores || (!priors.ptr && !priors.tbl) || !out_boxes || !out_scores || !out_labels || !out_prior || !out_count || !workspace)
+    return SSD3D_ERR_ARG;
+  if (N <= 0 || P <= 0 || n_classes < 2 || top_k <= 0 || P > 0x7fffffffll) return SSD3D_ERR_ARG;
+  const DetectLayout L = detect_layout(N, P, n_classes, top_k);
+  if (workspace_bytes < L.total) return SSD3D_ERR_ARG;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  uint8_t* ws = static_cast<uint8_t*>(workspace);
+  int* count = reinterpret_cast<int*>(ws + L.off_count);
+  float* boxes = reinterpret_cast<float*>(ws + L.off_boxes);
+  unsigned long long* cand = reinterpret_cast<unsigned long long*>(ws + L.off_cand);
+
+  cudaError_t e = cudaMemsetAsync(count, 0, (size_t)(L.off_boxes - L.off_count), st);
+  if (e != cudaSuccess) return (int)e;
+  if (status) {
+    e = cudaMemsetAsync(status, 0, 4, st);
+    if (e != cudaSuccess) return (int)e;
+  }
+  {
+    dim3 grid((unsigned)((P + 255) / 256), (unsigned)N);
+    SSD3D_LAUNCH_PDL(decode_filter_kernel, grid, dim3(256), 0, st, locs, scores, priors, (long long)P, n_classes, min_score, boxes,
+                     cand, count);
+  }
+  return detect_select(L, ws, N, P, n_classes, max_overlap, top_k, out_boxes, out_scores, out_labels, out_prior,
+                       out_count, status, st);
 }
 
 extern "C" int ssd3d_detect_objects(const float* locs, const float* scores, const float* priors, int N, int64_t P,

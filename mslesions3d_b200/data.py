@@ -2,6 +2,7 @@
 boxes, prepared once at load), ``Augment`` (the augmentation drawn per slot inside the captured training step,
 csrc/augment.cu) and ``epoch_order`` (the per-epoch permutation).  ``LSSD3D.fit_epoch`` trains on them with one
 CUDA-graph replay per step: sampling, augmentation, ground-truth extraction and packing, then the fused step.
+``window_origins`` is the grid of network-input windows over a larger scan that ``LSSD3D.predict_scans`` detects on.
 
 The reference prepares its batches with MONAI transform pipelines on CPU workers (datasets.py): a host pipeline
 cannot augment at the rate the fused step consumes volumes.
@@ -9,6 +10,7 @@ cannot augment at the rate the fused step consumes volumes.
 from __future__ import annotations
 
 import dataclasses
+import math
 import os
 from typing import Optional, Sequence, Tuple
 
@@ -56,6 +58,34 @@ class Augment:
                              % (self.rot90_axes, out[a0], out[a1]))
         if out[2] % 16:
             raise ValueError("the last input_size extent must be a multiple of 16, got %d" % out[2])
+
+
+def window_strides(window: Sequence[int], overlap: float) -> Tuple[int, int, int]:
+    """Per-axis step between neighbouring windows: max(1, floor(w * (1 - overlap)))."""
+    overlap = float(overlap)
+    if not 0.0 <= overlap < 1.0:
+        raise ValueError("overlap must lie in [0, 1), got %r" % (overlap,))
+    return tuple(max(1, int(math.floor(int(w) * (1.0 - overlap)))) for w in window)
+
+
+def window_origins(scan_shape: Sequence[int], window: Sequence[int], overlap: float):
+    """The sliding-window grid over a scan of spatial shape ``scan_shape`` -> (n_d, n_h, n_w, origins), origins a
+    (T, 3) int64 array of window corners, T = n_d * n_h * n_w, window t = (i_d * n_h + i_h) * n_w + i_w (W fastest).
+    Per axis ``n = ceil((S - w) / stride) + 1`` windows start at ``min(i * stride, S - w)``: they cover the scan
+    and the last one ends flush with it.  Scans smaller than the window are not padded: ValueError."""
+    scan_shape, window = tuple(int(v) for v in scan_shape), tuple(int(v) for v in window)
+    if len(scan_shape) != 3 or len(window) != 3:
+        raise ValueError("scan_shape and window must be (D, H, W)")
+    strides = window_strides(window, overlap)
+    if any(s < w for s, w in zip(scan_shape, window)):
+        raise ValueError("scan %r is smaller than the window %r on some axis (scans are not padded)"
+                         % (scan_shape, window))
+    axes = []
+    for s, w, st in zip(scan_shape, window, strides):
+        n = -(-(s - w) // st) + 1
+        axes.append([min(i * st, s - w) for i in range(n)])
+    grid = np.stack(np.meshgrid(*[np.asarray(a, dtype=np.int64) for a in axes], indexing="ij"), -1).reshape(-1, 3)
+    return len(axes[0]), len(axes[1]), len(axes[2]), grid
 
 
 def epoch_order(n_subjects: int, epoch: int, seed: int = 0) -> torch.Tensor:

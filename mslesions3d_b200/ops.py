@@ -1194,3 +1194,94 @@ def gt_pack(boxes: torch.Tensor, labels: torch.Tensor, meta: torch.Tensor, per_v
     _lib.check(rc, "ssd3d_gt_pack")
     LAUNCHES[0] += 1
     return gb, gl, offs, status
+
+
+# ----------------------------------------------------------------------------------------------
+# sliding-window inference over scans larger than the network input (csrc/windows.cu, LSSD3D.predict_scans)
+# ----------------------------------------------------------------------------------------------
+def window_map(scan_shape, window, origins) -> Tuple[Tuple[float, float, float], torch.Tensor]:
+    """Factors of the window -> scan coordinate map x' = x * scale_k + offset[t, k] (spatial axis k), each rounded
+    to fp32 once: scale_k = fp32(w_k / S_k), offset[t, k] = fp32(o_k / S_k).  -> (scale (3 floats), offset (T, 3)
+    fp32 CPU tensor)."""
+    scale = tuple(f32(int(w) / int(s)) for w, s in zip(window, scan_shape))
+    o = np.asarray(origins, dtype=np.float64).reshape(-1, 3)
+    offset = (o / np.asarray([float(s) for s in scan_shape])).astype(np.float32)
+    return scale, torch.from_numpy(offset)
+
+
+def window_gather(src: torch.Tensor, window, overlap: float, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """The sliding windows of scans src (S, C, D, H, W) fp32 / bf16 (grid of ``data.window_origins``) -> (S*T, C, d, h, w)
+    bf16 NCDHW, scan-major; ``out`` may be a static buffer of that shape (a captured step)."""
+    from .data import window_origins, window_strides
+    _need_cuda(src)
+    if src.dim() != 5 or src.dtype not in (torch.float32, BF16) or not src.is_contiguous():
+        raise RuntimeError("expected contiguous scans (S, C, D, H, W) fp32/bf16")
+    s, c, dd, hh, ww = src.shape
+    d, h, w = (int(v) for v in window)
+    nd, nh, nw, _ = window_origins((dd, hh, ww), (d, h, w), overlap)
+    sd, sh, sw = window_strides((d, h, w), overlap)
+    n = s * nd * nh * nw
+    if out is None:
+        out = torch.empty((n, c, d, h, w), dtype=BF16, device=src.device)
+    if tuple(out.shape) != (n, c, d, h, w) or out.dtype != BF16 or not out.is_contiguous():
+        raise RuntimeError("window_gather: out must be a contiguous (%d, %d, %d, %d, %d) bf16 tensor" % (n, c, d, h, w))
+    rc = _lib.load().ssd3d_window_gather(src.data_ptr(), int(src.dtype == BF16), s, c, dd, hh, ww, d, h, w, sd, sh, sw,
+                                         out.data_ptr(), _stream())
+    _lib.check(rc, "ssd3d_window_gather")
+    LAUNCHES[0] += 1
+    return out
+
+
+def merge_windows(boxes: torch.Tensor, scores: torch.Tensor, labels: torch.Tensor, count: torch.Tensor, n_scans: int,
+                  scan_shape, window, overlap: float, n_classes: int, min_score: float, max_overlap: float,
+                  top_k: int, offset: Optional[torch.Tensor] = None, workspace: Optional[torch.Tensor] = None,
+                  out=None, out_count: Optional[torch.Tensor] = None,
+                  status: Optional[torch.Tensor] = None) -> DetectOutput:
+    """Per-window detections -- the padded ``detect_objects_padded`` outputs over n_scans * T windows: boxes
+    (S*T, K, 6), scores (S*T, K), labels (S*T, K) int64, count (S*T) int32 -- merged into per-scan detections in the
+    scan's fractional coordinates (see ``ssd3d_merge_windows`` in the header), no host sync.  ``offset``: the
+    (T, 3) fp32 device tensor of ``window_map`` (made here when None); ``out`` / ``out_count`` / ``status``: static
+    buffers like ``detect_objects_padded``'s.  ``prior`` of the result holds the candidate index t * K + r."""
+    from .data import window_origins
+    _need_cuda(boxes, scores, labels, count)
+    nd, nh, nw, origins = window_origins(scan_shape, window, overlap)
+    t = nd * nh * nw
+    n, k = int(scores.shape[0]), int(scores.shape[1])
+    if n != int(n_scans) * t or tuple(boxes.shape) != (n, k, 6) or tuple(labels.shape) != (n, k) or \
+            tuple(count.shape) != (n,):
+        raise RuntimeError("merge_windows: expected boxes (S*T, K, 6), scores / labels (S*T, K), count (S*T) with "
+                           "S*T = %d * %d" % (n_scans, t))
+    if boxes.dtype != torch.float32 or scores.dtype != torch.float32 or labels.dtype != torch.int64 or \
+            count.dtype != torch.int32 or not all(x.is_contiguous() for x in (boxes, scores, labels, count)):
+        raise RuntimeError("merge_windows: boxes / scores fp32, labels int64 and count int32, all contiguous")
+    top_k = int(top_k)
+    if detect_needs_long_lists(t * k, top_k):
+        raise ValueError("merge_windows: top_k = %d over %d windows (%d candidates per scan) needs the any-length "
+                         "merge, which is not supported; lower top_k or the window count" % (top_k, t, t * k))
+    dev = boxes.device
+    scale, off_host = window_map(scan_shape, window, origins)
+    if offset is None:
+        offset = off_host.to(dev)
+    lib = _lib.load()
+    s = int(n_scans)
+    need = lib.ssd3d_merge_windows_workspace_bytes(s, t, k, int(n_classes), top_k)
+    if workspace is None or workspace.numel() < need:
+        workspace = torch.empty((need,), dtype=torch.uint8, device=dev)
+    if out is None:
+        out = (torch.empty((s, top_k, 6), dtype=torch.float32, device=dev),
+               torch.empty((s, top_k), dtype=torch.float32, device=dev),
+               torch.empty((s, top_k), dtype=torch.int64, device=dev),
+               torch.empty((s, top_k), dtype=torch.int64, device=dev))
+    ob, osc, ol, op = out
+    if out_count is None:
+        out_count = torch.empty((s,), dtype=torch.int32, device=dev)
+    if status is None:
+        status = torch.empty((1,), dtype=torch.int32, device=dev)
+    rc = lib.ssd3d_merge_windows(boxes.data_ptr(), scores.data_ptr(), labels.data_ptr(), count.data_ptr(), s, t, k,
+                                 offset.data_ptr(), scale[0], scale[1], scale[2], int(n_classes), f32(min_score),
+                                 f32(max_overlap), top_k, ob.data_ptr(), osc.data_ptr(), ol.data_ptr(), op.data_ptr(),
+                                 out_count.data_ptr(), workspace.data_ptr(), workspace.numel(), status.data_ptr(),
+                                 _stream())
+    _lib.check(rc, "ssd3d_merge_windows")
+    LAUNCHES[0] += 4
+    return DetectOutput(ob, osc, ol, op, out_count, status)

@@ -10,6 +10,8 @@ PyTorch-Lightning ``.ckpt`` files (``state_dict`` + ``hyper_parameters``).  Outp
 (predict.py:155-232,85-150,279-281): per subject ``sub-{id}_preds.csv`` / ``.json`` and the box-outline volume
 ``sub-{id}_preds.nii.gz`` (NIfTI-1 written by ``mslesions3d_b200/nifti.py``), ``aa_metrics_per_subject_(min_IoU=0.5|0.1).json`` from the device-side
 ``calculate_mAP``, plus one ``predictions.json`` with every subject's boxes / labels / scores.
+With ``--window_overlap`` the volumes may be larger than the network input: they go through
+``LSSD3D.predict_scans`` (sliding windows merged per scan) and every output refers to the whole scan.
 """
 from __future__ import annotations
 
@@ -51,6 +53,11 @@ def build_parser() -> argparse.ArgumentParser:
                         help="whether to save the prediction volumes (NIfTI) and predictions.json")
     parser.add_argument('-bs', '--batch_size', type=int, default=8, help="volumes per forward (reference: 1)")
     parser.add_argument('-n', '--n_subjects', type=int, default=16, help="synthetic subjects when no dataset file")
+    parser.add_argument('--window_overlap', type=float, default=None,
+                        help="detect on whole scans larger than the network input: sliding input_size windows "
+                             "overlapping by this fraction, merged per scan (LSSD3D.predict_scans)")
+    parser.add_argument('--scan_size', type=int, nargs=3, default=None,
+                        help="spatial size of the synthetic volumes (default: the model's input size)")
     return parser
 
 
@@ -151,7 +158,7 @@ def compute_subjects_mAP(model, subjects, det, gt_boxes, gt_labels, output_dir=r
 
 def predict_example(model_path, output_dir, dataset_path, dataset_name, n_classes=1, subject=None, percentage=1.,
                     predict_subset="train", min_score=0.5, top_k=10, num_workers=8, save_images=True, model_name=None,
-                    batch_size=8, n_subjects=16, model=None):
+                    batch_size=8, n_subjects=16, model=None, window_overlap=None, scan_size=None):
     torch.manual_seed(970205)
     output_dir = output_dir if dataset_name is None else pjoin(output_dir, dataset_name)
     output_dir = output_dir if model_name is None else pjoin(output_dir, model_name)
@@ -176,8 +183,8 @@ def predict_example(model_path, output_dir, dataset_path, dataset_name, n_classe
         vols = load_volumes(dataset_path, n_subjects, model.input_channels, tuple(model.input_size), percentage)
     else:   # synthetic cube volumes come with their ground-truth boxes (generate_artificial_dataset.py)
         n = max(1, int(round(n_subjects * percentage)))
-        vols, gt_boxes, gt_labels = synthetic.make_batch(n, model.input_channels, tuple(model.input_size),
-                                                         with_boxes=True)
+        size = tuple(scan_size) if scan_size is not None else tuple(model.input_size)
+        vols, gt_boxes, gt_labels = synthetic.make_batch(n, model.input_channels, size, with_boxes=True)
     if subjects is None:
         subjects = list(range(vols.shape[0]))
     if subject is not None:
@@ -187,12 +194,16 @@ def predict_example(model_path, output_dir, dataset_path, dataset_name, n_classe
             gt_boxes, gt_labels = gt_boxes[k:k + 1], gt_labels[k:k + 1]
     det_locs, det_labels, det_scores = [], [], []
     with torch.no_grad():
-        batches = ({"img": torch.from_numpy(vols[s:s + batch_size]).pin_memory()}
-                   for s in range(0, vols.shape[0], batch_size))
-        for locs, labels, scores in model.predict_batches(batches):      # Trainer.predict of the reference
-            det_locs += locs
-            det_labels += labels
-            det_scores += scores
+        if window_overlap is not None:      # whole scans: boxes come back as fractions of the scan's shape
+            det_locs, det_labels, det_scores = model.predict_scans(torch.from_numpy(np.ascontiguousarray(vols)),
+                                                                   overlap=window_overlap)
+        else:
+            batches = ({"img": torch.from_numpy(vols[s:s + batch_size]).pin_memory()}
+                       for s in range(0, vols.shape[0], batch_size))
+            for locs, labels, scores in model.predict_batches(batches):      # Trainer.predict of the reference
+                det_locs += locs
+                det_labels += labels
+                det_scores += scores
     results = {str(subjects[i]): {"boxes": det_locs[i].cpu().tolist(), "labels": det_labels[i].cpu().tolist(),
                                   "scores": det_scores[i].cpu().tolist()} for i in range(len(det_locs))}
     if output_dir is not None:
@@ -216,7 +227,8 @@ def main(argv=None):
                         dataset_name=args.dataset_name, n_classes=args.n_classes, subject=args.subject,
                         percentage=args.percentage, predict_subset=psubset, min_score=args.min_score,
                         top_k=args.top_k, num_workers=args.num_workers, save_images=args.save_images,
-                        model_name=args.model_name, batch_size=args.batch_size, n_subjects=args.n_subjects)
+                        model_name=args.model_name, batch_size=args.batch_size, n_subjects=args.n_subjects,
+                        window_overlap=args.window_overlap, scan_size=args.scan_size)
 
 
 if __name__ == "__main__":

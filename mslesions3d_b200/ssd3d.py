@@ -361,13 +361,15 @@ class _InferencePlan:
         main.wait_stream(tail)
         self.locs, self.scores = locs, scores
 
-    def _views(self, buf: torch.Tensor, k: int):
+    @staticmethod
+    def _views(buf: torch.Tensor, k: int):
         """(boxes (N,K,6) f32, scores (N,K) f32, labels (N,K) i64, prior (N,K) i64) views of a packed buffer."""
-        nk = self.n * k
-        labels = buf[:nk * 8].view(torch.int64).view(self.n, k)
-        prior = buf[nk * 8:nk * 16].view(torch.int64).view(self.n, k)
-        boxes = buf[nk * 16:nk * 40].view(torch.float32).view(self.n, k, 6)
-        scores = buf[nk * 40:nk * 44].view(torch.float32).view(self.n, k)
+        n = buf.numel() // (44 * k)
+        nk = n * k
+        labels = buf[:nk * 8].view(torch.int64).view(n, k)
+        prior = buf[nk * 8:nk * 16].view(torch.int64).view(n, k)
+        boxes = buf[nk * 16:nk * 40].view(torch.float32).view(n, k, 6)
+        scores = buf[nk * 40:nk * 44].view(torch.float32).view(n, k)
         return boxes, scores, labels, prior
 
     def launch(self, image: torch.Tensor, copy_stream=None, own_stream: bool = False, caller_stream=None):
@@ -413,24 +415,33 @@ class _InferencePlan:
         self.host_meta.copy_(self.meta, non_blocking=True)
         self.done.record(compute)
 
-    def results(self, model: "LSSD3D", post_stream=None, to_host: bool = False, caller_stream=None):
-        """Wait for this plan's latest launch (not for later work on the stream), check the flags, and hand
-        out fresh per-image tensors: the static buffers are copied on ``post_stream`` (device clones, or
-        pinned-host copies when ``to_host``) so that the next steps already queued are not delayed."""
-        self.done.synchronize()
+    @property
+    def result_buf(self) -> torch.Tensor:
+        """The packed static output buffer that ``results`` hands out."""
+        return self.outbuf
+
+    def _checked_counts(self, model: "LSSD3D"):
+        """Per-image counts of the latest launch, after raising on its NaN bits and detect status."""
         meta = self.host_meta.tolist()
         if meta[-1]:
             model._raise_on_nan_bits(meta[-1])
         if meta[-2] & 1:
             raise RuntimeError("detect_objects: more than %d candidates above min_score for one (image, class)"
                                % _lib.SORT_MAX)
-        counts = meta[:self.n]
+        return meta[:self.n]
+
+    def results(self, model: "LSSD3D", post_stream=None, to_host: bool = False, caller_stream=None):
+        """Wait for this plan's latest launch (not for later work on the stream), check the flags, and hand
+        out fresh per-image tensors: the static buffers are copied on ``post_stream`` (device clones, or
+        pinned-host copies when ``to_host``) so that the next steps already queued are not delayed."""
+        self.done.synchronize()
+        counts = self._checked_counts(model)
         current = caller_stream if caller_stream is not None else torch.cuda.current_stream()
         stream = post_stream if post_stream is not None else current
         if stream is not current:
             torch.cuda.set_stream(stream)
         try:
-            buf = self.outbuf.to("cpu", non_blocking=False) if to_host else self.outbuf.clone()
+            buf = self.result_buf.to("cpu", non_blocking=False) if to_host else self.result_buf.clone()
             self.cloned.record(stream)
         finally:
             if stream is not current:
@@ -441,6 +452,80 @@ class _InferencePlan:
         boxes, scores, labels, _ = self._views(buf, int(self.args[2]))
         return ([boxes[i, :k] for i, k in enumerate(counts)], [labels[i, :k] for i, k in enumerate(counts)],
                 [scores[i, :k] for i, k in enumerate(counts)])
+
+
+class _WindowPlan(_InferencePlan):
+    """Sliding-window detection over ``scan_shape[0]`` scans of one shape, captured into one CUDA graph: gather of the
+    ``input_size`` windows into the static input batch (csrc/windows.cu), the network on the window batch (the stem
+    included: its input is the plan's own buffer), per-window ``detect_objects`` and the merge into per-scan
+    detections.  Scans are copied into a static buffer before each replay; the per-scan counts, both detect status
+    words and the NaN bits are read back with one device->host copy."""
+
+    def __init__(self, model: "LSSD3D", scan_shape, scan_dtype, overlap, min_score, max_overlap, top_k):
+        from .data import window_origins
+        dev = model.device
+        s, c = int(scan_shape[0]), int(scan_shape[1])
+        self.window = tuple(int(v) for v in model.input_size)
+        self.overlap = float(overlap)
+        nd, nh, nw, origins = window_origins(scan_shape[2:], self.window, self.overlap)
+        self.n_scans, self.n_windows = s, nd * nh * nw
+        self.scan_spatial = tuple(int(v) for v in scan_shape[2:])
+        self.scans = torch.zeros(tuple(scan_shape), dtype=scan_dtype, device=dev)
+        self.offset = ops.window_map(self.scan_spatial, self.window, origins)[1].to(dev)
+        self.merge_ws = torch.empty((_lib.load().ssd3d_merge_windows_workspace_bytes(
+            s, self.n_windows, int(top_k), model.n_classes, int(top_k)),), dtype=torch.uint8, device=dev)
+        # [scan counts | merge status | per-window detect status | NaN bits]
+        self.wmeta = torch.zeros((s + 3,), dtype=torch.int32, device=dev)
+        self.host_wmeta = torch.zeros((s + 3,), dtype=torch.int32).pin_memory()
+        super().__init__(model, (s * self.n_windows, c) + self.window, torch.bfloat16, min_score, max_overlap, top_k,
+                         fuse_blocks=True)
+        self.n_kernels -= 1                  # the stem is inside the graph here
+
+    def _run_with_flag(self, model: "LSSD3D", flag: torch.Tensor):
+        ops.window_gather(self.scans, self.window, self.overlap, out=self.inp)
+        self._front(self.inp, self.stem_out)
+        super()._run_with_flag(model, flag)
+        ms, mo, k = self.args
+        s, k = self.n_scans, int(k)
+        self.mergebuf = torch.empty((s * k * 44,), dtype=torch.uint8, device=self.inp.device)
+        b_, s_, l_, p_ = self._views(self.mergebuf, k)
+        win = self.out
+        ops.merge_windows(win.boxes, win.scores, win.labels, win.count, s, self.scan_spatial, self.window,
+                          self.overlap, model.n_classes, ms, mo, k, offset=self.offset, workspace=self.merge_ws,
+                          out=(b_, s_, l_, p_), out_count=self.wmeta[:s], status=self.wmeta[s:s + 1])
+        self.wmeta[s + 1:].copy_(self.meta[self.n:])
+
+    def _launch(self, scans: torch.Tensor, copy_stream, compute):
+        compute.wait_event(self.cloned)          # static outputs of the previous use of this plan were consumed
+        if scans.is_cuda or copy_stream is None:
+            self.scans.copy_(scans, non_blocking=True)
+        else:
+            torch.cuda.set_stream(copy_stream)
+            try:
+                copy_stream.wait_event(self.done)    # the previous gather that read this buffer has run
+                self.scans.copy_(scans, non_blocking=True)
+                self.copied.record(copy_stream)
+            finally:
+                torch.cuda.set_stream(compute)
+            compute.wait_event(self.copied)
+        self.graph.replay()
+        ops.LAUNCHES[0] += self.n_kernels
+        self.host_wmeta.copy_(self.wmeta, non_blocking=True)
+        self.done.record(compute)
+
+    @property
+    def result_buf(self) -> torch.Tensor:
+        return self.mergebuf
+
+    def _checked_counts(self, model: "LSSD3D"):
+        meta = self.host_wmeta.tolist()
+        s = self.n_scans
+        if meta[s + 2]:
+            model._raise_on_nan_bits(meta[s + 2])
+        if (meta[s] | meta[s + 1]) & 1:
+            raise RuntimeError("detect_objects: more than %d candidates above min_score for one (image, class)"
+                               % _lib.SORT_MAX)
+        return meta[:s]
 
 
 class LSSD3D(_LightningBase):
@@ -759,6 +844,80 @@ class LSSD3D(_LightningBase):
             slot = (slot + 1) % depth
         while inflight:
             yield inflight.pop(0).results(self, post_stream, to_host, caller)
+
+    def predict_scans(self, scans, overlap: float = 0.5, scans_per_step: int = 1, to_host: bool = False):
+        """Sliding-window detection over whole scans larger than ``input_size`` -> per-scan lists (boxes, labels,
+        scores), boxes as fractions of the scan's shape (the coordinates ``gt_boxes_from_segmentation`` gives for the
+        scan's mask).  ``scans``: normalised volumes (S, C, D, H, W) on the host or the device, or a
+        ``data.DeviceDataset``.  Every scan is tiled into ``input_size`` windows (``data.window_origins``); each
+        step -- one CUDA-graph replay over ``scans_per_step`` scans -- gathers the windows, runs the network and
+        ``detect_objects`` on them as one batch, maps the detections into the scan and merges them per scan and
+        class with the same sort -> truncation -> greedy NMS -> top-k (``min_score``, ``max_overlap``, ``top_k``
+        apply per window and in the merge).  One device->host read per step; steps are pipelined over plan slots
+        like ``predict_batches``.  One window over a scan of exactly ``input_size`` gives ``predict_step``'s result."""
+        from .data import DeviceDataset, window_origins
+        if self.device.type != "cuda":
+            raise RuntimeError("LSSD3D.predict_scans needs the model on a CUDA device; there is no CPU path")
+        if self.training:
+            raise RuntimeError("predict_scans needs eval() mode (BatchNorm running statistics)")
+        vols = scans.images if isinstance(scans, DeviceDataset) else scans
+        if not isinstance(vols, torch.Tensor):
+            vols = torch.as_tensor(np.ascontiguousarray(vols))
+        if vols.dim() != 5:
+            raise ValueError("scans must be (S, C, D, H, W), got %r" % (tuple(vols.shape),))
+        if int(vols.shape[1]) != int(self.input_channels):
+            raise ValueError("scans have %d channels, the model takes %d" % (int(vols.shape[1]), self.input_channels))
+        nd, nh, nw, _ = window_origins(vols.shape[2:], self.input_size, overlap)
+        if ops.detect_needs_long_lists(nd * nh * nw * int(self.top_k), self.top_k):
+            raise ValueError("top_k = %d over %d windows needs the any-length merge, which is not supported; lower "
+                             "top_k or the window count" % (int(self.top_k), nd * nh * nw))
+        if vols.dtype not in (torch.float32, torch.bfloat16):
+            vols = vols.float()
+        per = max(1, int(scans_per_step))
+        if self.__dict__.get("_copy_stream") is None:
+            self.__dict__["_copy_stream"] = torch.cuda.Stream(device=self.device)
+            self.__dict__["_post_stream"] = torch.cuda.Stream(device=self.device)
+        copy_stream, post_stream = self.__dict__["_copy_stream"], self.__dict__["_post_stream"]
+        caller = torch.cuda.current_stream()
+        # a step is a whole window batch: two in flight overlap one step's tail with the next one's big layers
+        depth = max(1, min(2, int(self.pipeline_depth)))
+        boxes, labels, scores = [], [], []
+
+        def collect(plan):
+            b, l, s = plan.results(self, post_stream, to_host, caller)
+            boxes.extend(b)
+            labels.extend(l)
+            scores.extend(s)
+
+        inflight, slot = [], 0
+        for first in range(0, int(vols.shape[0]), per):
+            chunk = vols[first:first + per]
+            if not chunk.is_cuda:
+                chunk = chunk.contiguous().pin_memory()
+            if len(inflight) == depth:
+                collect(inflight.pop(0))
+            plan = self._window_plan_for(tuple(chunk.shape), chunk.dtype, overlap, slot)
+            plan.launch(chunk, copy_stream, own_stream=True, caller_stream=caller)
+            inflight.append(plan)
+            slot = (slot + 1) % depth
+        while inflight:
+            collect(inflight.pop(0))
+        return boxes, labels, scores
+
+    def _window_plan_for(self, shape, dtype, overlap, slot: int) -> _WindowPlan:
+        if self.training:
+            raise RuntimeError("predict_scans needs eval() mode (BatchNorm running statistics)")
+        key = ("windows", shape, dtype, float(overlap), str(self.device), float(self.min_score),
+               float(self.max_overlap), int(self.top_k), slot)
+        ver = self._state_version()
+        plan = self._plans.get(key)
+        if plan is None or plan.key != ver:
+            if len(self._plans) > 24:
+                self._plans.clear()
+            plan = _WindowPlan(self, shape, dtype, overlap, self.min_score, self.max_overlap, self.top_k)
+            plan.key = ver
+            self._plans[key] = plan
+        return plan
 
     def _predict_step_eager(self, image):
         prev = self.defer_nan_check
