@@ -512,6 +512,40 @@ int ssd3d_gt_boxes_from_instances(const void* seg, int seg_dtype, int N, int D, 
  *         global slot, boxes of the subject}.
  * d, h, w <= Ds, Hs, Ws; w % 16 == 0 (16-byte stores); probabilities in [0, 1].
  *
+ * ssd3d_augment_affine_batch is ssd3d_augment_batch with a random rotation and zoom of the crop, resampled from the
+ * whole source volume, in the same single launch.  Same arguments plus affine_prob in [0, 1] and the host arrays
+ * rotate_range[3] (radians, each in [0, pi]) and zoom_range[3] (each in [0, 1)); anything else (NaN included) is
+ * SSD3D_ERR_ARG before any CUDA call.  Calls 0-3 and record words 0-15 are exactly those of ssd3d_augment_batch for
+ * the same state, and the state advances the same way.  Two more calls per slot:
+ *   call 4 {affine u, theta0 u, theta1 u, theta2 u}, call 5 {z0 u, z1 u, z2 u, -}
+ * The affine is applied when u01 < affine_prob, with theta_i = fp32_rn(rotate_range[i] * fp32_rn(fp32_rn(2 u01) - 1))
+ * and z_a = fp32_rn(1 + fp32_rn(zoom_range[a] * fp32_rn(fp32_rn(2 u01) - 1))); a slot without it records theta = 0,
+ * z = 1 and M = I.  Axes are indexed (d, h, w) = (0, 1, 2).  With c_i = cos theta_i, s_i = sin theta_i (device
+ * sincosf, fp32):
+ *   R0 = [[1, 0, 0], [0, c0, -s0], [0, s0, c0]]    rotation in the (h, w) plane
+ *   R1 = [[c1, 0, -s1], [0, 1, 0], [s1, 0, c1]]    rotation in the (d, w) plane
+ *   R2 = [[c2, -s2, 0], [s2, c2, 0], [0, 0, 1]]    rotation in the (d, h) plane
+ *   (in every plane (lo, hi): R[lo][lo] = R[hi][hi] = c, R[lo][hi] = -s, R[hi][lo] = s)
+ *   R = (R0 R1) R2 and M[a][c] = fp32_rn(R[a][c] / z_c), i.e. M = R diag(1/z), every product entry
+ *   fp32_rn(fp32_rn(A[i][0] B[0][j] + A[i][1] B[1][j]) + A[i][2] B[2][j]).  A zoom above 1 magnifies.
+ * M is computed once per slot on the device and recorded (device sincosf is not numpy's).  Per output voxel:
+ *   1. the crop -> rot90 -> flip signed permutation of ssd3d_augment_batch maps the output index to the crop
+ *      index p (integers; the crop has extent n_c = (d, h, w)[c] on source axis c);
+ *   2. u_c = p_c - (n_c - 1) / 2 (exact in fp32);
+ *   3. x_a = fp32_rn(fp32_rn(fp32_rn(M[a][0] u_0 + M[a][1] u_1) + M[a][2] u_2) + (o_a + (n_a - 1) / 2)), every
+ *      product rounded separately (no FMA), o the crop offset of record words 1-3: a rotation about the crop
+ *      centre, sampling the whole source;
+ *   4. image: trilinear with i = floor(x), t = x - i (exact); a tap outside [0, S_a - 1] on any axis reads 0
+ *      (MONAI padding_mode "zeros"), a bf16 source is read as its fp32 value; lerp along W, then H, then D,
+ *      lerp(v0, v1, t) = fp32_rn(fp32_rn(v0 * fp32_rn(1 - t)) + fp32_rn(v1 * t)); the channels share the
+ *      coordinates; then step 4 (intensity, bf16 round) of ssd3d_augment_batch;
+ *   5. mask: nearest, index floor(fp32_rn(x + 0.5)) per axis, 0 outside the source.
+ * With M = I the output equals ssd3d_augment_batch's (coordinates are integers, t = 0; equal values for finite
+ * data).  The positive crop still picks a window that holds the lesion box before the affine; the lesion can then
+ * partly leave the view, and nearest resampling can split a thin lesion into several components.
+ *   record (N, 32) int32: words 0-15 as ssd3d_augment_batch, 16 affine drawn, 17-19 theta (fp32 bits), 20-22 z
+ *         (fp32 bits), 23-31 M row-major (row = source axis, column = crop axis; fp32 bits).
+ *
  * ssd3d_gt_pack turns the per-image output of ssd3d_gt_boxes_from_segmentation (boxes (N, max_boxes, 6), labels
  * (N, max_boxes), counts, n_components) into the packed ground truth of the training step: gt_boxes
  * (N * per_volume, 6), gt_labels (N * per_volume) int64 and offsets (N + 1) int32 (the ssd3d_match_priors input),
@@ -525,6 +559,12 @@ int ssd3d_augment_batch(const void* src, int src_is_bf16, const uint8_t* masks, 
                         int d, int h, int w, float pos_ratio, float flip_prob, float rot90_prob, int rot_axis0,
                         int rot_axis1, float scale, float shift, void* out, uint8_t* out_mask, int32_t* record,
                         void* stream);
+int ssd3d_augment_affine_batch(const void* src, int src_is_bf16, const uint8_t* masks, int S, int C, int Ds, int Hs,
+                               int Ws, const int32_t* order, int64_t* state, const int32_t* boxes,
+                               const int32_t* box_offsets, int N, int d, int h, int w, float pos_ratio,
+                               float flip_prob, float rot90_prob, int rot_axis0, int rot_axis1, float scale,
+                               float shift, float affine_prob, const float* rotate_range, const float* zoom_range,
+                               void* out, uint8_t* out_mask, int32_t* record, void* stream);
 int ssd3d_gt_pack(const float* boxes, const int64_t* labels, const int32_t* counts, const int32_t* n_components,
                   int N, int max_boxes, int per_volume, float* gt_boxes, int64_t* gt_labels, int32_t* offsets,
                   int32_t* status, void* stream);

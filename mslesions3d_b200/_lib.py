@@ -122,6 +122,9 @@ SIGNATURES = {
     # ---- training batches from a device-resident data set ----
     "ssd3d_augment_batch": (c_int, [P, c_int, P, c_int, c_int, c_int, c_int, c_int, P, P, P, P, c_int, c_int, c_int,
                                     c_int, c_float, c_float, c_float, c_int, c_int, c_float, c_float, P, P, P, P]),
+    "ssd3d_augment_affine_batch": (c_int, [P, c_int, P, c_int, c_int, c_int, c_int, c_int, P, P, P, P, c_int, c_int,
+                                           c_int, c_int, c_float, c_float, c_float, c_int, c_int, c_float, c_float,
+                                           c_float, P, P, P, P, P, P]),
     "ssd3d_gt_pack": (c_int, [P, P, P, P, c_int, c_int, c_int, P, P, P, P, P]),
     # ---- sliding-window inference ----
     "ssd3d_window_gather": (c_int, [P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,

@@ -75,6 +75,31 @@ __device__ void aug_draw(const AugArgs& a, const long long* __restrict__ state, 
   rec[15] = nb;
 }
 
+// the geometry of record rec as a signed permutation: crop axis c takes output axis q[c], reversed or not -- rot90
+// first (np.rot90 on the crop), then the flips of the output axes
+__device__ __forceinline__ void aug_perm(const AugArgs& a, const int* rec, int* q, int* rev) {
+  q[0] = 0; q[1] = 1; q[2] = 2;
+  int r[3] = {0, 0, 0};
+  const int k = rec[4], a0 = a.ra0, a1 = a.ra1;
+  if (k == 1) { q[a0] = a1; q[a1] = a0; r[a1] = 1; }
+  else if (k == 2) { r[a0] = 1; r[a1] = 1; }
+  else if (k == 3) { q[a0] = a1; q[a1] = a0; r[a0] = 1; }
+#pragma unroll
+  for (int c = 0; c < 3; ++c) rev[c] = r[c] ^ rec[5 + q[c]];
+}
+
+// every block has read the state (before its own increment below): the last one advances it for the next batch
+__device__ __forceinline__ void aug_advance_state(long long* state) {
+  __threadfence();
+  const unsigned long long total = (unsigned long long)gridDim.x * gridDim.y * gridDim.z;
+  if (atomicAdd(reinterpret_cast<unsigned long long*>(state + 5), 1ull) == total - 1) {
+    state[1] += 1;
+    state[2] += 1;
+    state[5] = 0;
+    __threadfence();
+  }
+}
+
 // grid: (tiles over (tile axis, W), AUG_YB-plane groups of the remaining axis, N); 256 threads
 template <typename TIn>
 __global__ void __launch_bounds__(256) augment_kernel(AugArgs a, const TIn* __restrict__ src,
@@ -90,19 +115,13 @@ __global__ void __launch_bounds__(256) augment_kernel(AugArgs a, const TIn* __re
   const int ext[3] = {a.d, a.h, a.w};
   if (tid == 0) {
     aug_draw(a, state, order, boxes, box_off, b, rec);
-    // crop axis c takes output axis q[c], reversed or not: rot90 first (np.rot90 on the crop), then the flips of
-    // the output axes
-    int q[3] = {0, 1, 2}, rev[3] = {0, 0, 0};
-    const int k = rec[4], a0 = a.ra0, a1 = a.ra1;
-    if (k == 1) { q[a0] = a1; q[a1] = a0; rev[a1] = 1; }
-    else if (k == 2) { rev[a0] = 1; rev[a1] = 1; }
-    else if (k == 3) { q[a0] = a1; q[a1] = a0; rev[a0] = 1; }
+    int q[3], rev[3];
+    aug_perm(a, rec, q, rev);
     const long long ss[3] = {(long long)a.Hs * a.Ws, (long long)a.Ws, 1};
     long long base = 0;
     for (int c = 0; c < 3; ++c) {
-      const int r = rev[c] ^ rec[5 + q[c]];
-      base += (long long)(rec[1 + c] + (r ? ext[q[c]] - 1 : 0)) * ss[c];
-      s_coef[q[c]] = r ? -ss[c] : ss[c];
+      base += (long long)(rec[1 + c] + (rev[c] ? ext[q[c]] - 1 : 0)) * ss[c];
+      s_coef[q[c]] = rev[c] ? -ss[c] : ss[c];
     }
     s_base = base;
     if (blockIdx.x == 0 && blockIdx.y == 0) for (int i = 0; i < 16; ++i) record[b * 16 + i] = rec[i];
@@ -160,17 +179,176 @@ __global__ void __launch_bounds__(256) augment_kernel(AugArgs a, const TIn* __re
       __syncthreads();
     }
   }
-  // every block has read the state (before its own increment below): the last one advances it for the next batch
+  if (tid == 0) aug_advance_state(state);
+}
+
+constexpr int AFF_TW = 64;       // output tile of one warp: AFF_TW (W) x 4 (H) of one D plane; 8 voxels per lane
+constexpr int AFF_WARPS = 4;     // warps per block = D planes per tile
+constexpr int AFF_DB = 4;        // tiles along D per block (the draws are paid once for all of them)
+
+struct AffArgs {
+  float prob, rot[3], zoom[3];
+};
+
+// words 16..31 of slot b's record: affine drawn, theta, z, M (layout in include/ssd3d_b200.h)
+__device__ void affine_draw(const AugArgs& a, const AffArgs& f, const long long* __restrict__ state, int b,
+                            int* rec) {
+  const unsigned long long seed = (unsigned long long)state[0], ctr = (unsigned long long)state[1];
+  const uint32_t g = (uint32_t)(state[3] * a.N + b), k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
+  const Philox4 r4 = philox4x32_10(g, (uint32_t)ctr, (uint32_t)(ctr >> 32), 4u, k0, k1);
+  const Philox4 r5 = philox4x32_10(g, (uint32_t)ctr, (uint32_t)(ctr >> 32), 5u, k0, k1);
+  const bool on = u01(r4.v[0]) < f.prob;
+  float th[3] = {0.f, 0.f, 0.f}, z[3] = {1.f, 1.f, 1.f}, M[3][3] = {{1.f, 0.f, 0.f}, {0.f, 1.f, 0.f}, {0.f, 0.f, 1.f}};
+  if (on) {
+    float s[3], c[3];
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+      th[i] = __fmul_rn(f.rot[i], __fsub_rn(__fmul_rn(2.f, u01(r4.v[1 + i])), 1.f));
+      z[i] = __fadd_rn(1.f, __fmul_rn(f.zoom[i], __fsub_rn(__fmul_rn(2.f, u01(r5.v[i])), 1.f)));
+      sincosf(th[i], &s[i], &c[i]);
+    }
+    // R0 in the (h, w) plane, R1 in (d, w), R2 in (d, h): R[lo][lo] = R[hi][hi] = cos, R[lo][hi] = -sin, R[hi][lo] = sin
+    const float R0[3][3] = {{1.f, 0.f, 0.f}, {0.f, c[0], -s[0]}, {0.f, s[0], c[0]}};
+    const float R1[3][3] = {{c[1], 0.f, -s[1]}, {0.f, 1.f, 0.f}, {s[1], 0.f, c[1]}};
+    const float R2[3][3] = {{c[2], -s[2], 0.f}, {s[2], c[2], 0.f}, {0.f, 0.f, 1.f}};
+    float T[3][3];
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+#pragma unroll
+      for (int j = 0; j < 3; ++j)
+        T[i][j] = __fadd_rn(__fadd_rn(__fmul_rn(R0[i][0], R1[0][j]), __fmul_rn(R0[i][1], R1[1][j])),
+                            __fmul_rn(R0[i][2], R1[2][j]));
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+#pragma unroll
+      for (int j = 0; j < 3; ++j)
+        M[i][j] = __fdiv_rn(__fadd_rn(__fadd_rn(__fmul_rn(T[i][0], R2[0][j]), __fmul_rn(T[i][1], R2[1][j])),
+                                      __fmul_rn(T[i][2], R2[2][j])), z[j]);
+  }
+  rec[16] = on ? 1 : 0;
+#pragma unroll
+  for (int i = 0; i < 3; ++i) {
+    rec[17 + i] = __float_as_int(th[i]);
+    rec[20 + i] = __float_as_int(z[i]);
+  }
+#pragma unroll
+  for (int i = 0; i < 9; ++i) rec[23 + i] = __float_as_int(M[i / 3][i % 3]);
+}
+
+// fp32_rn(fp32_rn(v0 * (1 - t)) + fp32_rn(v1 * t)), omt = fp32_rn(1 - t)
+__device__ __forceinline__ float aff_lerp(float v0, float v1, float t, float omt) {
+  return __fadd_rn(__fmul_rn(v0, omt), __fmul_rn(v1, t));
+}
+
+// grid: (W tiles x H tiles of 4, groups of AFF_DB * AFF_WARPS D planes, N); 32 * AFF_WARPS threads.  Warp wz of
+// the block computes output plane od = (blockIdx.y * AFF_DB + it) * AFF_WARPS + wz, rows oh = tile_h * 4 + lane / 8,
+// voxels ow = tile_w * AFF_TW + j * 8 + lane % 8 (adjacent lanes read adjacent source voxels when M is near the
+// identity); results go through shared memory so that each lane stores 8 consecutive W voxels (one 16-byte bf16
+// store per channel, one 8-byte mask store).
+template <typename TIn>
+__global__ void __launch_bounds__(32 * AFF_WARPS) augment_affine_kernel(
+    AugArgs a, AffArgs f, const TIn* __restrict__ src, const uint8_t* __restrict__ masks,
+    const int* __restrict__ order, long long* __restrict__ state, const int* __restrict__ boxes,
+    const int* __restrict__ box_off, __nv_bfloat16* __restrict__ out, uint8_t* __restrict__ out_mask,
+    int* __restrict__ record) {
+  __shared__ int rec[32];
+  __shared__ int s_q[3], s_rev[3];
+  __shared__ __align__(16) __nv_bfloat16 s_img[AFF_WARPS][4][AFF_TW];
+  __shared__ __align__(16) uint8_t s_msk[AFF_WARPS][4][AFF_TW];
+  const int tid = threadIdx.x, b = blockIdx.z, lane = tid & 31, wz = tid >> 5, tx = lane & 7, ty = lane >> 3;
   if (tid == 0) {
-    __threadfence();
-    const unsigned long long total = (unsigned long long)gridDim.x * gridDim.y * gridDim.z;
-    if (atomicAdd(reinterpret_cast<unsigned long long*>(state + 5), 1ull) == total - 1) {
-      state[1] += 1;
-      state[2] += 1;
-      state[5] = 0;
-      __threadfence();
+    aug_draw(a, state, order, boxes, box_off, b, rec);
+    affine_draw(a, f, state, b, rec);
+    int q[3], rev[3];
+    aug_perm(a, rec, q, rev);
+    for (int c = 0; c < 3; ++c) { s_q[c] = q[c]; s_rev[c] = rev[c]; }
+    if (blockIdx.x == 0 && blockIdx.y == 0) for (int i = 0; i < 32; ++i) record[b * 32 + i] = rec[i];
+  }
+  __syncthreads();
+  const int ext[3] = {a.d, a.h, a.w}, srcx[3] = {a.Ds, a.Hs, a.Ws};
+  float M[3][3], half[3], cen[3];
+  int q[3], rev[3];
+#pragma unroll
+  for (int c = 0; c < 3; ++c) {
+    q[c] = s_q[c];
+    rev[c] = s_rev[c];
+    half[c] = __fmul_rn(0.5f, (float)(ext[c] - 1));                       // (n_c - 1) / 2, exact
+    cen[c] = __fadd_rn((float)rec[1 + c], half[c]);                       // o_c + (n_c - 1) / 2, exact
+#pragma unroll
+    for (int j = 0; j < 3; ++j) M[c][j] = __int_as_float(rec[23 + c * 3 + j]);
+  }
+  const int subj = rec[0];
+  const float scale1 = __fadd_rn(1.f, __int_as_float(rec[10])), shift = __int_as_float(rec[11]);
+  const int plane = a.Hs * a.Ws;
+  const long long vox_s = (long long)a.Ds * plane, vox_o = (long long)a.d * a.h * a.w;
+  const uint8_t* msrc = masks + (long long)subj * vox_s;
+  const TIn* isrc = src + (long long)subj * a.C * vox_s;
+  const int tiles_w = (a.w + AFF_TW - 1) / AFF_TW;
+  const int oh = (blockIdx.x / tiles_w) * 4 + ty, ow_t = (blockIdx.x % tiles_w) * AFF_TW;
+  for (int it = 0; it < AFF_DB; ++it) {
+    const int od = (blockIdx.y * AFF_DB + it) * AFF_WARPS + wz;
+    if (od >= a.d) break;                                                 // warp-uniform
+    const bool row = oh < a.h;
+    const bool store = row && ow_t + tx * 8 < a.w;
+    const long long obase = (long long)od * a.h * a.w + (long long)oh * a.w + ow_t + tx * 8;
+    // the coordinates are recomputed per channel: cheaper than holding 8 voxels' taps and weights in registers
+    for (int ch = 0; ch < a.C; ++ch) {
+      const TIn* sc = isrc + (long long)ch * vox_s;
+#pragma unroll 4
+      for (int j = 0; j < 8; ++j) {
+        const int o[3] = {od, oh, ow_t + j * 8 + tx};
+        const bool live = row && o[2] < a.w;
+        float u[3];
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+          const int oq = o[q[c]];
+          u[c] = __fsub_rn((float)(rev[c] ? ext[c] - 1 - oq : oq), half[c]);
+        }
+        int i0[3], nn[3];
+        bool lo[3], hi[3];
+        float t[3];
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+          const float x = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(M[c][0], u[0]), __fmul_rn(M[c][1], u[1])),
+                                              __fmul_rn(M[c][2], u[2])), cen[c]);
+          const float fl = floorf(x);
+          i0[c] = (int)fl;
+          t[c] = __fsub_rn(x, fl);
+          nn[c] = (int)floorf(__fadd_rn(x, 0.5f));
+          lo[c] = i0[c] >= 0 && i0[c] < srcx[c];                           // tap i0 inside the source
+          hi[c] = i0[c] >= -1 && i0[c] < srcx[c] - 1;                      // tap i0 + 1 inside the source
+        }
+        if (ch == 0) {
+          const bool in = live && nn[0] >= 0 && nn[0] < a.Ds && nn[1] >= 0 && nn[1] < a.Hs && nn[2] >= 0 &&
+                          nn[2] < a.Ws;
+          s_msk[wz][ty][j * 8 + tx] = in ? __ldg(msrc + (nn[0] * a.Hs + nn[1]) * a.Ws + nn[2]) : (uint8_t)0;
+        }
+        const int base = (i0[0] * a.Hs + i0[1]) * a.Ws + i0[2];
+        float v[8];                                                         // taps (dd, dh, dw), dw fastest
+#pragma unroll
+        for (int k = 0; k < 8; ++k) {
+          const int dd = k >> 2, dh = (k >> 1) & 1, dw = k & 1;
+          const bool ok = live && (dd ? hi[0] : lo[0]) && (dh ? hi[1] : lo[1]) && (dw ? hi[2] : lo[2]);
+          v[k] = ok ? (float)__ldg(sc + base + dd * plane + dh * a.Ws + dw) : 0.f;
+        }
+        const float mw = __fsub_rn(1.f, t[2]), mh = __fsub_rn(1.f, t[1]), md = __fsub_rn(1.f, t[0]);
+        const float c00 = aff_lerp(v[0], v[1], t[2], mw), c01 = aff_lerp(v[2], v[3], t[2], mw);
+        const float c10 = aff_lerp(v[4], v[5], t[2], mw), c11 = aff_lerp(v[6], v[7], t[2], mw);
+        const float val = aff_lerp(aff_lerp(c00, c01, t[1], mh), aff_lerp(c10, c11, t[1], mh), t[0], md);
+        s_img[wz][ty][j * 8 + tx] = __float2bfloat16_rn(__fadd_rn(__fmul_rn(val, scale1), shift));
+      }
+      __syncwarp();
+      if (store) {
+        *reinterpret_cast<uint4*>(out + ((long long)b * a.C + ch) * vox_o + obase) =
+            *reinterpret_cast<const uint4*>(&s_img[wz][ty][tx * 8]);
+        if (ch == 0)
+          *reinterpret_cast<uint2*>(out_mask + b * vox_o + obase) =
+              *reinterpret_cast<const uint2*>(&s_msk[wz][ty][tx * 8]);
+      }
+      __syncwarp();
     }
   }
+  if (tid == 0) aug_advance_state(state);
 }
 
 // one block: per-volume overflow test, offsets (exclusive scan of the counts) and the row copy
@@ -211,11 +389,12 @@ __global__ void __launch_bounds__(256) gt_pack_kernel(const float* __restrict__ 
 
 using namespace ssd3d;
 
-extern "C" int ssd3d_augment_batch(const void* src, int src_is_bf16, const uint8_t* masks, int S, int C, int Ds, int Hs,
-                                   int Ws, const int32_t* order, int64_t* state, const int32_t* boxes,
-                                   const int32_t* box_offsets, int N, int d, int h, int w, float pos_ratio,
-                                   float flip_prob, float rot90_prob, int rot_axis0, int rot_axis1, float scale,
-                                   float shift, void* out, uint8_t* out_mask, int32_t* record, void* stream) {
+// the argument checks shared by ssd3d_augment_batch and ssd3d_augment_affine_batch
+static int aug_check(const void* src, const uint8_t* masks, const int32_t* order, const int64_t* state,
+                     const int32_t* boxes, const int32_t* box_offsets, const void* out, const uint8_t* out_mask,
+                     const int32_t* record, int S, int C, int Ds, int Hs, int Ws, int N, int d, int h, int w,
+                     float pos_ratio, float flip_prob, float rot90_prob, int rot_axis0, int rot_axis1, float scale,
+                     float shift) {
   if (!src || !masks || !order || !state || !boxes || !box_offsets || !out || !out_mask || !record) return SSD3D_ERR_ARG;
   if (S <= 0 || C <= 0 || N <= 0 || d <= 0 || h <= 0 || w <= 0 || d > Ds || h > Hs || w > Ws) return SSD3D_ERR_ARG;
   if (!(pos_ratio >= 0.f && pos_ratio <= 1.f) || !(flip_prob >= 0.f && flip_prob <= 1.f) ||
@@ -225,6 +404,53 @@ extern "C" int ssd3d_augment_batch(const void* src, int src_is_bf16, const uint8
   const int ext[3] = {d, h, w};
   if (rot90_prob > 0.f && ext[rot_axis0] != ext[rot_axis1]) return SSD3D_ERR_ARG;
   if (w % 16 != 0 || (long long)Ds * Hs * Ws >= (1ll << 31) || h > 65535 || d > 65535) return SSD3D_ERR_UNSUPPORTED;
+  return SSD3D_OK;
+}
+
+extern "C" int ssd3d_augment_affine_batch(const void* src, int src_is_bf16, const uint8_t* masks, int S, int C, int Ds,
+                                          int Hs, int Ws, const int32_t* order, int64_t* state, const int32_t* boxes,
+                                          const int32_t* box_offsets, int N, int d, int h, int w, float pos_ratio,
+                                          float flip_prob, float rot90_prob, int rot_axis0, int rot_axis1, float scale,
+                                          float shift, float affine_prob, const float* rotate_range,
+                                          const float* zoom_range, void* out, uint8_t* out_mask, int32_t* record,
+                                          void* stream) {
+  const int rc = aug_check(src, masks, order, state, boxes, box_offsets, out, out_mask, record, S, C, Ds, Hs, Ws, N, d,
+                           h, w, pos_ratio, flip_prob, rot90_prob, rot_axis0, rot_axis1, scale, shift);
+  if (rc != SSD3D_OK) return rc;
+  if (!rotate_range || !zoom_range || !(affine_prob >= 0.f && affine_prob <= 1.f)) return SSD3D_ERR_ARG;
+  AffArgs f{affine_prob, {0.f, 0.f, 0.f}, {0.f, 0.f, 0.f}};
+  for (int i = 0; i < 3; ++i) {
+    // the negated comparisons also refuse NaN; fp32(pi) = 3.14159274f (rounded up) is accepted
+    if (!(rotate_range[i] >= 0.f && rotate_range[i] <= 3.14159274f) || !(zoom_range[i] >= 0.f && zoom_range[i] < 1.f))
+      return SSD3D_ERR_ARG;
+    f.rot[i] = rotate_range[i];
+    f.zoom[i] = zoom_range[i];
+  }
+  AugArgs a{S, C, Ds, Hs, Ws, N, d, h, w, rot_axis0, rot_axis1, 1, pos_ratio, flip_prob, rot90_prob, scale, shift};
+  const dim3 grid((unsigned)(((w + AFF_TW - 1) / AFF_TW) * ((h + 3) / 4)),
+                  (unsigned)((d + AFF_DB * AFF_WARPS - 1) / (AFF_DB * AFF_WARPS)), (unsigned)N);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (src_is_bf16)
+    augment_affine_kernel<__nv_bfloat16><<<grid, 32 * AFF_WARPS, 0, st>>>(
+        a, f, static_cast<const __nv_bfloat16*>(src), masks, order, reinterpret_cast<long long*>(state), boxes,
+        box_offsets, static_cast<__nv_bfloat16*>(out), out_mask, record);
+  else
+    augment_affine_kernel<float><<<grid, 32 * AFF_WARPS, 0, st>>>(
+        a, f, static_cast<const float*>(src), masks, order, reinterpret_cast<long long*>(state), boxes, box_offsets,
+        static_cast<__nv_bfloat16*>(out), out_mask, record);
+  SSD3D_CHECK_LAUNCH();
+  return SSD3D_OK;
+}
+
+extern "C" int ssd3d_augment_batch(const void* src, int src_is_bf16, const uint8_t* masks, int S, int C, int Ds, int Hs,
+                                   int Ws, const int32_t* order, int64_t* state, const int32_t* boxes,
+                                   const int32_t* box_offsets, int N, int d, int h, int w, float pos_ratio,
+                                   float flip_prob, float rot90_prob, int rot_axis0, int rot_axis1, float scale,
+                                   float shift, void* out, uint8_t* out_mask, int32_t* record, void* stream) {
+  const int rc = aug_check(src, masks, order, state, boxes, box_offsets, out, out_mask, record, S, C, Ds, Hs, Ws, N, d,
+                           h, w, pos_ratio, flip_prob, rot90_prob, rot_axis0, rot_axis1, scale, shift);
+  if (rc != SSD3D_OK) return rc;
+  const int ext[3] = {d, h, w};
   // Source W is read along output W, or -- after a rotation in a plane holding W -- along that plane's other
   // axis, which then is the tile axis for every draw (the planes' extents are equal, so the grid is the same)
   const int X = rot90_prob > 0.f && rot_axis0 == 2 ? rot_axis1 : (rot90_prob > 0.f && rot_axis1 == 2 ? rot_axis0 : 1);

@@ -26,11 +26,22 @@ class Augment:
 
     * crop to the model's ``input_size``: with probability ``pos_ratio`` (and only if the subject has a lesion)
       around one of its lesions, otherwise anywhere;
+    * with probability ``affine_prob``, a rotation about the crop's centre by ``theta_i ~ U(-rotate_range[i],
+      rotate_range[i])`` radians in the (h, w), (d, w) and (d, h) planes and a zoom by ``z_a ~ U(1 - zoom_range[a],
+      1 + zoom_range[a])`` per axis (above 1 magnifies), resampled from the whole source volume: trilinear for the
+      image, nearest for the mask, zeros outside the source (exact semantics: ``ssd3d_augment_affine_batch``);
     * ``np.rot90(x, k, axes=rot90_axes)``, k uniform in {1, 2, 3}, with probability ``rot90_prob``;
     * ``np.flip`` of each spatial axis with probability ``flip_prob``;
     * ``x * (1 + f) + o`` with ``f ~ U(-scale, scale)``, ``o ~ U(-shift, shift)`` per volume (shared by its channels).
 
-    ``Augment()`` on a data set of ``input_size`` volumes is the identity (up to the bf16 rounding of the input)."""
+    The corners of a rotated crop hold source data wherever the source extends past the crop (MONAI's crop-then-
+    rotate pads them); zeros appear only outside the source.  A positive crop is chosen to hold the lesion box before
+    the rotation and zoom, so the lesion can partly leave the view afterwards; the ground truth is extracted from the
+    resampled mask, so the labels always match the image.  Nearest resampling can split a thin lesion into several
+    components; a step whose volumes then exceed ``max_boxes_per_volume`` is skipped like any overflowing step.
+
+    ``Augment()`` on a data set of ``input_size`` volumes is the identity (up to the bf16 rounding of the input);
+    without the affine (``affine_prob == 0``) the batches are those of ``ssd3d_augment_batch``."""
     pos_ratio: float = 0.0
     flip_prob: float = 0.0
     rot90_prob: float = 0.0
@@ -38,16 +49,29 @@ class Augment:
     scale: float = 0.0
     shift: float = 0.0
     seed: int = 0
+    affine_prob: float = 0.0
+    rotate_range: Tuple[float, float, float] = (0.0, 0.0, 0.0)
+    zoom_range: Tuple[float, float, float] = (0.0, 0.0, 0.0)
 
     def validate(self, input_size: Sequence[int], source_size: Sequence[int]) -> None:
         """Raise ValueError unless this augmentation can turn ``source_size`` volumes into ``input_size`` ones."""
         out, src = tuple(int(v) for v in input_size), tuple(int(v) for v in source_size)
-        for name in ("pos_ratio", "flip_prob", "rot90_prob"):
+        for name in ("pos_ratio", "flip_prob", "rot90_prob", "affine_prob"):
             p = getattr(self, name)
             if not 0.0 <= p <= 1.0:
                 raise ValueError("%s=%r is not a probability in [0, 1]" % (name, p))
         if self.scale < 0 or self.shift < 0:
             raise ValueError("scale and shift are half-widths and must be >= 0")
+        for name in ("rotate_range", "zoom_range"):
+            r = getattr(self, name)
+            # a tuple: the Augment is hashed as part of the captured epoch plan's key
+            if (not isinstance(r, tuple) or len(r) != 3
+                    or not all(isinstance(v, (int, float)) and not isinstance(v, bool) for v in r)):
+                raise ValueError("%s must be a tuple of three numbers, got %r" % (name, r))
+        if not all(0.0 <= v <= math.pi for v in self.rotate_range):
+            raise ValueError("rotate_range=%r must lie in [0, pi] (radians)" % (self.rotate_range,))
+        if not all(0.0 <= v < 1.0 for v in self.zoom_range):
+            raise ValueError("zoom_range=%r must lie in [0, 1)" % (self.zoom_range,))
         if len(out) != 3 or len(src) != 3 or any(s < o for s, o in zip(src, out)):
             raise ValueError("source volumes %r are smaller than the model's input_size %r" % (src, out))
         a0, a1 = (int(v) for v in self.rot90_axes)

@@ -4,6 +4,7 @@ all arithmetic happens in ``libssd3d_b200.so``.  CPU tensors are an error, never
 """
 from __future__ import annotations
 
+import ctypes
 from typing import List, Optional, Sequence, Tuple
 
 import numpy as np
@@ -1147,6 +1148,38 @@ def augment_batch(src: torch.Tensor, masks: torch.Tensor, order: torch.Tensor, s
     masks (S, Ds, Hs, Ws) uint8, order (S) int32, state (8) int64 (advanced by the call), boxes (B, 6) int32 voxel
     boxes, box_offsets (S + 1) int32 -> (images (N, C, d, h, w) bf16, masks (N, d, h, w) uint8, record (N, 16)
     int32).  ``out``: the three output tensors to write (static buffers of a captured step)."""
+    args, out = _augment_args(src, masks, order, state, boxes, box_offsets, batch_size, out_size, pos_ratio,
+                              flip_prob, rot90_prob, rot90_axes, scale, shift, 16, out)
+    rc = _lib.load().ssd3d_augment_batch(*args, *(t.data_ptr() for t in out), _stream())
+    _lib.check(rc, "ssd3d_augment_batch")
+    LAUNCHES[0] += 1
+    return out
+
+
+def augment_affine_batch(src: torch.Tensor, masks: torch.Tensor, order: torch.Tensor, state: torch.Tensor,
+                         boxes: torch.Tensor, box_offsets: torch.Tensor, batch_size: int, out_size,
+                         pos_ratio: float = 0.0, flip_prob: float = 0.0, rot90_prob: float = 0.0, rot90_axes=(0, 1),
+                         scale: float = 0.0, shift: float = 0.0, affine_prob: float = 0.0, rotate_range=(0, 0, 0),
+                         zoom_range=(0, 0, 0), out=None):
+    """``augment_batch`` with a random rotation (``rotate_range`` radians per plane) and zoom (``zoom_range`` per
+    axis) of the crop, applied with probability ``affine_prob`` (see ``ssd3d_augment_affine_batch`` in the header)
+    -> (images, masks, record (N, 32) int32: words 0-15 those of ``augment_batch``, 16 affine drawn, 17-19 theta,
+    20-22 z, 23-31 the 3x3 matrix M, fp32 bits)."""
+    args, out = _augment_args(src, masks, order, state, boxes, box_offsets, batch_size, out_size, pos_ratio,
+                              flip_prob, rot90_prob, rot90_axes, scale, shift, 32, out)
+    rot, zoom = (ctypes.c_float * 3)(*(float(v) for v in rotate_range)), (ctypes.c_float * 3)(*(float(v) for v in
+                                                                                                 zoom_range))
+    rc = _lib.load().ssd3d_augment_affine_batch(*args, float(affine_prob), rot, zoom, *(t.data_ptr() for t in out),
+                                                _stream())
+    _lib.check(rc, "ssd3d_augment_affine_batch")
+    LAUNCHES[0] += 1
+    return out
+
+
+def _augment_args(src, masks, order, state, boxes, box_offsets, batch_size, out_size, pos_ratio, flip_prob,
+                  rot90_prob, rot90_axes, scale, shift, record_words, out):
+    """The checked leading arguments shared by ssd3d_augment_batch and ssd3d_augment_affine_batch, and the three
+    output tensors (allocated unless ``out`` is given)."""
     _need_cuda(src, masks, order, state, boxes, box_offsets)
     if src.dim() != 5 or masks.dim() != 4 or src.dtype not in (torch.float32, BF16) or masks.dtype != torch.uint8:
         raise RuntimeError("expected src (S, C, D, H, W) fp32/bf16 and masks (S, D, H, W) uint8")
@@ -1159,16 +1192,11 @@ def augment_batch(src: torch.Tensor, masks: torch.Tensor, order: torch.Tensor, s
     if out is None:
         out = (torch.empty((n, c, d, h, w), dtype=BF16, device=src.device),
                torch.empty((n, d, h, w), dtype=torch.uint8, device=src.device),
-               torch.empty((n, 16), dtype=torch.int32, device=src.device))
-    img, msk, rec = out
-    rc = _lib.load().ssd3d_augment_batch(src.data_ptr(), int(src.dtype == BF16), masks.data_ptr(), s, c, ds, hs, ws,
-                                         order.data_ptr(), state.data_ptr(), boxes.data_ptr(), box_offsets.data_ptr(),
-                                         n, d, h, w, float(pos_ratio), float(flip_prob), float(rot90_prob),
-                                         int(rot90_axes[0]), int(rot90_axes[1]), float(scale), float(shift),
-                                         img.data_ptr(), msk.data_ptr(), rec.data_ptr(), _stream())
-    _lib.check(rc, "ssd3d_augment_batch")
-    LAUNCHES[0] += 1
-    return img, msk, rec
+               torch.empty((n, record_words), dtype=torch.int32, device=src.device))
+    args = (src.data_ptr(), int(src.dtype == BF16), masks.data_ptr(), s, c, ds, hs, ws, order.data_ptr(),
+            state.data_ptr(), boxes.data_ptr(), box_offsets.data_ptr(), n, d, h, w, float(pos_ratio), float(flip_prob),
+            float(rot90_prob), int(rot90_axes[0]), int(rot90_axes[1]), float(scale), float(shift))
+    return args, tuple(out)
 
 
 def gt_pack(boxes: torch.Tensor, labels: torch.Tensor, meta: torch.Tensor, per_volume: int, out=None,
