@@ -533,13 +533,26 @@ def detect_objects_padded(locs: torch.Tensor, scores: torch.Tensor, priors: torc
     return DetectOutput(out_boxes, out_scores, out_labels, out_prior, out_count, status)
 
 
-def detect_lists(out: DetectOutput, return_prior: bool = False):
-    """Turn the padded result into the reference's three Python lists (one D2H read of the counts)."""
-    host = torch.cat([out.count, out.status]).cpu()
-    if int(host[-1]) & 1:
+def raise_on_status(nan_bits: int, detect_status: int = 0) -> None:
+    """Raise on the NaN bits a forward ORed into its flag (the reference's exceptions, ssd3d.py:95-98,255-262) and
+    on the status word of ``detect_objects`` (bit 0: an (image, class) list outgrew one sort block)."""
+    if nan_bits & _lib.NAN_BACKBONE:
+        print("Yesssss this NaN error again in the base network")
+        raise Exception("Yesssss this NaN error again in the base network")
+    if nan_bits & _lib.NAN_SCORES:
+        raise Exception("Oh no not this NaN error again... (forward SSD), CLASSES_SCORES is nan!")
+    if nan_bits & _lib.NAN_LOCS:
+        raise Exception("Oh no not this NaN error again... (forward SSD), LOCS is nan!")
+    if detect_status & 1:
         raise RuntimeError("detect_objects: more than %d candidates above min_score for one (image, class); "
                            "raise min_score (limit of this version)" % _lib.SORT_MAX)
-    counts = host[:-1].tolist()
+
+
+def detect_lists(out: DetectOutput, return_prior: bool = False):
+    """Turn the padded result into the reference's three Python lists (one D2H read of the counts)."""
+    host = torch.cat([out.count, out.status]).tolist()
+    raise_on_status(0, host[-1])
+    counts = host[:-1]
     b = [out.boxes[i, :k] for i, k in enumerate(counts)]
     l = [out.labels[i, :k] for i, k in enumerate(counts)]
     s = [out.scores[i, :k] for i, k in enumerate(counts)]

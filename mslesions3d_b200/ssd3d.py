@@ -249,32 +249,65 @@ class PredictionConvolutions(nn.Module):
 TAIL_FROM = 3   # first backbone layer of a captured inference plan on the high-priority stream
 
 
+def _checked_counts(meta: List[int], n_out: int) -> List[int]:
+    """Decode a read-back vector ``[per-output counts | detect status words | NaN bits]``: raise on its NaN bits
+    and status words, return the counts."""
+    status = 0
+    for word in meta[n_out:-1]:
+        status |= word
+    ops.raise_on_status(meta[-1], status)
+    return meta[:n_out]
+
+
 class _InferencePlan:
     """forward + detect_objects for one input signature, captured once into a CUDA graph.
 
     The network is 19 small kernels (~20 us each at the benchmark size) plus 4 detection kernels: launched
     one by one from Python the step is host-bound, so the whole sequence is recorded on first use and
-    replayed with a single launch.  Inputs are copied into a static buffer; outputs live in static buffers
-    whose per-image counts, the detect status word and the NaN flag are packed in one int32 vector that is
-    read back with a single device->host copy."""
+    replayed with a single launch.  Outputs live in static buffers; the per-output counts, the detect status
+    words and the plan's NaN word are one int32 vector that is read back with a single device->host copy.
 
-    def __init__(self, model: "LSSD3D", shape, dtype, min_score, max_overlap, top_k, fuse_blocks: bool):
+    A batch plan (``overlap`` None) takes an image batch of ``shape``.  The stem runs outside the graph, so that
+    a device-resident batch is consumed in place (no staging copy of the largest tensor of the step); a host batch
+    goes through the static input buffer.
+
+    A window plan (``overlap`` given) takes ``shape[0]`` whole scans of ``shape``: the graph also gathers their
+    ``input_size`` windows into the network's input batch (csrc/windows.cu) in front -- so the stem is inside, its
+    input being the plan's own buffer -- and merges the per-window detections into per-scan ones behind.  The scans
+    are copied into the static input buffer before each replay."""
+
+    def __init__(self, model: "LSSD3D", shape, dtype, fuse_blocks: bool, overlap: Optional[float] = None):
         dev = model.device
         self.fuse_blocks = fuse_blocks      # Blocks run as the fused depthwise->pointwise kernel where it applies
-        n = shape[0]
-        self.key = None
-        self.inp = torch.empty(shape, dtype=dtype, device=dev)
-        self.meta = torch.zeros((n + 2,), dtype=torch.int32, device=dev)
-        self.host_meta = torch.zeros((n + 2,), dtype=torch.int32).pin_memory()
-        self.args = (min_score, max_overlap, top_k)
-        self.n = n
+        self.args = (model.min_score, model.max_overlap, int(model.top_k))
+        self.inp = torch.zeros(shape, dtype=dtype, device=dev)
+        self.windowed = overlap is not None
+        if self.windowed:
+            from .data import window_origins
+            s, c = int(shape[0]), int(shape[1])
+            self.window = tuple(int(v) for v in model.input_size)
+            self.overlap = float(overlap)
+            self.scan_spatial = tuple(int(v) for v in shape[2:])
+            nd, nh, nw, origins = window_origins(self.scan_spatial, self.window, self.overlap)
+            self.offset = ops.window_map(self.scan_spatial, self.window, origins)[1].to(dev)
+            self.merge_ws = torch.empty((_lib.load().ssd3d_merge_windows_workspace_bytes(
+                s, nd * nh * nw, self.args[2], model.n_classes, self.args[2]),), dtype=torch.uint8, device=dev)
+            self.windows = torch.zeros((s * nd * nh * nw, c) + self.window, dtype=torch.bfloat16, device=dev)
+            net_in = self.windows
+        else:
+            net_in = self.inp
+        self.n, self.n_out = int(net_in.shape[0]), int(shape[0])
+        # [per-output counts | detect status (| merge status) | NaN bits]; the NaN word is the plan's own (plans may
+        # overlap), the last element of this vector
+        n_status = 2 if self.windowed else 1
+        self.meta = torch.zeros((self.n_out + n_status + 1,), dtype=torch.int32, device=dev)
+        self.host_meta = torch.zeros_like(self.meta, device="cpu").pin_memory()
+        self.flag = self.meta[-1:]
         self.out = None
-        self.graph = None
         self.done = torch.cuda.Event()       # graph + metadata read-back of the latest launch finished
         self.cloned = torch.cuda.Event()     # results of the latest launch were copied out of the static buffers
-        self.copied = torch.cuda.Event()     # the latest host batch has arrived in the static input buffer
+        self.copied = torch.cuda.Event()     # the latest host input has arrived in the static input buffer
         self.stem = model.base.features[0]
-        self.flag = torch.zeros((1,), dtype=torch.int32, device=dev)   # this plan's own NaN word: plans may overlap
         self.stream = torch.cuda.Stream(device=dev)                     # compute stream of the streaming API
         # Later stages run at higher stream priority (recorded into the graph's kernel nodes): when two batches
         # are in flight, the latency-bound tail of the older one (small maps, heads, sort/NMS: a few CTAs each)
@@ -284,8 +317,7 @@ class _InferencePlan:
         side = torch.cuda.Stream(device=dev)
         side.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(side), torch.no_grad():
-            self.inp.zero_()
-            self.stem_out = self._front(self.inp, None)   # static buffer the captured graph reads
+            self.stem_out = self.stem(net_in)   # static buffer the captured graph reads
             for _ in range(2):                # warm-up: lazy module loading, function attributes, packing
                 self._run(model)
         torch.cuda.current_stream().wait_stream(side)
@@ -294,17 +326,11 @@ class _InferencePlan:
         before = ops.LAUNCHES[0]
         with torch.no_grad(), torch.cuda.graph(graph):
             self._run(model)
-        self.n_kernels = ops.LAUNCHES[0] - before + 1  # library kernels per step (graph + the eager stem)
+        self.n_kernels = ops.LAUNCHES[0] - before     # library kernels in the graph
         self.graph = graph
 
-    def _front(self, image: torch.Tensor, out):
-        """features[0] on ``image``.  It runs outside the graph so that a device-resident batch is consumed in place
-        (no staging copy of the largest tensor of the step); a host batch goes through the static input buffer."""
-        return self.stem(image, out=out)
-
     def _run(self, model: "LSSD3D"):
-        dev = self.inp.device
-        model.base.nan_flag(dev)
+        model.base.nan_flag(self.inp.device)
         prev_flag = model.base.use_nan_flag(self.flag)
         try:
             self._run_with_flag(model, self.flag)
@@ -314,13 +340,17 @@ class _InferencePlan:
     def _run_with_flag(self, model: "LSSD3D", flag: torch.Tensor):
         dev = self.inp.device
         flag.zero_()
+        net_in = self.inp
+        if self.windowed:
+            net_in = ops.window_gather(self.inp, self.window, self.overlap, out=self.windows)
+            self.stem(net_in, out=self.stem_out)
         # Backbone on the main stream; every head forks onto its own stream as soon as its feature map
         # exists, so the head GEMMs overlap the small tail layers (which leave most SMs idle) and join
         # before detection.  Captured, these become parallel branches of the graph.
         main = torch.cuda.current_stream()
         base, pc = model.base, model.pred_convs
         keys = list(model.aspect_ratios.keys())
-        dims, _ = base.get_feature_map_infos(tuple(self.inp.shape[2:]))
+        dims, _ = base.get_feature_map_infos(tuple(net_in.shape[2:]))
         counts = [dims[k][0] * dims[k][1] * dims[k][2] * pc.n_boxes[k] for k in keys]
         offs = [int(sum(counts[:j])) for j in range(len(keys))]
         locs = torch.empty((self.n, int(sum(counts)), 6), dtype=torch.float32, device=dev)
@@ -345,21 +375,26 @@ class _InferencePlan:
         if cur is main:
             tail.wait_stream(main)
         ms, mo, k = self.args
-        k = int(k)
+        n_out = self.n_out
         # one packed result buffer (labels | prior | boxes | scores) so that handing results out is ONE copy
-        nk = self.n * k
-        self.outbuf = torch.empty((nk * (8 + 8 + 24 + 4),), dtype=torch.uint8, device=dev)
-        self.out_views = self._views(self.outbuf, k)
+        detected = torch.empty((self.n * k * 44,), dtype=torch.uint8, device=dev)
         with torch.cuda.stream(tail):
             for hs in self.head_streams:
                 tail.wait_stream(hs)
-            b_, s_, l_, p_ = self.out_views
             self.out = ops.detect_objects_padded(locs, scores, model._prior_source(dev), ms, mo, k,
-                                                 out_count=self.meta[:self.n], status=self.meta[self.n:self.n + 1],
-                                                 out=(b_, s_, l_, p_))
-            self.meta[self.n + 1:].copy_(flag)
+                                                 out_count=None if self.windowed else self.meta[:n_out],
+                                                 status=self.meta[n_out:n_out + 1], out=self._views(detected, k))
         main.wait_stream(tail)
         self.locs, self.scores = locs, scores
+        if self.windowed:
+            self.result = torch.empty((n_out * k * 44,), dtype=torch.uint8, device=dev)
+            win = self.out
+            ops.merge_windows(win.boxes, win.scores, win.labels, win.count, n_out, self.scan_spatial, self.window,
+                              self.overlap, model.n_classes, ms, mo, k, offset=self.offset, workspace=self.merge_ws,
+                              out=self._views(self.result, k), out_count=self.meta[:n_out],
+                              status=self.meta[n_out + 1:n_out + 2])
+        else:
+            self.result = detected
 
     @staticmethod
     def _views(buf: torch.Tensor, k: int):
@@ -372,76 +407,63 @@ class _InferencePlan:
         scores = buf[nk * 40:nk * 44].view(torch.float32).view(n, k)
         return boxes, scores, labels, prior
 
-    def launch(self, image: torch.Tensor, copy_stream=None, own_stream: bool = False, caller_stream=None):
-        """Queue one step: stem on the batch (a host batch is first copied in, on ``copy_stream`` if given, so
-        that the copy overlaps the previous step), replay of the captured rest, asynchronous read-back of the
-        4*(N+2) metadata bytes.  With ``own_stream`` the step runs on this plan's stream (after everything
-        already queued on the caller's stream), so that consecutive batches on different plan slots overlap:
-        the small tail layers of one batch leave most SMs idle for the big first layers of the next."""
+    def launch(self, x: torch.Tensor, copy_stream=None, own_stream: bool = False, caller_stream=None):
+        """Queue one step: a host input is first copied into the static input buffer (on ``copy_stream`` if given,
+        so that the copy overlaps the previous step), then a batch plan runs the stem, then the captured graph is
+        replayed and the read-back vector copied to the host asynchronously.  With ``own_stream`` the step runs on
+        this plan's stream (after everything already queued on the caller's stream), so that consecutive steps on
+        different plan slots overlap: the small tail layers of one step leave most SMs idle for the big first
+        layers of the next."""
         if own_stream:
             caller = caller_stream if caller_stream is not None else torch.cuda.current_stream()
             self.stream.wait_stream(caller)
             torch.cuda.set_stream(self.stream)       # (the context manager costs several current_stream() calls)
             try:
-                self._launch(image, copy_stream, self.stream)
+                self._launch(x, copy_stream, self.stream)
             finally:
                 torch.cuda.set_stream(caller)
         else:
-            self._launch(image, copy_stream, caller_stream if caller_stream is not None else torch.cuda.current_stream())
+            self._launch(x, copy_stream, caller_stream if caller_stream is not None else torch.cuda.current_stream())
 
-    def _launch(self, image: torch.Tensor, copy_stream, compute):
+    def _launch(self, x: torch.Tensor, copy_stream, compute):
         compute.wait_event(self.cloned)          # static outputs of the previous use of this plan were consumed
-        if image.is_cuda:
+        if x.is_cuda and not self.windowed:
             # the batch (or its dtype-converted temporary) was allocated on the caller's stream but is read by the
             # stem on `compute`: tell the caching allocator, or the block could be handed out again while the
             # kernel still reads it (up to pipeline_depth batches are in flight)
-            image.record_stream(compute)
-            self._front(image, self.stem_out)
+            x.record_stream(compute)
+            self.stem(x, out=self.stem_out)
         else:
-            if copy_stream is None:
-                self.inp.copy_(image, non_blocking=True)
+            if x.is_cuda or copy_stream is None:
+                self.inp.copy_(x, non_blocking=True)
             else:
                 torch.cuda.set_stream(copy_stream)
                 try:
-                    copy_stream.wait_event(self.done)    # the previous stem that read this buffer has run
-                    self.inp.copy_(image, non_blocking=True)
+                    copy_stream.wait_event(self.done)    # the previous step that read this buffer has run
+                    self.inp.copy_(x, non_blocking=True)
                     self.copied.record(copy_stream)
                 finally:
                     torch.cuda.set_stream(compute)
                 compute.wait_event(self.copied)
-            self._front(self.inp, self.stem_out)
+            if not self.windowed:
+                self.stem(self.inp, out=self.stem_out)
         self.graph.replay()
         ops.LAUNCHES[0] += self.n_kernels
         self.host_meta.copy_(self.meta, non_blocking=True)
         self.done.record(compute)
 
-    @property
-    def result_buf(self) -> torch.Tensor:
-        """The packed static output buffer that ``results`` hands out."""
-        return self.outbuf
-
-    def _checked_counts(self, model: "LSSD3D"):
-        """Per-image counts of the latest launch, after raising on its NaN bits and detect status."""
-        meta = self.host_meta.tolist()
-        if meta[-1]:
-            model._raise_on_nan_bits(meta[-1])
-        if meta[-2] & 1:
-            raise RuntimeError("detect_objects: more than %d candidates above min_score for one (image, class)"
-                               % _lib.SORT_MAX)
-        return meta[:self.n]
-
-    def results(self, model: "LSSD3D", post_stream=None, to_host: bool = False, caller_stream=None):
+    def results(self, post_stream=None, to_host: bool = False, caller_stream=None):
         """Wait for this plan's latest launch (not for later work on the stream), check the flags, and hand
-        out fresh per-image tensors: the static buffers are copied on ``post_stream`` (device clones, or
+        out fresh per-output tensors: the static buffers are copied on ``post_stream`` (device clones, or
         pinned-host copies when ``to_host``) so that the next steps already queued are not delayed."""
         self.done.synchronize()
-        counts = self._checked_counts(model)
+        counts = _checked_counts(self.host_meta.tolist(), self.n_out)
         current = caller_stream if caller_stream is not None else torch.cuda.current_stream()
         stream = post_stream if post_stream is not None else current
         if stream is not current:
             torch.cuda.set_stream(stream)
         try:
-            buf = self.result_buf.to("cpu", non_blocking=False) if to_host else self.result_buf.clone()
+            buf = self.result.to("cpu", non_blocking=False) if to_host else self.result.clone()
             self.cloned.record(stream)
         finally:
             if stream is not current:
@@ -449,83 +471,9 @@ class _InferencePlan:
         if not to_host and stream is not current:
             current.wait_event(self.cloned)      # later work on the caller's stream sees complete tensors
             buf.record_stream(current)           # allocated on `stream`, used (and eventually freed) by the caller's
-        boxes, scores, labels, _ = self._views(buf, int(self.args[2]))
+        boxes, scores, labels, _ = self._views(buf, self.args[2])
         return ([boxes[i, :k] for i, k in enumerate(counts)], [labels[i, :k] for i, k in enumerate(counts)],
                 [scores[i, :k] for i, k in enumerate(counts)])
-
-
-class _WindowPlan(_InferencePlan):
-    """Sliding-window detection over ``scan_shape[0]`` scans of one shape, captured into one CUDA graph: gather of the
-    ``input_size`` windows into the static input batch (csrc/windows.cu), the network on the window batch (the stem
-    included: its input is the plan's own buffer), per-window ``detect_objects`` and the merge into per-scan
-    detections.  Scans are copied into a static buffer before each replay; the per-scan counts, both detect status
-    words and the NaN bits are read back with one device->host copy."""
-
-    def __init__(self, model: "LSSD3D", scan_shape, scan_dtype, overlap, min_score, max_overlap, top_k):
-        from .data import window_origins
-        dev = model.device
-        s, c = int(scan_shape[0]), int(scan_shape[1])
-        self.window = tuple(int(v) for v in model.input_size)
-        self.overlap = float(overlap)
-        nd, nh, nw, origins = window_origins(scan_shape[2:], self.window, self.overlap)
-        self.n_scans, self.n_windows = s, nd * nh * nw
-        self.scan_spatial = tuple(int(v) for v in scan_shape[2:])
-        self.scans = torch.zeros(tuple(scan_shape), dtype=scan_dtype, device=dev)
-        self.offset = ops.window_map(self.scan_spatial, self.window, origins)[1].to(dev)
-        self.merge_ws = torch.empty((_lib.load().ssd3d_merge_windows_workspace_bytes(
-            s, self.n_windows, int(top_k), model.n_classes, int(top_k)),), dtype=torch.uint8, device=dev)
-        # [scan counts | merge status | per-window detect status | NaN bits]
-        self.wmeta = torch.zeros((s + 3,), dtype=torch.int32, device=dev)
-        self.host_wmeta = torch.zeros((s + 3,), dtype=torch.int32).pin_memory()
-        super().__init__(model, (s * self.n_windows, c) + self.window, torch.bfloat16, min_score, max_overlap, top_k,
-                         fuse_blocks=True)
-        self.n_kernels -= 1                  # the stem is inside the graph here
-
-    def _run_with_flag(self, model: "LSSD3D", flag: torch.Tensor):
-        ops.window_gather(self.scans, self.window, self.overlap, out=self.inp)
-        self._front(self.inp, self.stem_out)
-        super()._run_with_flag(model, flag)
-        ms, mo, k = self.args
-        s, k = self.n_scans, int(k)
-        self.mergebuf = torch.empty((s * k * 44,), dtype=torch.uint8, device=self.inp.device)
-        b_, s_, l_, p_ = self._views(self.mergebuf, k)
-        win = self.out
-        ops.merge_windows(win.boxes, win.scores, win.labels, win.count, s, self.scan_spatial, self.window,
-                          self.overlap, model.n_classes, ms, mo, k, offset=self.offset, workspace=self.merge_ws,
-                          out=(b_, s_, l_, p_), out_count=self.wmeta[:s], status=self.wmeta[s:s + 1])
-        self.wmeta[s + 1:].copy_(self.meta[self.n:])
-
-    def _launch(self, scans: torch.Tensor, copy_stream, compute):
-        compute.wait_event(self.cloned)          # static outputs of the previous use of this plan were consumed
-        if scans.is_cuda or copy_stream is None:
-            self.scans.copy_(scans, non_blocking=True)
-        else:
-            torch.cuda.set_stream(copy_stream)
-            try:
-                copy_stream.wait_event(self.done)    # the previous gather that read this buffer has run
-                self.scans.copy_(scans, non_blocking=True)
-                self.copied.record(copy_stream)
-            finally:
-                torch.cuda.set_stream(compute)
-            compute.wait_event(self.copied)
-        self.graph.replay()
-        ops.LAUNCHES[0] += self.n_kernels
-        self.host_wmeta.copy_(self.wmeta, non_blocking=True)
-        self.done.record(compute)
-
-    @property
-    def result_buf(self) -> torch.Tensor:
-        return self.mergebuf
-
-    def _checked_counts(self, model: "LSSD3D"):
-        meta = self.host_wmeta.tolist()
-        s = self.n_scans
-        if meta[s + 2]:
-            model._raise_on_nan_bits(meta[s + 2])
-        if (meta[s] | meta[s + 1]) & 1:
-            raise RuntimeError("detect_objects: more than %d candidates above min_score for one (image, class)"
-                               % _lib.SORT_MAX)
-        return meta[:s]
 
 
 class LSSD3D(_LightningBase):
@@ -700,17 +648,7 @@ class LSSD3D(_LightningBase):
         bits = int(flag.item())
         if bits:
             flag.zero_()
-        self._raise_on_nan_bits(bits)
-
-    @staticmethod
-    def _raise_on_nan_bits(bits: int):
-        if bits & _lib.NAN_BACKBONE:
-            print("Yesssss this NaN error again in the base network")
-            raise Exception("Yesssss this NaN error again in the base network")
-        if bits & _lib.NAN_SCORES:
-            raise Exception("Oh no not this NaN error again... (forward SSD), CLASSES_SCORES is nan!")
-        if bits & _lib.NAN_LOCS:
-            raise Exception("Oh no not this NaN error again... (forward SSD), LOCS is nan!")
+        ops.raise_on_status(bits)
 
     def forward(self, image):
         """image (N, Cin, D, H, W) -> locs (N,P,6), classes_scores (N,P,n_classes) fp32 (ssd3d.py:248-263).
@@ -781,22 +719,47 @@ class LSSD3D(_LightningBase):
             eng.packed.refresh()     # values were copied into the flat buffer in place
         return out
 
-    def _plan_for(self, image: torch.Tensor, slot: int = 0, fuse_blocks: bool = True) -> _InferencePlan:
+    def _plan_for(self, image: torch.Tensor, slot: int = 0, fuse_blocks: bool = True,
+                  overlap: Optional[float] = None) -> _InferencePlan:
+        """The captured plan of pipeline slot ``slot`` for ``image``: a batch, or with ``overlap`` scans to tile into
+        windows.  Plans are recaptured when the model's state changed since, and all are dropped past 24."""
         if self.training:
             raise RuntimeError("predict_step needs eval() mode (BatchNorm running statistics)")
         dtype = image.dtype if image.dtype in (torch.float32, torch.bfloat16) else torch.float32
-        key = (tuple(image.shape), dtype, str(self.device), float(self.min_score), float(self.max_overlap),
-               int(self.top_k), slot, fuse_blocks)
+        key = (tuple(image.shape), dtype, None if overlap is None else float(overlap), str(self.device),
+               float(self.min_score), float(self.max_overlap), int(self.top_k), slot, fuse_blocks)
         ver = self._state_version()
         plan = self._plans.get(key)
         if plan is None or plan.key != ver:
             if len(self._plans) > 24:
                 self._plans.clear()
-            plan = _InferencePlan(self, tuple(image.shape), dtype, self.min_score, self.max_overlap, self.top_k,
-                                  fuse_blocks)
+            plan = _InferencePlan(self, tuple(image.shape), dtype, fuse_blocks, overlap)
             plan.key = ver
             self._plans[key] = plan
         return plan
+
+    def _pipelined(self, inputs, depth: int, fuse_blocks: bool, overlap: Optional[float], to_host: bool):
+        """Generator of per-step (boxes, labels, scores) over the tensors ``inputs``, software-pipelined over ``depth``
+        plan slots: input i+1 is copied (copy stream) and launched before the host waits for step i, and step i's
+        results leave the static buffers on a third stream."""
+        if self.__dict__.get("_copy_stream") is None:
+            self.__dict__["_copy_stream"] = torch.cuda.Stream(device=self.device)
+            self.__dict__["_post_stream"] = torch.cuda.Stream(device=self.device)
+        copy_stream, post_stream = self.__dict__["_copy_stream"], self.__dict__["_post_stream"]
+        caller = torch.cuda.current_stream()
+        inflight = []
+        slot = 0
+        for x in inputs:
+            if len(inflight) == depth:
+                yield inflight.pop(0).results(post_stream, to_host, caller)
+            plan = self._plan_for(x, slot, fuse_blocks, overlap)
+            if x.dtype != plan.inp.dtype:
+                x = x.to(plan.inp.dtype)
+            plan.launch(x, copy_stream, own_stream=True, caller_stream=caller)
+            inflight.append(plan)
+            slot = (slot + 1) % depth
+        while inflight:
+            yield inflight.pop(0).results(post_stream, to_host, caller)
 
     def predict_step(self, batch, batch_idx: int = 0, dataloader_idx: int = None):
         """forward + detect_objects (ssd3d.py:692-702): eager stem + one CUDA-graph replay and a single host
@@ -809,41 +772,23 @@ class LSSD3D(_LightningBase):
             raise RuntimeError("LSSD3D.predict_step needs the model on a CUDA device; there is no CPU path")
         plan = self._plan_for(image)
         plan.launch(image if image.dtype == plan.inp.dtype else image.to(plan.inp.dtype))
-        return plan.results(self)
+        return plan.results()
 
     def predict_batches(self, batches, to_host: bool = False):
         """Generator over an iterable of batches (dicts with "img", as a DataLoader yields them) -> per-batch
         (boxes, labels, scores).  What ``Trainer.predict(model, loader)`` does in the reference
-        (predict.py:262-263), software-pipelined over two plan slots: batch i+1 is copied (copy stream) and
-        launched before the host waits for batch i, and batch i's results leave the static buffers on a
+        (predict.py:262-263), software-pipelined over ``pipeline_depth`` plan slots: batch i+1 is copied (copy
+        stream) and launched before the host waits for batch i, and batch i's results leave the static buffers on a
         third stream.  ``to_host=True`` returns CPU tensors (one device->host copy per output)."""
         if self.device.type != "cuda":
             raise RuntimeError("LSSD3D.predict_batches needs the model on a CUDA device; there is no CPU path")
-        if self.__dict__.get("_copy_stream") is None:
-            self.__dict__["_copy_stream"] = torch.cuda.Stream(device=self.device)
-            self.__dict__["_post_stream"] = torch.cuda.Stream(device=self.device)
-        copy_stream, post_stream = self.__dict__["_copy_stream"], self.__dict__["_post_stream"]
         if ops.detect_needs_long_lists(self.priors_cxcycz.shape[0], self.top_k):
             for batch in batches:          # candidate lists of any length: no captured plan, one batch at a time
                 b, l, s = self._predict_step_eager(batch["img"])
                 yield ([t.cpu() for t in b], [t.cpu() for t in l], [t.cpu() for t in s]) if to_host else (b, l, s)
             return
-        caller = torch.cuda.current_stream()
-        depth = max(1, int(self.pipeline_depth))
-        inflight = []
-        slot = 0
-        for batch in batches:
-            image = batch["img"]
-            if len(inflight) == depth:
-                yield inflight.pop(0).results(self, post_stream, to_host, caller)
-            plan = self._plan_for(image, slot, fuse_blocks=False)
-            if image.dtype != plan.inp.dtype:
-                image = image.to(plan.inp.dtype)
-            plan.launch(image, copy_stream, own_stream=True, caller_stream=caller)
-            inflight.append(plan)
-            slot = (slot + 1) % depth
-        while inflight:
-            yield inflight.pop(0).results(self, post_stream, to_host, caller)
+        yield from self._pipelined((batch["img"] for batch in batches), max(1, int(self.pipeline_depth)), False,
+                                   None, to_host)
 
     def predict_scans(self, scans, overlap: float = 0.5, scans_per_step: int = 1, to_host: bool = False):
         """Sliding-window detection over whole scans larger than ``input_size`` -> per-scan lists (boxes, labels,
@@ -874,50 +819,16 @@ class LSSD3D(_LightningBase):
         if vols.dtype not in (torch.float32, torch.bfloat16):
             vols = vols.float()
         per = max(1, int(scans_per_step))
-        if self.__dict__.get("_copy_stream") is None:
-            self.__dict__["_copy_stream"] = torch.cuda.Stream(device=self.device)
-            self.__dict__["_post_stream"] = torch.cuda.Stream(device=self.device)
-        copy_stream, post_stream = self.__dict__["_copy_stream"], self.__dict__["_post_stream"]
-        caller = torch.cuda.current_stream()
+        chunks = (vols[first:first + per] for first in range(0, int(vols.shape[0]), per))
         # a step is a whole window batch: two in flight overlap one step's tail with the next one's big layers
-        depth = max(1, min(2, int(self.pipeline_depth)))
+        steps = self._pipelined((c if c.is_cuda else c.contiguous().pin_memory() for c in chunks),
+                                max(1, min(2, int(self.pipeline_depth))), True, overlap, to_host)
         boxes, labels, scores = [], [], []
-
-        def collect(plan):
-            b, l, s = plan.results(self, post_stream, to_host, caller)
+        for b, l, s in steps:
             boxes.extend(b)
             labels.extend(l)
             scores.extend(s)
-
-        inflight, slot = [], 0
-        for first in range(0, int(vols.shape[0]), per):
-            chunk = vols[first:first + per]
-            if not chunk.is_cuda:
-                chunk = chunk.contiguous().pin_memory()
-            if len(inflight) == depth:
-                collect(inflight.pop(0))
-            plan = self._window_plan_for(tuple(chunk.shape), chunk.dtype, overlap, slot)
-            plan.launch(chunk, copy_stream, own_stream=True, caller_stream=caller)
-            inflight.append(plan)
-            slot = (slot + 1) % depth
-        while inflight:
-            collect(inflight.pop(0))
         return boxes, labels, scores
-
-    def _window_plan_for(self, shape, dtype, overlap, slot: int) -> _WindowPlan:
-        if self.training:
-            raise RuntimeError("predict_scans needs eval() mode (BatchNorm running statistics)")
-        key = ("windows", shape, dtype, float(overlap), str(self.device), float(self.min_score),
-               float(self.max_overlap), int(self.top_k), slot)
-        ver = self._state_version()
-        plan = self._plans.get(key)
-        if plan is None or plan.key != ver:
-            if len(self._plans) > 24:
-                self._plans.clear()
-            plan = _WindowPlan(self, shape, dtype, overlap, self.min_score, self.max_overlap, self.top_k)
-            plan.key = ver
-            self._plans[key] = plan
-        return plan
 
     def _predict_step_eager(self, image):
         prev = self.defer_nan_check
@@ -936,13 +847,10 @@ class LSSD3D(_LightningBase):
         out = ops.detect_objects_padded(predicted_locs, predicted_scores, priors, self.min_score, self.max_overlap,
                                         self.top_k)
         flag = self.base.nan_flag(predicted_locs.device)
-        host = torch.cat([out.count, out.status, flag]).cpu()   # the one device->host read of the step
-        if int(host[-1]):
-            self._raise_on_nan(flag)
-        if int(host[-2]) & 1:
-            raise RuntimeError("detect_objects: more than %d candidates above min_score for one (image, class)"
-                               % _lib.SORT_MAX)
-        counts = host[:-2].tolist()
+        meta = torch.cat([out.count, out.status, flag]).tolist()   # the one device->host read of the step
+        if meta[-1]:
+            flag.zero_()
+        counts = _checked_counts(meta, out.count.shape[0])
         det_boxes = [out.boxes[i, :k] for i, k in enumerate(counts)]
         det_label = [out.labels[i, :k] for i, k in enumerate(counts)]
         det_scores = [out.scores[i, :k] for i, k in enumerate(counts)]
@@ -964,17 +872,26 @@ class LSSD3D(_LightningBase):
                 mod._packed = None
         self.__dict__.get("_plans", {}).clear()
 
+    @staticmethod
+    def _distributed(world_size, allreduce):
+        """(world size, gradient all-reduce, rank) of a training call; what the caller leaves None comes from
+        torch.distributed when it is initialised."""
+        import torch.distributed as dist
+        dist_on = dist.is_available() and dist.is_initialized()
+        if world_size is None:
+            world_size = dist.get_world_size() if dist_on else 1
+        if allreduce is None and world_size > 1:
+            allreduce = dist.all_reduce
+        rank = dist.get_rank() if dist_on and world_size > 1 else 0
+        return world_size, allreduce, rank
+
     def fit_step(self, batch, world_size: int = None, allreduce=None):
         """forward + MultiBox loss + backward + (gradient all-reduce) + Adam in one call, everything on the
         device (training.py).  With torch.distributed initialised the flat gradient buffer is summed over
         ranks with one NCCL all-reduce and averaged inside the Adam kernel (DDP semantics, SURVEY.md 8e).
         Returns the (2,) device tensor [conf_loss, loc_loss]."""
         from . import training
-        import torch.distributed as dist
-        if world_size is None:
-            world_size = dist.get_world_size() if (dist.is_available() and dist.is_initialized()) else 1
-        if allreduce is None and world_size > 1:
-            allreduce = dist.all_reduce
+        world_size, allreduce, _ = self._distributed(world_size, allreduce)
         if not self.training:
             raise RuntimeError("fit_step needs train() mode")
         return training.fit_step(self, batch, world_size, allreduce)
@@ -990,15 +907,9 @@ class LSSD3D(_LightningBase):
         A step in which a volume has more than ``max_boxes_per_volume`` boxes (a crop can split a lesion) is
         skipped like a non-finite one; the epoch then raises at its end."""
         from . import training
-        import torch.distributed as dist
-        dist_on = dist.is_available() and dist.is_initialized()
-        if world_size is None:
-            world_size = dist.get_world_size() if dist_on else 1
-        if allreduce is None and world_size > 1:
-            allreduce = dist.all_reduce
+        world_size, allreduce, rank = self._distributed(world_size, allreduce)
         if not self.training:
             raise RuntimeError("fit_epoch needs train() mode")
-        rank = dist.get_rank() if dist_on and world_size > 1 else 0
         return training.fit_epoch(self, dataset, batch_size, augment, epoch, world_size, allreduce, rank,
                                   max_boxes_per_volume)
 

@@ -502,16 +502,17 @@ class _TrainPlan:
     other node), Adam and the re-packing of the bf16 weights.  Nothing in it depends on a host scalar: the step
     counter, the cosine learning-rate schedule and the skip-on-NaN decision live on the device
     (``ssd3d_adam_step_dev``).  Inputs are staged into static buffers: the image batch, the concatenated
-    ground-truth boxes / labels (capacity ``tmax`` rows) and the per-image offsets."""
+    ground-truth boxes / labels (capacity ``tmax`` rows) and the per-image offsets.  Without ``use_cuda_graph`` the
+    plan is not captured and ``_step`` runs the same step body on the staged buffers eagerly."""
 
-    def __init__(self, model, images: torch.Tensor, tmax: int, world_size: int, allreduce):
+    def __init__(self, model, shape, dtype, tmax: int, world_size: int, allreduce):
         eng = model.train_engine()
         self.flat = eng.flatten()
         dev = model.device
-        n = images.shape[0]
+        n = shape[0]
         self.n, self.tmax = n, tmax
         self.world_size, self.allreduce = world_size, allreduce
-        self.image = torch.empty(tuple(images.shape), dtype=images.dtype, device=dev)
+        self.image = torch.empty(tuple(shape), dtype=dtype, device=dev)
         self.gt_boxes = torch.zeros((tmax, 6), dtype=torch.float32, device=dev)
         self.gt_labels = torch.zeros((tmax,), dtype=torch.int64, device=dev)
         self.offsets = torch.zeros((n + 1,), dtype=torch.int32, device=dev)
@@ -634,59 +635,62 @@ def _optimizer_step(model, flat, world_size, allreduce):
     model.train_engine().packed.refresh()      # every packed weight layout for the next step: two launches
 
 
+def _install(model, key, plan: _TrainPlan) -> None:
+    """Capture ``plan`` (its inputs staged: the warm-up steps run on them) unless the model runs its steps eagerly,
+    and cache it under ``key``; at most 4 plans are kept."""
+    if model.use_cuda_graph:
+        model.invalidate_packed()
+        plan.capture(model)
+    plans = model.train_engine().plans
+    plans.pop(key, None)
+    if len(plans) >= 4:
+        plans.clear()
+    plans[key] = plan
+
+
+def _step(model, plan: _TrainPlan) -> None:
+    """One optimisation step on ``plan``'s staged inputs: its graph replayed, then the optimizer if the collective
+    could not be captured; without a graph (``use_cuda_graph`` False) the same step body runs eagerly."""
+    eng = model.train_engine()
+    if plan.allreduce is None:
+        eng.collective_mode = "none"
+    elif plan.optimizer_in_graph:
+        eng.collective_mode = "nccl all_reduce of the flat gradient, captured in the step's CUDA graph"
+    else:
+        eng.collective_mode = "all_reduce after the graph replay"
+    with torch.no_grad():
+        if plan.graph is None:
+            plan._run(model, True)
+        else:
+            plan.graph.replay()
+            ops.LAUNCHES[0] += plan.n_kernels
+            if not plan.optimizer_in_graph:
+                _optimizer_step(model, plan.flat, plan.world_size, plan.allreduce)
+
+
 def fit_step(model, batch, world_size: int = 1, allreduce=None):
     """One fused optimisation step: forward, MultiBox loss + its gradient, backward into the flat gradient
     buffer, (all-reduce), fused Adam.  Returns a (2,) device tensor [conf_loss, loc_loss] -- no host sync.
     With ``model.use_cuda_graph`` the whole step is one CUDA-graph replay."""
-    eng = model.train_engine()
-    flat = eng.flatten()
-    dev = model.device
     images, gt_boxes, gt_labels = batch["img"], batch["boxes"], batch["labels"]
     if images.dtype not in (torch.float32, torch.bfloat16):
         images = images.float()
-    eng.collective_mode = "none" if allreduce is None else ("nccl all_reduce of the flat gradient, captured in the "
-                                                            "step's CUDA graph")
-    if model.use_cuda_graph:
-        total = sum(int(b.shape[0]) for b in gt_boxes)
-        key = (tuple(images.shape), images.dtype, int(world_size), allreduce)
-        plan = eng.plans.get(key)
-        if plan is None or plan.tmax < total:
-            tmax = 64
-            while tmax < total:
-                tmax *= 2
-            plan = _TrainPlan(model, images, tmax, world_size, allreduce)
-            plan.load(images, gt_boxes, gt_labels)
-            model.invalidate_packed()
-            plan.capture(model)
-            eng.plans.pop(key, None)
-            if len(eng.plans) >= 4:
-                eng.plans.clear()
-            eng.plans[key] = plan
-        else:
-            plan.load(images, gt_boxes, gt_labels)
-        plan.graph.replay()
-        ops.LAUNCHES[0] += plan.n_kernels
-        with torch.no_grad():
-            if not plan.optimizer_in_graph:
-                eng.collective_mode = "none" if allreduce is None else "all_reduce after the graph replay"
-                _optimizer_step(model, flat, world_size, allreduce)
-            model.invalidate_packed()
-            return plan.loss.clone()
-    gt_boxes = [b.to(dev) for b in gt_boxes]
-    gt_labels = [l.to(dev) for l in gt_labels]
-    with torch.no_grad():
-        locs, scores = eng.forward(images, eng.packed)
-        lf = model.loss_fn
-        lf_m = lf.match(gt_boxes, gt_labels)
-        out, n_pos, g_locs, g_scores = ops.multibox_loss(locs, scores, lf_m["true_classes"], lf_m["true_locs"],
-                                                         alpha=float(lf.alpha), hard_negative_mining=lf.hard_negative_mining,
-                                                         neg_pos_ratio=lf.neg_pos_ratio, want_grads=True)
-        grads = _Grads(((n, p) for n, p in model.named_parameters() if p.requires_grad and n != "rescale_factors"),
-                       flat)
-        eng.backward(g_locs, g_scores, grads)
-        _optimizer_step(model, flat, world_size, allreduce)
-        model.invalidate_packed()
-    return out
+    model.train_engine().flatten()
+    total = sum(int(b.shape[0]) for b in gt_boxes)
+    key = (tuple(images.shape), images.dtype, int(world_size), allreduce, bool(model.use_cuda_graph))
+    plan = model.train_engine().plans.get(key)
+    if plan is None or plan.tmax < total:
+        tmax = 64
+        while tmax < total:
+            tmax *= 2
+        plan = _TrainPlan(model, images.shape, images.dtype, tmax, world_size, allreduce)
+        plan.load(images, gt_boxes, gt_labels)
+        _install(model, key, plan)
+    else:
+        plan.load(images, gt_boxes, gt_labels)
+    _step(model, plan)
+    model.invalidate_packed()
+    return plan.loss.clone()
 
 
 class _EpochPlan(_TrainPlan):
@@ -700,8 +704,7 @@ class _EpochPlan(_TrainPlan):
         dev = model.device
         d, h, w = (int(v) for v in model.input_size)
         c = dataset.channels
-        super().__init__(model, torch.empty((n, c, d, h, w), dtype=torch.bfloat16, device="meta"), n * per_volume,
-                         world_size, allreduce)
+        super().__init__(model, (n, c, d, h, w), torch.bfloat16, n * per_volume, world_size, allreduce)
         self.dataset, self.augment, self.per_volume = dataset, augment, per_volume
         self.mask = torch.empty((n, d, h, w), dtype=torch.uint8, device=dev)
         self.record = torch.empty((n, 32 if augment.affine_prob > 0 else 16), dtype=torch.int32, device=dev)
@@ -760,36 +763,24 @@ def fit_epoch(model, dataset, batch_size: int, augment=None, epoch: int = 0, wor
     n, per_volume = int(batch_size), int(max_boxes_per_volume)
     if n < 1 or per_volume < 1:
         raise ValueError("batch_size and max_boxes_per_volume must be >= 1")
-    eng = model.train_engine()
-    eng.flatten()
-    eng.collective_mode = "none" if allreduce is None else ("nccl all_reduce of the flat gradient, captured in the "
-                                                            "step's CUDA graph")
+    model.train_engine().flatten()
     steps = -(-len(dataset) // (n * world_size))
     key = ("epoch", id(dataset), augment, n, per_volume, tuple(model.input_size), int(world_size), int(rank),
            allreduce)
-    plan = eng.plans.get(key)
+    plan = model.train_engine().plans.get(key)
     if plan is None or plan.dataset is not dataset:
         plan = _EpochPlan(model, dataset, augment, n, per_volume, world_size, allreduce)
         plan.start_epoch(epoch, steps, rank)
-        model.invalidate_packed()
-        plan.capture(model)
-        eng.plans.pop(key, None)
-        if len(eng.plans) >= 4:
-            eng.plans.clear()
-        eng.plans[key] = plan
+        _install(model, key, plan)
     plan.start_epoch(epoch, steps, rank)
     dev = model.device
     losses = torch.empty((steps, 2), dtype=torch.float32, device=dev)
     subjects = torch.empty((steps, n), dtype=torch.int32, device=dev)
-    with torch.no_grad():
-        for i in range(steps):
-            plan.graph.replay()
-            ops.LAUNCHES[0] += plan.n_kernels
-            if not plan.optimizer_in_graph:
-                _optimizer_step(model, plan.flat, world_size, allreduce)
-            losses[i].copy_(plan.loss)
-            subjects[i].copy_(plan.record[:, 0])
-        model.invalidate_packed()
+    for i in range(steps):
+        _step(model, plan)
+        losses[i].copy_(plan.loss)
+        subjects[i].copy_(plan.record[:, 0])
+    model.invalidate_packed()
     overflows = int(plan.pack_status[1].item())         # the one host read of the epoch
     if overflows:
         raise RuntimeError("%d of %d steps had more ground-truth boxes in a volume than max_boxes_per_volume=%d (or "

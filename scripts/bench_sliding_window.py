@@ -73,7 +73,7 @@ def run_case(name, cfg, n_scans, rounds):
     with torch.no_grad():
         m.predict_scans(scans, OVERLAP)                      # capture + warm-up of both plan slots
         m.predict_step({"img": win})
-        plan = m._window_plan_for(tuple(scans[:1].shape), scans.dtype, OVERLAP, 0)
+        plan = m._plan_for(scans[:1], 0, True, OVERLAP)
         wo = plan.out
         ws = torch.empty_like(plan.merge_ws)
         out = {"scans_per_s": [], "ms_per_step": [], "gather_ms": [], "merge_ms": [], "predict_step_windows_ms": []}
