@@ -546,6 +546,41 @@ int ssd3d_gt_boxes_from_instances(const void* seg, int seg_dtype, int N, int D, 
  *   record (N, 32) int32: words 0-15 as ssd3d_augment_batch, 16 affine drawn, 17-19 theta (fp32 bits), 20-22 z
  *         (fp32 bits), 23-31 M row-major (row = source axis, column = crop axis; fp32 bits).
  *
+ * ssd3d_augment_elastic_batch is ssd3d_augment_affine_batch with a random elastic deformation of the crop: a cubic
+ * B-spline displacement field drawn per slot, in the same single launch.  Same arguments plus elastic_prob in [0, 1]
+ * and the host arrays elastic_points[3] (control points G_c per crop axis c = d, h, w, each in [4, 16]) and
+ * elastic_magnitude[3] (maximum displacement m_c in source voxels, finite, >= 0, and m_c < 0.4 s_c whenever m_c > 0,
+ * the sufficient injectivity bound s / 2.48 of a cubic B-spline field, Choi & Lee 2000); anything else (NaN
+ * included) is SSD3D_ERR_ARG before any CUDA call.  Calls 0-5 and record words 0-31 are exactly those of
+ * ssd3d_augment_affine_batch for the same state, and the state advances the same way.  More calls per slot:
+ *   call 6 {elastic u, -, -, -}: the field applies when u01 < elastic_prob;
+ *   call 7 + k {dd u, dh u, dw u, -} for control point k = (k_d G_h + k_h) G_w + k_w, displacement
+ *   P[k]_c = fp32_rn(m_c * fp32_rn(fp32_rn(2 u01) - 1)) (crop axes c = d, h, w), so draws stay a pure function of
+ *   (seed, draw counter, slot).
+ * The control points form a uniform cubic B-spline grid over the crop (extent n_c): spacing s_c = (n_c - 1) / (G_c - 3),
+ * point k_c at crop index (k_c - 1) s_c, one point outside each end.  Per crop axis, with the inverse spacing
+ * r_c = fp32_rn((G_c - 3) / (n_c - 1)) (one correctly rounded fp32 division; r_c = 0 when n_c = 1), at crop index p:
+ *   t = fp32_rn(p * r_c), j = min(floor(t), G_c - 4), f = t - j (exact), g = fp32_rn(1 - f),
+ *   B = {h(g), c(f), c(g), h(f)}, h(x) = fp32_rn(fp32_rn(fp32_rn(x * x) * x) * fp32(1/6)),
+ *   c(x) = fp32_rn(fp32_rn(fp32_rn(0.5 * fp32_rn(fp32_rn(x * x) * x)) - fp32_rn(x * x)) + fp32(2/3))
+ *   (the uniform cubic B-spline weights (1-f)^3/6, (3f^3 - 6f^2 + 4)/6, (-3f^3 + 3f^2 + 3f + 1)/6, f^3/6).
+ * The order of the 64-term sum follows the output axes: let K, R and L be the crop axes that output d, h and w read
+ * after rot90 (without rot90, K = d, R = h, L = w); then per component, every product rounded and every sum
+ * starting from +0 and adding terms in the order shown:
+ *   V[a][e] = sum_{b=0..3} fp32_rn(B_b(f_R) * P[j_K + a, j_R + b, j_L + e])       (R innermost)
+ *   T[e]    = sum_{a=0..3} fp32_rn(B_a(f_K) * V[a][e])
+ *   delta   = sum_{e=0..3} fp32_rn(B_e(f_L) * T[e])                                (L outermost)
+ * (P indexed by its K, R and L control indices).  The source coordinate is the affine one with u replaced by
+ * u + delta: u'_c = fp32_rn(u_c + delta_c), x_a = fp32_rn(fp32_rn(fp32_rn(M[a][0] u'_0 + M[a][1] u'_1) + M[a][2] u'_2)
+ * + (o_a + (n_a - 1) / 2)) -- first the crop-frame deformation, then the rotation and zoom, then the crop -> rot90 ->
+ * flip mapping of the output index to p; image taps, mask taps, zeros outside the source, intensity and the bf16
+ * round are exactly those of ssd3d_augment_affine_batch.  By construction:
+ *   a slot that does not draw the field, or with m = 0, gets delta = 0 exactly (u' = u), so its output, and words
+ *   0-31 of its record, are bit-identical to ssd3d_augment_affine_batch's;
+ *   |delta_c| <= m_c up to fp32 rounding (the weights are >= 0 and sum to 1), so a positive crop's lesion moves by at
+ *   most m source voxels more than under the affine alone.
+ *   record (N, 33) int32: words 0-31 as ssd3d_augment_affine_batch, 32 field drawn.
+ *
  * ssd3d_gt_pack turns the per-image output of ssd3d_gt_boxes_from_segmentation (boxes (N, max_boxes, 6), labels
  * (N, max_boxes), counts, n_components) into the packed ground truth of the training step: gt_boxes
  * (N * per_volume, 6), gt_labels (N * per_volume) int64 and offsets (N + 1) int32 (the ssd3d_match_priors input),
@@ -565,6 +600,13 @@ int ssd3d_augment_affine_batch(const void* src, int src_is_bf16, const uint8_t* 
                                float flip_prob, float rot90_prob, int rot_axis0, int rot_axis1, float scale,
                                float shift, float affine_prob, const float* rotate_range, const float* zoom_range,
                                void* out, uint8_t* out_mask, int32_t* record, void* stream);
+int ssd3d_augment_elastic_batch(const void* src, int src_is_bf16, const uint8_t* masks, int S, int C, int Ds, int Hs,
+                                int Ws, const int32_t* order, int64_t* state, const int32_t* boxes,
+                                const int32_t* box_offsets, int N, int d, int h, int w, float pos_ratio,
+                                float flip_prob, float rot90_prob, int rot_axis0, int rot_axis1, float scale,
+                                float shift, float affine_prob, const float* rotate_range, const float* zoom_range,
+                                float elastic_prob, const int32_t* elastic_points, const float* elastic_magnitude,
+                                void* out, uint8_t* out_mask, int32_t* record, void* stream);
 int ssd3d_gt_pack(const float* boxes, const int64_t* labels, const int32_t* counts, const int32_t* n_components,
                   int N, int max_boxes, int per_volume, float* gt_boxes, int64_t* gt_labels, int32_t* offsets,
                   int32_t* status, void* stream);

@@ -125,6 +125,9 @@ SIGNATURES = {
     "ssd3d_augment_affine_batch": (c_int, [P, c_int, P, c_int, c_int, c_int, c_int, c_int, P, P, P, P, c_int, c_int,
                                            c_int, c_int, c_float, c_float, c_float, c_int, c_int, c_float, c_float,
                                            c_float, P, P, P, P, P, P]),
+    "ssd3d_augment_elastic_batch": (c_int, [P, c_int, P, c_int, c_int, c_int, c_int, c_int, P, P, P, P, c_int, c_int,
+                                            c_int, c_int, c_float, c_float, c_float, c_int, c_int, c_float, c_float,
+                                            c_float, P, P, c_float, P, P, P, P, P, P]),
     "ssd3d_gt_pack": (c_int, [P, P, P, P, c_int, c_int, c_int, P, P, P, P, P]),
     # ---- sliding-window inference ----
     "ssd3d_window_gather": (c_int, [P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,

@@ -240,18 +240,85 @@ __device__ __forceinline__ float aff_lerp(float v0, float v1, float t, float omt
   return __fadd_rn(__fmul_rn(v0, omt), __fmul_rn(v1, t));
 }
 
+constexpr int ELA_GMAX = 16;    // control points per crop axis, at most
+constexpr int ELA_DROW = AFF_TW + 8;   // a row of the warp's field table (the pad keeps the 4 rows' lanes apart)
+
+struct ElaArgs {
+  float prob, m[3], r[3];        // r_c = fp32_rn((G_c - 3) / (n_c - 1)), 0 when n_c = 1
+  int G[3], gmax;                // gmax = max G_c: the stride of the shared tables
+};
+
+// dynamic shared memory of the field, in floats: s_v (4 rows x K x L x 3), s_t (per warp 4 rows x L x 3), s_d (per
+// warp 3 components x 4 rows x ELA_DROW), then the 4 rows' R weights and intervals
+__host__ __device__ __forceinline__ int ela_smem_floats(int gmax) {
+  return 4 * gmax * gmax * 3 + AFF_WARPS * 4 * gmax * 3 + AFF_WARPS * 3 * 4 * ELA_DROW + 4 * 4 + 4;
+}
+
+__device__ __forceinline__ int sel3(int c, int v0, int v1, int v2) { return c == 0 ? v0 : (c == 1 ? v1 : v2); }
+__device__ __forceinline__ float sel3f(int c, float v0, float v1, float v2) { return c == 0 ? v0 : (c == 1 ? v1 : v2); }
+
+// the cubic B-spline interval and weights of crop index p on an axis with inverse spacing r and G control points:
+// t = fp32_rn(p * r), j = min(floor(t), G - 4), f = t - j (exact), w = {h(1 - f), c(f), c(1 - f), h(f)} with
+// h(x) = x^3 / 6 and c(x) = x^3 / 2 - x^2 + 2 / 3, every operation rounded as written in include/ssd3d_b200.h
+__device__ __forceinline__ float bspline_h(float x) {
+  return __fmul_rn(__fmul_rn(__fmul_rn(x, x), x), 1.f / 6.f);
+}
+__device__ __forceinline__ float bspline_c(float x) {
+  const float x2 = __fmul_rn(x, x);
+  return __fadd_rn(__fsub_rn(__fmul_rn(0.5f, __fmul_rn(x2, x)), x2), 2.f / 3.f);
+}
+__device__ __forceinline__ int bspline_j(int p, float r, int G) {
+  return min((int)floorf(__fmul_rn((float)p, r)), G - 4);
+}
+__device__ __forceinline__ int bspline_w(int p, float r, int G, float* w) {
+  const float t = __fmul_rn((float)p, r);
+  const int j = min((int)floorf(t), G - 4);
+  const float f = __fsub_rn(t, (float)j), g = __fsub_rn(1.f, f);
+  w[0] = bspline_h(g);
+  w[1] = bspline_c(f);
+  w[2] = bspline_c(g);
+  w[3] = bspline_h(f);
+  return j;
+}
+
+// word 32 of slot b's record: whether the slot draws the field (Philox call 6)
+__device__ __forceinline__ int elastic_drawn(const AugArgs& a, const ElaArgs& e, const long long* __restrict__ state,
+                                             int b) {
+  const unsigned long long seed = (unsigned long long)state[0], ctr = (unsigned long long)state[1];
+  const uint32_t g = (uint32_t)(state[3] * a.N + b);
+  const Philox4 r6 = philox4x32_10(g, (uint32_t)ctr, (uint32_t)(ctr >> 32), 6u, (uint32_t)seed, (uint32_t)(seed >> 32));
+  return u01(r6.v[0]) < e.prob ? 1 : 0;
+}
+
 // grid: (W tiles x H tiles of 4, groups of AFF_DB * AFF_WARPS D planes, N); 32 * AFF_WARPS threads.  Warp wz of
 // the block computes output plane od = (blockIdx.y * AFF_DB + it) * AFF_WARPS + wz, rows oh = tile_h * 4 + lane / 8,
 // voxels ow = tile_w * AFF_TW + j * 8 + lane % 8 (adjacent lanes read adjacent source voxels when M is near the
 // identity); results go through shared memory so that each lane stores 8 consecutive W voxels (one 16-byte bf16
 // store per channel, one 8-byte mask store).
-template <typename TIn>
-__global__ void __launch_bounds__(32 * AFF_WARPS) augment_affine_kernel(
+//
+// ELASTIC (ssd3d_augment_elastic_batch) adds the B-spline displacement to the crop coordinate before M.  The crop
+// axes read from output D, H and W (K, R and L below) follow from the slot's rot90 permutation; a block's output box
+// spans 16 D planes, 4 H rows and 64 W voxels, so it touches at most G control points per axis.  The block draws
+// those once and contracts R (s_v: 4 rows x K x L x 3); each warp contracts its plane's K per iteration (s_t: 4 rows
+// x L x 3) and then sums 4 L taps per component for its 4 x 64 voxels (s_d), which the voxel loop adds to u.  That
+// nesting is the summation order the header states.  The tables are dynamic shared memory and e is the last
+// parameter, so the ELASTIC = false instantiation compiles to the same code as before the field existed.
+// (ELASTIC: at least 6 blocks per SM, which holds it to 77 registers without spills; 96 unbounded)
+template <typename TIn, bool ELASTIC>
+__global__ void __launch_bounds__(32 * AFF_WARPS, ELASTIC ? 6 : 0) augment_affine_kernel(
     AugArgs a, AffArgs f, const TIn* __restrict__ src, const uint8_t* __restrict__ masks,
     const int* __restrict__ order, long long* __restrict__ state, const int* __restrict__ boxes,
     const int* __restrict__ box_off, __nv_bfloat16* __restrict__ out, uint8_t* __restrict__ out_mask,
-    int* __restrict__ record) {
-  __shared__ int rec[32];
+    int* __restrict__ record, ElaArgs e) {
+  constexpr int RW = ELASTIC ? 33 : 32;                                   // record words
+  extern __shared__ float s_ela[];                                        // ELASTIC: ela_smem_floats(e.gmax)
+  const int gs = e.gmax;
+  float* s_v = s_ela;
+  float* s_t = s_v + 4 * gs * gs * 3;
+  float* s_d = s_t + AFF_WARPS * 4 * gs * 3;
+  float* s_wR = s_d + AFF_WARPS * 3 * 4 * ELA_DROW;
+  int* s_jR = reinterpret_cast<int*>(s_wR + 16);
+  __shared__ int rec[RW];
   __shared__ int s_q[3], s_rev[3];
   __shared__ __align__(16) __nv_bfloat16 s_img[AFF_WARPS][4][AFF_TW];
   __shared__ __align__(16) uint8_t s_msk[AFF_WARPS][4][AFF_TW];
@@ -259,10 +326,11 @@ __global__ void __launch_bounds__(32 * AFF_WARPS) augment_affine_kernel(
   if (tid == 0) {
     aug_draw(a, state, order, boxes, box_off, b, rec);
     affine_draw(a, f, state, b, rec);
+    if constexpr (ELASTIC) rec[32] = elastic_drawn(a, e, state, b);
     int q[3], rev[3];
     aug_perm(a, rec, q, rev);
     for (int c = 0; c < 3; ++c) { s_q[c] = q[c]; s_rev[c] = rev[c]; }
-    if (blockIdx.x == 0 && blockIdx.y == 0) for (int i = 0; i < 32; ++i) record[b * 32 + i] = rec[i];
+    if (blockIdx.x == 0 && blockIdx.y == 0) for (int i = 0; i < RW; ++i) record[b * RW + i] = rec[i];
   }
   __syncthreads();
   const int ext[3] = {a.d, a.h, a.w}, srcx[3] = {a.Ds, a.Hs, a.Ws};
@@ -285,9 +353,110 @@ __global__ void __launch_bounds__(32 * AFF_WARPS) augment_affine_kernel(
   const TIn* isrc = src + (long long)subj * a.C * vox_s;
   const int tiles_w = (a.w + AFF_TW - 1) / AFF_TW;
   const int oh = (blockIdx.x / tiles_w) * 4 + ty, ow_t = (blockIdx.x % tiles_w) * AFF_TW;
+  // the field's per-block set-up (ELASTIC, slot draws it): crop axes cK, cR, cL read from output D, H, W
+  bool el_on = false;
+  int revK = 0, revL = 0, GK = 4, GL = 4, kK0 = 0, kL0 = 0, nL = 4;
+  float rK = 0.f, rL = 0.f;
+  if constexpr (ELASTIC) {
+    el_on = rec[32] != 0;
+    if (el_on) {
+      const int cK = q[0] == 0 ? 0 : (q[1] == 0 ? 1 : 2), cR = q[0] == 1 ? 0 : (q[1] == 1 ? 1 : 2), cL = 3 - cK - cR;
+      const int revR = sel3(cR, rev[0], rev[1], rev[2]), GR = sel3(cR, e.G[0], e.G[1], e.G[2]);
+      const float rR = sel3f(cR, e.r[0], e.r[1], e.r[2]);
+      revK = sel3(cK, rev[0], rev[1], rev[2]);
+      revL = sel3(cL, rev[0], rev[1], rev[2]);
+      GK = sel3(cK, e.G[0], e.G[1], e.G[2]);
+      GL = sel3(cL, e.G[0], e.G[1], e.G[2]);
+      rK = sel3f(cK, e.r[0], e.r[1], e.r[2]);
+      rL = sel3f(cL, e.r[0], e.r[1], e.r[2]);
+      // the block's output box, clamped to the output; crop index p = rev ? n - 1 - o : o (n_c = ext of the output
+      // axis it reads: rot90 only swaps axes of equal extent), so the touched control points are [j(lo), j(hi) + 3]
+      const int od0 = blockIdx.y * AFF_DB * AFF_WARPS, od1 = min(od0 + AFF_DB * AFF_WARPS, a.d) - 1;
+      const int oh0 = (blockIdx.x / tiles_w) * 4, oh1 = min(oh0 + 4, a.h) - 1, ow1 = min(ow_t + AFF_TW, a.w) - 1;
+      kK0 = bspline_j(revK ? a.d - 1 - od1 : od0, rK, GK);
+      const int nK = bspline_j(revK ? a.d - 1 - od0 : od1, rK, GK) + 4 - kK0;
+      const int kR0 = bspline_j(revR ? a.h - 1 - oh1 : oh0, rR, GR);
+      const int nR = bspline_j(revR ? a.h - 1 - oh0 : oh1, rR, GR) + 4 - kR0;
+      kL0 = bspline_j(revL ? a.w - 1 - ow1 : ow_t, rL, GL);
+      nL = bspline_j(revL ? a.w - 1 - ow_t : ow1, rL, GL) + 4 - kL0;
+      if (tid < 4) {                                                      // the 4 rows' R weights
+        const int o = min(oh0 + tid, oh1);
+        s_jR[tid] = bspline_w(revR ? a.h - 1 - o : o, rR, GR, s_wR + tid * 4);
+      }
+      __syncthreads();
+      const int G1 = e.G[1], G2 = e.G[2];
+      const int sK = sel3(cK, G1 * G2, G2, 1), sR = sel3(cR, G1 * G2, G2, 1), sL = sel3(cL, G1 * G2, G2, 1);
+      // the state is read here by every thread: it cannot advance before this block has finished (aug_advance_state)
+      const unsigned long long seed = (unsigned long long)state[0], ctr = (unsigned long long)state[1];
+      const uint32_t g = (uint32_t)(state[3] * a.N + b), k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
+      for (int i = tid; i < nK * nL; i += 32 * AFF_WARPS) {
+        const int kk = i / nL, kl = i % nL;
+        float acc[4][3];
+#pragma unroll
+        for (int r = 0; r < 4; ++r)
+#pragma unroll
+          for (int c = 0; c < 3; ++c) acc[r][c] = 0.f;
+        for (int kr = kR0; kr < kR0 + nR; ++kr) {
+          // control point k of the slot: Philox call 7 + k, displacement {d, h, w} = m * (2 u01 - 1)
+          const uint32_t k = (uint32_t)((kK0 + kk) * sK + kr * sR + (kL0 + kl) * sL);
+          const Philox4 pr = philox4x32_10(g, (uint32_t)ctr, (uint32_t)(ctr >> 32), 7u + k, k0, k1);
+          float dl[3];
+#pragma unroll
+          for (int c = 0; c < 3; ++c) dl[c] = __fmul_rn(e.m[c], __fsub_rn(__fmul_rn(2.f, u01(pr.v[c])), 1.f));
+#pragma unroll
+          for (int r = 0; r < 4; ++r) {
+            const int bb = kr - s_jR[r];
+            if (bb >= 0 && bb < 4) {
+              const float wb = s_wR[r * 4 + bb];
+#pragma unroll
+              for (int c = 0; c < 3; ++c) acc[r][c] = __fadd_rn(acc[r][c], __fmul_rn(wb, dl[c]));
+            }
+          }
+        }
+#pragma unroll
+        for (int r = 0; r < 4; ++r)
+#pragma unroll
+          for (int c = 0; c < 3; ++c) s_v[((r * gs + kk) * gs + kl) * 3 + c] = acc[r][c];
+      }
+      __syncthreads();                                                    // block-uniform: el_on is the slot's
+    }
+  }
   for (int it = 0; it < AFF_DB; ++it) {
     const int od = (blockIdx.y * AFF_DB + it) * AFF_WARPS + wz;
     if (od >= a.d) break;                                                 // warp-uniform
+    if constexpr (ELASTIC) {
+      if (el_on) {                                                        // this plane's K contraction
+        float wK[4];
+        const int jK = bspline_w(revK ? a.d - 1 - od : od, rK, GK, wK) - kK0;
+        for (int i = lane; i < 4 * nL; i += 32) {
+          const int r = i / nL, kl = i % nL;
+#pragma unroll
+          for (int c = 0; c < 3; ++c) {
+            float s = 0.f;
+#pragma unroll
+            for (int ai = 0; ai < 4; ++ai)
+              s = __fadd_rn(s, __fmul_rn(wK[ai], s_v[((r * gs + jK + ai) * gs + kl) * 3 + c]));
+            s_t[((wz * 4 + r) * gs + kl) * 3 + c] = s;
+          }
+        }
+        __syncwarp();
+        // the field of the warp's 4 x 64 voxels: 4 L taps per component (voxels past the output take the last one's)
+        for (int i = lane; i < 4 * AFF_TW; i += 32) {
+          const int r = i / AFF_TW, ol = i % AFF_TW, ow = min(ow_t + ol, a.w - 1);
+          float wL[4];
+          const int jl = bspline_w(revL ? a.w - 1 - ow : ow, rL, GL, wL) - kL0;
+          const float* tr = s_t + ((wz * 4 + r) * gs + jl) * 3;
+#pragma unroll
+          for (int c = 0; c < 3; ++c) {
+            float s = 0.f;
+#pragma unroll
+            for (int ei = 0; ei < 4; ++ei) s = __fadd_rn(s, __fmul_rn(wL[ei], tr[ei * 3 + c]));
+            s_d[((wz * 3 + c) * 4 + r) * ELA_DROW + ol] = s;
+          }
+        }
+        __syncwarp();
+      }
+    }
     const bool row = oh < a.h;
     const bool store = row && ow_t + tx * 8 < a.w;
     const long long obase = (long long)od * a.h * a.w + (long long)oh * a.w + ow_t + tx * 8;
@@ -303,6 +472,13 @@ __global__ void __launch_bounds__(32 * AFF_WARPS) augment_affine_kernel(
         for (int c = 0; c < 3; ++c) {
           const int oq = o[q[c]];
           u[c] = __fsub_rn((float)(rev[c] ? ext[c] - 1 - oq : oq), half[c]);
+        }
+        if constexpr (ELASTIC) {
+          if (el_on) {                                                    // u += the field
+            const float* dr = s_d + (wz * 12 + ty) * ELA_DROW + j * 8 + tx;
+#pragma unroll
+            for (int c = 0; c < 3; ++c) u[c] = __fadd_rn(u[c], dr[c * 4 * ELA_DROW]);
+          }
         }
         int i0[3], nn[3];
         bool lo[3], hi[3];
@@ -407,6 +583,41 @@ static int aug_check(const void* src, const uint8_t* masks, const int32_t* order
   return SSD3D_OK;
 }
 
+// the affine arguments of ssd3d_augment_affine_batch and ssd3d_augment_elastic_batch
+static int aff_check(float affine_prob, const float* rotate_range, const float* zoom_range, AffArgs* f) {
+  if (!rotate_range || !zoom_range || !(affine_prob >= 0.f && affine_prob <= 1.f)) return SSD3D_ERR_ARG;
+  *f = AffArgs{affine_prob, {0.f, 0.f, 0.f}, {0.f, 0.f, 0.f}};
+  for (int i = 0; i < 3; ++i) {
+    // the negated comparisons also refuse NaN; fp32(pi) = 3.14159274f (rounded up) is accepted
+    if (!(rotate_range[i] >= 0.f && rotate_range[i] <= 3.14159274f) || !(zoom_range[i] >= 0.f && zoom_range[i] < 1.f))
+      return SSD3D_ERR_ARG;
+    f->rot[i] = rotate_range[i];
+    f->zoom[i] = zoom_range[i];
+  }
+  return SSD3D_OK;
+}
+
+// the launch of augment_affine_kernel<TIn, ELASTIC> shared by ssd3d_augment_affine_batch and ssd3d_augment_elastic_batch
+template <bool ELASTIC>
+static int aff_launch(const AugArgs& a, const AffArgs& f, const ElaArgs& e, const void* src, int src_is_bf16,
+                      const uint8_t* masks, const int32_t* order, int64_t* state, const int32_t* boxes,
+                      const int32_t* box_offsets, void* out, uint8_t* out_mask, int32_t* record, void* stream) {
+  const dim3 grid((unsigned)(((a.w + AFF_TW - 1) / AFF_TW) * ((a.h + 3) / 4)),
+                  (unsigned)((a.d + AFF_DB * AFF_WARPS - 1) / (AFF_DB * AFF_WARPS)), (unsigned)a.N);
+  const size_t smem = ELASTIC ? (size_t)ela_smem_floats(e.gmax) * sizeof(float) : 0;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (src_is_bf16)
+    augment_affine_kernel<__nv_bfloat16, ELASTIC><<<grid, 32 * AFF_WARPS, smem, st>>>(
+        a, f, static_cast<const __nv_bfloat16*>(src), masks, order, reinterpret_cast<long long*>(state), boxes,
+        box_offsets, static_cast<__nv_bfloat16*>(out), out_mask, record, e);
+  else
+    augment_affine_kernel<float, ELASTIC><<<grid, 32 * AFF_WARPS, smem, st>>>(
+        a, f, static_cast<const float*>(src), masks, order, reinterpret_cast<long long*>(state), boxes, box_offsets,
+        static_cast<__nv_bfloat16*>(out), out_mask, record, e);
+  SSD3D_CHECK_LAUNCH();
+  return SSD3D_OK;
+}
+
 extern "C" int ssd3d_augment_affine_batch(const void* src, int src_is_bf16, const uint8_t* masks, int S, int C, int Ds,
                                           int Hs, int Ws, const int32_t* order, int64_t* state, const int32_t* boxes,
                                           const int32_t* box_offsets, int N, int d, int h, int w, float pos_ratio,
@@ -417,29 +628,43 @@ extern "C" int ssd3d_augment_affine_batch(const void* src, int src_is_bf16, cons
   const int rc = aug_check(src, masks, order, state, boxes, box_offsets, out, out_mask, record, S, C, Ds, Hs, Ws, N, d,
                            h, w, pos_ratio, flip_prob, rot90_prob, rot_axis0, rot_axis1, scale, shift);
   if (rc != SSD3D_OK) return rc;
-  if (!rotate_range || !zoom_range || !(affine_prob >= 0.f && affine_prob <= 1.f)) return SSD3D_ERR_ARG;
-  AffArgs f{affine_prob, {0.f, 0.f, 0.f}, {0.f, 0.f, 0.f}};
-  for (int i = 0; i < 3; ++i) {
-    // the negated comparisons also refuse NaN; fp32(pi) = 3.14159274f (rounded up) is accepted
-    if (!(rotate_range[i] >= 0.f && rotate_range[i] <= 3.14159274f) || !(zoom_range[i] >= 0.f && zoom_range[i] < 1.f))
-      return SSD3D_ERR_ARG;
-    f.rot[i] = rotate_range[i];
-    f.zoom[i] = zoom_range[i];
+  AffArgs f;
+  if (aff_check(affine_prob, rotate_range, zoom_range, &f) != SSD3D_OK) return SSD3D_ERR_ARG;
+  const AugArgs a{S, C, Ds, Hs, Ws, N, d, h, w, rot_axis0, rot_axis1, 1, pos_ratio, flip_prob, rot90_prob, scale, shift};
+  return aff_launch<false>(a, f, ElaArgs{}, src, src_is_bf16, masks, order, state, boxes, box_offsets, out, out_mask, record,
+                         stream);
+}
+
+extern "C" int ssd3d_augment_elastic_batch(const void* src, int src_is_bf16, const uint8_t* masks, int S, int C, int Ds,
+                                           int Hs, int Ws, const int32_t* order, int64_t* state, const int32_t* boxes,
+                                           const int32_t* box_offsets, int N, int d, int h, int w, float pos_ratio,
+                                           float flip_prob, float rot90_prob, int rot_axis0, int rot_axis1,
+                                           float scale, float shift, float affine_prob, const float* rotate_range,
+                                           const float* zoom_range, float elastic_prob, const int32_t* elastic_points,
+                                           const float* elastic_magnitude, void* out, uint8_t* out_mask,
+                                           int32_t* record, void* stream) {
+  int rc = aug_check(src, masks, order, state, boxes, box_offsets, out, out_mask, record, S, C, Ds, Hs, Ws, N, d, h, w,
+                     pos_ratio, flip_prob, rot90_prob, rot_axis0, rot_axis1, scale, shift);
+  if (rc != SSD3D_OK) return rc;
+  AffArgs f;
+  if ((rc = aff_check(affine_prob, rotate_range, zoom_range, &f)) != SSD3D_OK) return rc;
+  if (!elastic_points || !elastic_magnitude || !(elastic_prob >= 0.f && elastic_prob <= 1.f)) return SSD3D_ERR_ARG;
+  ElaArgs e{elastic_prob, {0.f, 0.f, 0.f}, {0.f, 0.f, 0.f}, {4, 4, 4}, 4};
+  const int ext[3] = {d, h, w};
+  for (int c = 0; c < 3; ++c) {
+    const int G = elastic_points[c];
+    const float m = elastic_magnitude[c];
+    if (G < 4 || G > ELA_GMAX || !(m >= 0.f && m <= 3.40282347e38f)) return SSD3D_ERR_ARG;
+    // |delta| <= m < 0.4 s keeps the cubic B-spline warp injective (Choi & Lee 2000: s / 2.48)
+    if (m > 0.f && (double)m >= 0.4 * (double)(ext[c] - 1) / (double)(G - 3)) return SSD3D_ERR_ARG;
+    e.G[c] = G;
+    e.gmax = max(e.gmax, G);
+    e.m[c] = m;
+    e.r[c] = ext[c] > 1 ? (float)(G - 3) / (float)(ext[c] - 1) : 0.f;     // one correctly rounded fp32 division
   }
-  AugArgs a{S, C, Ds, Hs, Ws, N, d, h, w, rot_axis0, rot_axis1, 1, pos_ratio, flip_prob, rot90_prob, scale, shift};
-  const dim3 grid((unsigned)(((w + AFF_TW - 1) / AFF_TW) * ((h + 3) / 4)),
-                  (unsigned)((d + AFF_DB * AFF_WARPS - 1) / (AFF_DB * AFF_WARPS)), (unsigned)N);
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (src_is_bf16)
-    augment_affine_kernel<__nv_bfloat16><<<grid, 32 * AFF_WARPS, 0, st>>>(
-        a, f, static_cast<const __nv_bfloat16*>(src), masks, order, reinterpret_cast<long long*>(state), boxes,
-        box_offsets, static_cast<__nv_bfloat16*>(out), out_mask, record);
-  else
-    augment_affine_kernel<float><<<grid, 32 * AFF_WARPS, 0, st>>>(
-        a, f, static_cast<const float*>(src), masks, order, reinterpret_cast<long long*>(state), boxes, box_offsets,
-        static_cast<__nv_bfloat16*>(out), out_mask, record);
-  SSD3D_CHECK_LAUNCH();
-  return SSD3D_OK;
+  const AugArgs a{S, C, Ds, Hs, Ws, N, d, h, w, rot_axis0, rot_axis1, 1, pos_ratio, flip_prob, rot90_prob, scale, shift};
+  return aff_launch<true>(a, f, e, src, src_is_bf16, masks, order, state, boxes, box_offsets, out, out_mask, record,
+                         stream);
 }
 
 extern "C" int ssd3d_augment_batch(const void* src, int src_is_bf16, const uint8_t* masks, int S, int C, int Ds, int Hs,

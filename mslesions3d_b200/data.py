@@ -30,6 +30,11 @@ class Augment:
       rotate_range[i])`` radians in the (h, w), (d, w) and (d, h) planes and a zoom by ``z_a ~ U(1 - zoom_range[a],
       1 + zoom_range[a])`` per axis (above 1 magnifies), resampled from the whole source volume: trilinear for the
       image, nearest for the mask, zeros outside the source (exact semantics: ``ssd3d_augment_affine_batch``);
+    * with probability ``elastic_prob``, an elastic deformation of the crop before the rotation and zoom: a smooth
+      displacement field, a uniform cubic B-spline over ``elastic_points`` control points per crop axis (d, h, w)
+      whose displacements are drawn uniformly in ``[-elastic_magnitude[c], elastic_magnitude[c]]`` source voxels
+      (MONAI's ``Rand3DElasticd`` and TorchIO's ``RandomElasticDeformation`` build the same kind of field; exact
+      semantics: ``ssd3d_augment_elastic_batch``);
     * ``np.rot90(x, k, axes=rot90_axes)``, k uniform in {1, 2, 3}, with probability ``rot90_prob``;
     * ``np.flip`` of each spatial axis with probability ``flip_prob``;
     * ``x * (1 + f) + o`` with ``f ~ U(-scale, scale)``, ``o ~ U(-shift, shift)`` per volume (shared by its channels).
@@ -39,9 +44,13 @@ class Augment:
     the rotation and zoom, so the lesion can partly leave the view afterwards; the ground truth is extracted from the
     resampled mask, so the labels always match the image.  Nearest resampling can split a thin lesion into several
     components; a step whose volumes then exceed ``max_boxes_per_volume`` is skipped like any overflowing step.
+    The elastic field moves every voxel by at most ``elastic_magnitude`` per axis (the B-spline weights are a
+    partition of unity), so it moves a positive crop's lesion by at most that much more; ``validate`` keeps the
+    magnitude below 0.4 control-point spacings, where the warp cannot fold.
 
     ``Augment()`` on a data set of ``input_size`` volumes is the identity (up to the bf16 rounding of the input);
-    without the affine (``affine_prob == 0``) the batches are those of ``ssd3d_augment_batch``."""
+    without the affine and the field (``affine_prob == 0``, ``elastic_prob == 0``) the batches are those of
+    ``ssd3d_augment_batch``, and without the field those of ``ssd3d_augment_affine_batch``."""
     pos_ratio: float = 0.0
     flip_prob: float = 0.0
     rot90_prob: float = 0.0
@@ -52,11 +61,14 @@ class Augment:
     affine_prob: float = 0.0
     rotate_range: Tuple[float, float, float] = (0.0, 0.0, 0.0)
     zoom_range: Tuple[float, float, float] = (0.0, 0.0, 0.0)
+    elastic_prob: float = 0.0
+    elastic_points: Tuple[int, int, int] = (7, 7, 7)
+    elastic_magnitude: Tuple[float, float, float] = (0.0, 0.0, 0.0)
 
     def validate(self, input_size: Sequence[int], source_size: Sequence[int]) -> None:
         """Raise ValueError unless this augmentation can turn ``source_size`` volumes into ``input_size`` ones."""
         out, src = tuple(int(v) for v in input_size), tuple(int(v) for v in source_size)
-        for name in ("pos_ratio", "flip_prob", "rot90_prob", "affine_prob"):
+        for name in ("pos_ratio", "flip_prob", "rot90_prob", "affine_prob", "elastic_prob"):
             p = getattr(self, name)
             if not 0.0 <= p <= 1.0:
                 raise ValueError("%s=%r is not a probability in [0, 1]" % (name, p))
@@ -72,8 +84,24 @@ class Augment:
             raise ValueError("rotate_range=%r must lie in [0, pi] (radians)" % (self.rotate_range,))
         if not all(0.0 <= v < 1.0 for v in self.zoom_range):
             raise ValueError("zoom_range=%r must lie in [0, 1)" % (self.zoom_range,))
+        g, m = self.elastic_points, self.elastic_magnitude
+        if (not isinstance(g, tuple) or len(g) != 3
+                or not all(isinstance(v, int) and not isinstance(v, bool) and 4 <= v <= 16 for v in g)):
+            raise ValueError("elastic_points must be a tuple of three ints in [4, 16], got %r" % (g,))
+        if (not isinstance(m, tuple) or len(m) != 3
+                or not all(isinstance(v, (int, float)) and not isinstance(v, bool) and math.isfinite(v) and v >= 0
+                           for v in m)):
+            raise ValueError("elastic_magnitude must be a tuple of three finite numbers >= 0, got %r" % (m,))
         if len(out) != 3 or len(src) != 3 or any(s < o for s, o in zip(src, out)):
             raise ValueError("source volumes %r are smaller than the model's input_size %r" % (src, out))
+        for c in range(3):
+            # control-point spacing s = (n - 1) / (G - 3); |displacement| < 0.4 s keeps the cubic B-spline warp
+            # injective (the sufficient bound s / 2.48, Choi & Lee 2000)
+            limit = 0.4 * (out[c] - 1) / (g[c] - 3)
+            if m[c] > 0 and m[c] >= limit:
+                raise ValueError("elastic_magnitude[%d]=%r must stay below 0.4 control-point spacings = %g voxels "
+                                 "(input_size %d, elastic_points %d): the warp could fold"
+                                 % (c, m[c], limit, out[c], g[c]))
         a0, a1 = (int(v) for v in self.rot90_axes)
         if len(self.rot90_axes) != 2 or a0 == a1 or not (0 <= a0 <= 2 and 0 <= a1 <= 2):
             raise ValueError("rot90_axes must be two different spatial axes in 0..2, got %r" % (self.rot90_axes,))

@@ -1189,10 +1189,33 @@ def augment_affine_batch(src: torch.Tensor, masks: torch.Tensor, order: torch.Te
     return out
 
 
+def augment_elastic_batch(src: torch.Tensor, masks: torch.Tensor, order: torch.Tensor, state: torch.Tensor,
+                          boxes: torch.Tensor, box_offsets: torch.Tensor, batch_size: int, out_size,
+                          pos_ratio: float = 0.0, flip_prob: float = 0.0, rot90_prob: float = 0.0, rot90_axes=(0, 1),
+                          scale: float = 0.0, shift: float = 0.0, affine_prob: float = 0.0, rotate_range=(0, 0, 0),
+                          zoom_range=(0, 0, 0), elastic_prob: float = 0.0, elastic_points=(7, 7, 7),
+                          elastic_magnitude=(0, 0, 0), out=None):
+    """``augment_affine_batch`` with a random cubic B-spline deformation of the crop (``elastic_points`` control
+    points and at most ``elastic_magnitude`` source voxels of displacement per axis), applied with probability
+    ``elastic_prob`` (see ``ssd3d_augment_elastic_batch`` in the header) -> (images, masks, record (N, 33) int32:
+    words 0-31 those of ``augment_affine_batch``, 32 field drawn)."""
+    args, out = _augment_args(src, masks, order, state, boxes, box_offsets, batch_size, out_size, pos_ratio,
+                              flip_prob, rot90_prob, rot90_axes, scale, shift, 33, out)
+    rot, zoom = (ctypes.c_float * 3)(*(float(v) for v in rotate_range)), (ctypes.c_float * 3)(*(float(v) for v in
+                                                                                                 zoom_range))
+    pts = (ctypes.c_int32 * 3)(*(int(v) for v in elastic_points))
+    mag = (ctypes.c_float * 3)(*(float(v) for v in elastic_magnitude))
+    rc = _lib.load().ssd3d_augment_elastic_batch(*args, float(affine_prob), rot, zoom, float(elastic_prob), pts, mag,
+                                                 *(t.data_ptr() for t in out), _stream())
+    _lib.check(rc, "ssd3d_augment_elastic_batch")
+    LAUNCHES[0] += 1
+    return out
+
+
 def _augment_args(src, masks, order, state, boxes, box_offsets, batch_size, out_size, pos_ratio, flip_prob,
                   rot90_prob, rot90_axes, scale, shift, record_words, out):
-    """The checked leading arguments shared by ssd3d_augment_batch and ssd3d_augment_affine_batch, and the three
-    output tensors (allocated unless ``out`` is given)."""
+    """The checked leading arguments shared by ssd3d_augment_batch, ssd3d_augment_affine_batch and
+    ssd3d_augment_elastic_batch, and the three output tensors (allocated unless ``out`` is given)."""
     _need_cuda(src, masks, order, state, boxes, box_offsets)
     if src.dim() != 5 or masks.dim() != 4 or src.dtype not in (torch.float32, BF16) or masks.dtype != torch.uint8:
         raise RuntimeError("expected src (S, C, D, H, W) fp32/bf16 and masks (S, D, H, W) uint8")

@@ -695,8 +695,8 @@ def fit_step(model, batch, world_size: int = 1, allreduce=None):
 
 class _EpochPlan(_TrainPlan):
     """The fused step fed from a ``DeviceDataset``: the captured graph also samples and augments the batch straight
-    into the static image buffer (``ssd3d_augment_batch``, or ``ssd3d_augment_affine_batch`` when the augmentation
-    draws a rotation and zoom), extracts the ground truth of the augmented masks
+    into the static image buffer (``ssd3d_augment_batch``; ``ssd3d_augment_affine_batch`` when the augmentation
+    draws a rotation and zoom; ``ssd3d_augment_elastic_batch`` when it draws an elastic deformation), extracts the ground truth of the augmented masks
     (``ssd3d_gt_boxes_from_segmentation``) and packs it into the static GT buffers (``ssd3d_gt_pack``).  The draw
     state advances inside the graph, so every replay is the next step of the epoch with no host copy or sync."""
 
@@ -707,7 +707,8 @@ class _EpochPlan(_TrainPlan):
         super().__init__(model, (n, c, d, h, w), torch.bfloat16, n * per_volume, world_size, allreduce)
         self.dataset, self.augment, self.per_volume = dataset, augment, per_volume
         self.mask = torch.empty((n, d, h, w), dtype=torch.uint8, device=dev)
-        self.record = torch.empty((n, 32 if augment.affine_prob > 0 else 16), dtype=torch.int32, device=dev)
+        words = 33 if augment.elastic_prob > 0 else (32 if augment.affine_prob > 0 else 16)
+        self.record = torch.empty((n, words), dtype=torch.int32, device=dev)
         self.order = torch.zeros((len(dataset),), dtype=torch.int32, device=dev)
         # {seed, draw counter, step in epoch, rank, world size, kernel scratch, -, -}
         self.state = torch.zeros((8,), dtype=torch.int64, device=dev)
@@ -724,7 +725,10 @@ class _EpochPlan(_TrainPlan):
         a, ds = self.augment, self.dataset
         args = (ds.images, ds.masks, self.order, self.state, ds.boxes, ds.box_offsets, self.n, model.input_size,
                 a.pos_ratio, a.flip_prob, a.rot90_prob, a.rot90_axes, a.scale, a.shift)
-        if a.affine_prob > 0:
+        if a.elastic_prob > 0:
+            ops.augment_elastic_batch(*args, a.affine_prob, a.rotate_range, a.zoom_range, a.elastic_prob,
+                                      a.elastic_points, a.elastic_magnitude, out=(self.image, self.mask, self.record))
+        elif a.affine_prob > 0:
             ops.augment_affine_batch(*args, a.affine_prob, a.rotate_range, a.zoom_range,
                                      out=(self.image, self.mask, self.record))
         else:
