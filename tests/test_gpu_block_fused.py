@@ -6,6 +6,8 @@ import pytest
 import torch
 import torch.nn.functional as F
 
+from tests import bench_shapes as S
+
 pytestmark = pytest.mark.gpu
 
 CASES = [
@@ -19,6 +21,10 @@ CASES = [
     (128, 128, 1, 1, (5, 9, 12)),
     (128, 128, 1, 8, (16, 16, 16)),      # the benchmark's f3
 ]
+# the benchmark's f1 and f2 (batch 8, 64^3 and 32^3 inputs): the other blocks the fused kernel is built for
+# (csrc/conv_dwpw.cu:483-490)
+CASES = S.extend(CASES, [(b.cin, b.cout, b.stride, b.n, b.size) for b in S.table(S.INFER)["block"]
+                         if b.unit in ("f1", "f2", "f3")])
 
 
 def bf16r(t):

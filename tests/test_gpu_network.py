@@ -15,6 +15,7 @@ import torch
 import torch.nn.functional as F
 
 from oracle import ssd3d_oracle as O
+from tests import bench_shapes as S
 from tests.conftest import load_golden
 from tests.golden import golden_inputs as GI
 
@@ -68,7 +69,8 @@ def rand_bn(c, g):
     (2, (10, 22, 72), 2, torch.bfloat16, 2),       # banded-B kernel: ragged second row slot (Wo = 36), ragged H / D tiles
     (1, (12, 6, 128), 1, torch.bfloat16, 1),       # banded-B kernel: Ho = 3 -> 4 x 4 row slots, stride 1 along D
     (2, (33, 40, 96), 2, torch.bfloat16, 1),       # the training shape's row width (Wo = 48), odd depth
-])
+] + [(u.cin, u.size, u.stride_d, u.dtype, u.n) for u in S.table(S.INFER)["stem"]]     # the benchmark's batch of 8
+  + S.STEM_FWD_BOUNDARY)                                                              # banded-B vs gather at W = 64k
 def test_stem_conv(cin, size, sd, dtype, batch):
     ops = _ops()
     g = torch.Generator().manual_seed(cin * 100 + size[0])
@@ -83,11 +85,14 @@ def test_stem_conv(cin, size, sd, dtype, batch):
         kernels.append("tc")             # gather-based tcgen05 implicit GEMM
     if lib.ssd3d_stem_tz_supported(int(dtype == torch.bfloat16), cin, size[2]):
         kernels.append("tz")             # banded-B tcgen05 GEMM on raw TMA rows
+    got = {}
     for kernel in kernels:
-        got = ops.stem_conv_bn_relu(x.to(dtype).cuda(), ops.pack_stem_weight(w.cuda()), scale.cuda(), shift.cuda(), sd,
-                                    kernel=kernel)
-        assert got.dtype == torch.bfloat16 and got.is_contiguous(memory_format=torch.channels_last_3d)
-        assert_bf16_close(got, want, "stem %s" % (kernel or "auto"))
+        got[kernel] = ops.stem_conv_bn_relu(x.to(dtype).cuda(), ops.pack_stem_weight(w.cuda()), scale.cuda(), shift.cuda(),
+                                            sd, kernel=kernel)
+        assert got[kernel].dtype == torch.bfloat16 and got[kernel].is_contiguous(memory_format=torch.channels_last_3d)
+        assert_bf16_close(got[kernel], want, "stem %s" % (kernel or "auto"))
+    # the library's own choice is the kernel the shape selects, bit for bit
+    assert torch.equal(got[None], got[S.stem_kernel(dtype, cin, size[2])])
 
 
 @pytest.mark.parametrize("c,size,stride,batch", [
@@ -185,7 +190,7 @@ def test_pointwise_nan_flag():
     (128, (16, 16, 16), 8, 2),     # the benchmark's f3 head: kw-GEMM + stencil territory (M = 32768)
     (64, (21, 19, 23), 2, 2),      # M = 18354, ragged tiles on every axis
     (256, (16, 16, 16), 4, 2),
-])
+] + S.HEAD_KW_BOUNDARY)           # the kw-GEMM's 48- and 144-column tilings, at 147 and 148 tiles of 128 voxels
 @pytest.mark.parametrize("algo", [1, 2, 3])
 def test_head_conv_tcgen05(c, size, batch, n_classes, algo):
     ops = _ops()
@@ -193,6 +198,8 @@ def test_head_conv_tcgen05(c, size, batch, n_classes, algo):
         pytest.skip("halo-tile kernel needs C % 64 == 0 (the per-tap kernel covers C = 32)")
     if algo == 3 and (c % 64 or n_classes != 2 or batch * size[0] * size[1] * size[2] < 256):
         pytest.skip("kw-GEMM + stencil needs C % 64 == 0, NPAD == 16 and at least 256 voxels")
+    if algo == 3:
+        assert ops.head_kw_supported(torch.empty((batch, c) + size, device="meta"), 16)
     g = torch.Generator().manual_seed(c + size[2] + n_classes)
     bpl = 2
     x = bf16r(torch.randn((batch, c) + size, generator=g))

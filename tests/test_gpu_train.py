@@ -22,6 +22,7 @@ import torch.nn.functional as F
 
 from oracle import ssd3d_oracle as O
 from mslesions3d_b200 import synthetic
+from tests import bench_shapes as S
 
 pytestmark = pytest.mark.gpu
 
@@ -58,10 +59,14 @@ def rel_l2(got, want):
 # ---------------------------------------------------------------------------------------------------
 # train-mode BatchNorm + ReLU, forward and backward
 # ---------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("n,c,size", [(2, 32, (9, 10, 11)), (3, 64, (8, 8, 8)), (1, 128, (5, 6, 7)),
-                                      (2, 512, (2, 2, 2)), (4, 256, (3, 3, 3)), (2, 32, (24, 24, 24)),
-                                      # the single-kernel path takes M <= 4096 rows: the C3 tail, the cap, just above
-                                      (16, 256, (6, 6, 6)), (1, 32, (16, 16, 16)), (1, 32, (16, 16, 17))])
+@pytest.mark.parametrize("n,c,size", S.extend(
+    [(2, 32, (9, 10, 11)), (3, 64, (8, 8, 8)), (1, 128, (5, 6, 7)), (2, 512, (2, 2, 2)), (4, 256, (3, 3, 3)),
+     (2, 32, (24, 24, 24)),
+     # the cluster kernel takes up to 8192 rows (csrc/bn_unit.cu:634-636): the C3 tail, 4096 and 4352 rows
+     (16, 256, (6, 6, 6)), (1, 32, (16, 16, 16)), (1, 32, (16, 16, 17))],
+    # every BatchNorm input of the benchmarked training step (1.77 M rows of the stem down to the 432 of f7), then
+    # both sides of the cluster / tile and register-kept / streamed switches
+    S.bn_shapes(S.TRAIN), S.BN_BOUNDARY, S.BN_BOUNDARY_PASSES))
 def test_bn_train_relu_forward_backward(n, c, size):
     ops = _ops()
     g = torch.Generator().manual_seed(c + n)
@@ -100,11 +105,12 @@ def test_bn_train_relu_forward_backward(n, c, size):
     assert torch.equal(dg2, dgamma) and torch.equal(db2, dbeta)
 
 
-@pytest.mark.parametrize("n,c,size", [(16, 32, (24, 24, 24)), (4, 32, (48, 48, 48)), (16, 64, (12, 12, 12)),
-                                      (16, 1024, (3, 3, 3)), (16, 512, (6, 6, 6)), (16, 128, (6, 6, 6)), (1, 32, (1, 1, 3)),
-                                      (3, 128, (7, 5, 3)), (16, 256, (12, 12, 12)),
-                                      # more than 32768 rows: the grid-barrier kernel, C/8 = 32, 64, 128
-                                      (1, 256, (34, 33, 31)), (1, 512, (33, 32, 32)), (2, 1024, (17, 32, 32))])
+@pytest.mark.parametrize("n,c,size", S.extend(
+    [(16, 32, (24, 24, 24)), (4, 32, (48, 48, 48)), (16, 64, (12, 12, 12)), (16, 1024, (3, 3, 3)), (16, 512, (6, 6, 6)),
+     (16, 128, (6, 6, 6)), (1, 32, (1, 1, 3)), (3, 128, (7, 5, 3)), (16, 256, (12, 12, 12)),
+     # more than 32768 rows: the grid-barrier kernel, C/8 = 32, 64, 128
+     (1, 256, (34, 33, 31)), (1, 512, (33, 32, 32)), (2, 1024, (17, 32, 32))],
+    S.bn_shapes(S.TRAIN), S.BN_BOUNDARY))
 def test_bn_single_launch_matches_three_launch_passes(n, c, size):
     """csrc/bn_unit.cu (one launch, grid barriers) against the three-launch passes of train.cu on the same inputs:
     same statistics to fp32 rounding, same activations / gradients to 1 bf16 ulp; repeated launches (the barrier
@@ -158,9 +164,11 @@ def test_bn_train_nan_sets_flag():
 # ---------------------------------------------------------------------------------------------------
 # pointwise conv: raw forward, data gradient, weight gradient
 # ---------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("cin,cout,n,size", [(32, 64, 2, (12, 12, 12)), (64, 128, 2, (6, 7, 5)), (128, 128, 1, (6, 6, 6)),
-                                             (128, 256, 3, (3, 3, 3)), (256, 512, 2, (2, 2, 2)), (512, 512, 1, (3, 2, 2)),
-                                             (32, 64, 1, (37, 5, 3))])
+@pytest.mark.parametrize("cin,cout,n,size", S.extend(
+    [(32, 64, 2, (12, 12, 12)), (64, 128, 2, (6, 7, 5)), (128, 128, 1, (6, 6, 6)), (128, 256, 3, (3, 3, 3)),
+     (256, 512, 2, (2, 2, 2)), (512, 512, 1, (3, 2, 2)), (32, 64, 1, (37, 5, 3))],
+    # every pointwise unit of the benchmarked training step (f1: M = 221184)
+    [(u.cin, u.cout, u.n, u.size) for u in S.table(S.TRAIN)["pw"]]))
 def test_pointwise_raw_dgrad_wgrad(cin, cout, n, size):
     ops = _ops()
     g = torch.Generator().manual_seed(cin + cout)
@@ -187,12 +195,15 @@ def test_pointwise_raw_dgrad_wgrad(cin, cout, n, size):
 # ---------------------------------------------------------------------------------------------------
 # depthwise conv
 # ---------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("c,n,size,stride", [(32, 2, (12, 12, 12), 2), (64, 1, (9, 7, 11), 2), (128, 2, (6, 6, 6), 1),
-                                             (256, 1, (5, 4, 3), 2), (512, 2, (2, 2, 2), 1), (128, 1, (7, 8, 9), 1),
-                                             (32, 1, (24, 24, 24), 2),
-                                             # large enough for the TMA halo-tile forward / weight-gradient kernels
-                                             (32, 2, (32, 32, 32), 2), (64, 1, (24, 20, 28), 2), (128, 1, (16, 16, 16), 1),
-                                             (32, 1, (19, 21, 17), 2), (96, 2, (9, 12, 10), 1)])
+@pytest.mark.parametrize("c,n,size,stride", S.extend(
+    [(32, 2, (12, 12, 12), 2), (64, 1, (9, 7, 11), 2), (128, 2, (6, 6, 6), 1), (256, 1, (5, 4, 3), 2),
+     (512, 2, (2, 2, 2), 1), (128, 1, (7, 8, 9), 1), (32, 1, (24, 24, 24), 2),
+     # large enough for the TMA halo-tile forward / weight-gradient kernels
+     (32, 2, (32, 32, 32), 2), (64, 1, (24, 20, 28), 2), (128, 1, (16, 16, 16), 1), (32, 1, (19, 21, 17), 2),
+     (96, 2, (9, 12, 10), 1)],
+    # every depthwise unit of the benchmarked training step (f1-f3 halo tiles, f4-f7 the CUDA-core weight gradient),
+    # then both sides of the halo-tile / CUDA-core switch and the ends of the CUDA-core plan
+    [(u.c, u.n, u.size, u.stride) for u in S.table(S.TRAIN)["dw"]], S.DW_BOUNDARY))
 def test_depthwise_raw_dgrad_wgrad(c, n, size, stride):
     ops = _ops()
     g = torch.Generator().manual_seed(c + stride)
@@ -214,13 +225,19 @@ def test_depthwise_raw_dgrad_wgrad(c, n, size, stride):
 # ---------------------------------------------------------------------------------------------------
 # stem conv
 # ---------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("cin,n,size,sd,dtype", [(1, 2, (16, 16, 16), 2, torch.float32), (2, 1, (12, 16, 24), 1, torch.bfloat16),
-                                                 (1, 1, (9, 11, 13), 2, torch.float32), (3, 2, (8, 8, 8), 2, torch.float32),
-                                                 (4, 1, (8, 16, 8), 1, torch.bfloat16), (1, 2, (48, 48, 48), 2, torch.float32),
-                                                 # large enough for the halo-tile kernel (>= 148 tiles of 128 voxels)
-                                                 (2, 2, (40, 44, 48), 1, torch.bfloat16), (3, 2, (33, 50, 56), 2, torch.float32),
-                                                 (4, 3, (32, 48, 40), 2, torch.bfloat16), (1, 3, (31, 45, 72), 1, torch.bfloat16),
-                                                 (2, 1, (64, 64, 64), 2, torch.float32)])
+# the benchmarked training step's stem (fit_step on fp32 batches, fit_epoch on bf16 ones)
+BENCH_STEM = [(u.cin, u.n, u.size, u.stride_d, dt) for u in S.table(S.TRAIN)["stem"]
+              for dt in (torch.float32, torch.bfloat16)]
+
+
+@pytest.mark.parametrize("cin,n,size,sd,dtype", S.extend(
+    [(1, 2, (16, 16, 16), 2, torch.float32), (2, 1, (12, 16, 24), 1, torch.bfloat16), (1, 1, (9, 11, 13), 2, torch.float32),
+     (3, 2, (8, 8, 8), 2, torch.float32), (4, 1, (8, 16, 8), 1, torch.bfloat16), (1, 2, (48, 48, 48), 2, torch.float32),
+     # large enough for the halo-tile kernel (>= 148 tiles of 128 voxels)
+     (2, 2, (40, 44, 48), 1, torch.bfloat16), (3, 2, (33, 50, 56), 2, torch.float32),
+     (4, 3, (32, 48, 40), 2, torch.bfloat16), (1, 3, (31, 45, 72), 1, torch.bfloat16),
+     (2, 1, (64, 64, 64), 2, torch.float32)],
+    BENCH_STEM, S.STEM_WGRAD_BOUNDARY))
 def test_stem_raw_wgrad(cin, n, size, sd, dtype):
     ops = _ops()
     g = torch.Generator().manual_seed(cin * 7 + sd)
@@ -237,11 +254,13 @@ def test_stem_raw_wgrad(cin, n, size, sd, dtype):
     assert rel_l2(dw, w.grad) < 2e-3, rel_l2(dw, w.grad)
 
 
-@pytest.mark.parametrize("cin,n,size,sd,dtype", [(1, 2, (64, 64, 64), 2, torch.float32), (2, 1, (48, 64, 80), 2, torch.bfloat16),
-                                                 (1, 3, (40, 48, 56), 1, torch.float32)])
+@pytest.mark.parametrize("cin,n,size,sd,dtype", S.extend(
+    [(1, 2, (64, 64, 64), 2, torch.float32), (2, 1, (48, 64, 80), 2, torch.bfloat16), (1, 3, (40, 48, 56), 1, torch.float32)],
+    BENCH_STEM, S.STEM_WGRAD_BOUNDARY))
 def test_stem_unit_backward_fused_equals_two_step(cin, n, size, sd, dtype):
     """ssd3d_bn_unit_bwd(dz = NULL) + ssd3d_stem_wgrad_bn (the BatchNorm + ReLU backward applied to the gradient rows
-    inside the weight-gradient kernel, dz never written) against bn_relu_backward + stem_wgrad: bit-identical."""
+    inside the weight-gradient kernel, dz never written) against bn_relu_backward + stem_wgrad: bit-identical.  Below
+    M = 128 * 148 output voxels the fused path declines without launching anything."""
     ops = _ops()
     g = torch.Generator().manual_seed(11 * cin + n)
     x = bf16r(torch.randn((n, cin) + size, generator=g)).to(dtype).cuda()
@@ -255,7 +274,14 @@ def test_stem_unit_backward_fused_equals_two_step(cin, n, size, sd, dtype):
     a, st = ops.bn_train_relu(z, bn, None)
     ga = to_cl(bf16r(torch.randn(tuple(z.shape), generator=g)))
     dg1, db1, dw1 = torch.empty(32, device="cuda"), torch.empty(32, device="cuda"), torch.empty_like(w)
-    assert ops.stem_unit_backward(z, ga, st, dg1, db1, x, sd, dw1), "fused path refused a shape it should take"
+    before = ops.LAUNCHES[0]
+    fused = ops.stem_unit_backward(z, ga, st, dg1, db1, x, sd, dw1)
+    # the fused path runs on the TMA tile kernel, which takes M >= 128 * 148 rows (csrc/train.cu:1507, ops.py:858)
+    m = z.numel() // 32
+    if m < S.STEM_WGRAD_TILE_ROWS:
+        assert not fused and ops.LAUNCHES[0] == before, "fused path took M = %d rows" % m
+        return
+    assert fused, "fused path refused a shape it should take"
     dg2, db2, dw2 = torch.empty(32, device="cuda"), torch.empty(32, device="cuda"), torch.empty_like(w)
     dz = ops.bn_relu_backward(z, ga.clone(), st, dg2, db2)
     ops.stem_wgrad(dz, x, sd, dw2)
@@ -267,14 +293,17 @@ def test_stem_unit_backward_fused_equals_two_step(cin, n, size, sd, dtype):
 # ---------------------------------------------------------------------------------------------------
 # SSD heads: gradient rows, bias / weight / data gradients
 # ---------------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("c,n,size,ncls", [(128, 2, (6, 6, 6), 2), (256, 2, (3, 3, 3), 2), (512, 3, (2, 2, 2), 2),
-                                           (128, 1, (5, 7, 4), 2), (128, 1, (12, 12, 12), 2),
-                                           # n_classes >= 3: bpl*(6+n_classes) > 16 -> several 16-column groups
-                                           (128, 2, (6, 6, 6), 3), (256, 1, (4, 3, 5), 5), (128, 1, (5, 5, 5), 11),
-                                           # batches whose maps hold a 64-voxel box: the tcgen05 weight gradient
-                                           # (the C3 heads at batch 16; C = 64: half-empty channel tile; ragged boxes)
-                                           (256, 16, (3, 3, 3), 2), (256, 16, (6, 6, 6), 2), (512, 16, (3, 3, 3), 2),
-                                           (64, 2, (8, 8, 8), 2), (192, 5, (5, 3, 7), 3)])
+@pytest.mark.parametrize("c,n,size,ncls", S.extend(
+    [(128, 2, (6, 6, 6), 2), (256, 2, (3, 3, 3), 2), (512, 3, (2, 2, 2), 2), (128, 1, (5, 7, 4), 2),
+     (128, 1, (12, 12, 12), 2),
+     # n_classes >= 3: bpl*(6+n_classes) > 16 -> several 16-column groups
+     (128, 2, (6, 6, 6), 3), (256, 1, (4, 3, 5), 5), (128, 1, (5, 5, 5), 11),
+     # batches whose maps hold a 64-voxel box: the tcgen05 weight gradient
+     # (the C3 heads at batch 16; C = 64: half-empty channel tile; ragged boxes)
+     (256, 16, (3, 3, 3), 2), (256, 16, (6, 6, 6), 2), (512, 16, (3, 3, 3), 2), (64, 2, (8, 8, 8), 2),
+     (192, 5, (5, 3, 7), 3)],
+    # every head of the benchmarked training step (two boxes per location, as the body below assumes)
+    [(u.c, u.n, u.size, 2) for u in S.table(S.TRAIN)["head"]]))
 def test_head_backward(c, n, size, ncls):
     ops = _ops()
     bpl = 2
