@@ -581,6 +581,44 @@ int ssd3d_gt_boxes_from_instances(const void* seg, int seg_dtype, int N, int D, 
  *   most m source voxels more than under the affine alone.
  *   record (N, 33) int32: words 0-31 as ssd3d_augment_affine_batch, 32 field drawn.
  *
+ * ssd3d_augment_intensity_batch is the MR intensity augmentation: random gamma, bias field and Gaussian noise,
+ * applied in place to the bf16 batch image (N, C, d, h, w) that one of the three launches above has just written
+ * (after their geometry, step 4 and its bf16 round).  The masks are not touched.  The draws use the same Philox
+ * stream: key = seed, counter = (rank * N + b, c low, c high, call) with c = state[1] - 1, the draw counter the
+ * preceding augment launch consumed; the state is only read.  So every value is a pure function of (seed, c, global
+ * slot, voxel index), whatever N.  Per slot b:
+ *   call 2^16 {gamma u, bias u, noise u, log-gamma u}, call 2^16 + 1 {sigma u, -, -, -},
+ *   calls 2^16 + 2 + q (q = 0..4) {coefficient 4q .. 4q + 3 u};
+ *   gamma drawn when u01 < gamma_prob: gamma = expf(fp32_rn(gamma_log_range * fp32_rn(fp32_rn(2 u01) - 1))) (device
+ *   expf, once per slot; TorchIO's log-gamma), else 1; bias drawn when u01 < bias_prob: c_m =
+ *   fp32_rn(bias_coefficient * fp32_rn(fp32_rn(2 u01) - 1)), else 0; noise drawn when u01 < noise_prob:
+ *   sigma = fp32_rn(noise_std * u01), else 0.
+ * The 20 monomials m = (i, j, k), i + j + k <= 3, are ordered i outermost, then j, then k (m = 0: (0, 0, 0), 1: (0, 0,
+ * 1), ..., 19: (3, 0, 0)).  lo and hi are the minimum and maximum of the slot's bf16 values over all its channels
+ * (MONAI AdjustContrast), found only for a slot that draws gamma.  Per voxel x (fp32 value of the bf16), in order:
+ *   1. gamma, if drawn, gamma != 1 and hi != lo: r = fp32_rn(hi - lo), t = min(fp32_rn(fp32_rn(x - lo) *
+ *      fp32_rn(1 / r)), 1), y = fp32_rn(lo + fp32_rn(r * exp2f(fp32_rn(gamma * __log2f(t)))));
+ *   2. bias field, if drawn: u_a = fp32_rn(fp32_rn(p_a * fp32_rn(2 / (n_a - 1))) - 1) at output index p_a of the
+ *      axis of extent n_a (u_a = 0 when n_a = 1); per (d, h) row a_k = the sum over m with k_m = k, in monomial
+ *      order from +0, of fp32_rn(c_m * fp32_rn(u_d^i u_h^j)) (powers by repeated rounded products); P =
+ *      ((a_3 u_w + a_2) u_w + a_1) u_w + a_0, every operation rounded; y = fp32_rn(y * __expf(P)) -- one field per
+ *      slot (TorchIO's order-3 polynomial in exp), shared by its channels;
+ *   3. noise, if drawn and sigma != 0: y = fp32_rn(y + fp32_rn(sigma * n)), n ~ N(0, 1) independent per voxel and
+ *      channel: voxel i = ((ch * d + z) * h + y) * w + x of the slot, quad q = i / 4 takes call 2^24 + q, and
+ *      Box-Muller on words (0, 1) gives voxels 4q, 4q + 1 and on words (2, 3) voxels 4q + 2, 4q + 3: u1 =
+ *      ((word >> 8) + 1) 2^-24 in (0, 1], u2 = u01(word), rad = sqrtf(-2 logf(u1)), {rad cospi(2 u2), rad sinpi(2 u2)};
+ *   4. one bf16 round to nearest, in place.
+ * A step not drawn, or with zero strength (gamma = 1, hi = lo, sigma = 0; all c_m = 0 give a field of exactly 1),
+ * leaves the value alone, so a slot with none of the three keeps its input bit for bit.  exp2f, __log2f, __expf,
+ * logf and sincospif err by a few fp32 ulps, far below the bf16 round.
+ *   bias_prob, gamma_prob, noise_prob in [0, 1]; bias_coefficient in [0, 1]; gamma_log_range in [0, 1); noise_std
+ *   finite and >= 0; w % 16 == 0 (16-byte vectors); anything else (NaN included) is SSD3D_ERR_ARG before any CUDA
+ *   call.  N <= 65535 and C d h w / 4 <= 2^32 - 2^24, else SSD3D_ERR_UNSUPPORTED.
+ *   record (N, 27) int32 (fp32 bits from word 3): gamma drawn, bias drawn, noise drawn, gamma, lo, hi (0 and 0
+ *         without gamma), sigma, c_0 .. c_19.
+ *   workspace: ssd3d_augment_intensity_workspace_bytes(N, C, d, h, w) bytes when gamma_prob > 0 (else may be NULL):
+ *         the per-(slot, chunk) min / max partials.  Two launches, no atomics, no memsets, no host copies.
+ *
  * ssd3d_gt_pack turns the per-image output of ssd3d_gt_boxes_from_segmentation (boxes (N, max_boxes, 6), labels
  * (N, max_boxes), counts, n_components) into the packed ground truth of the training step: gt_boxes
  * (N * per_volume, 6), gt_labels (N * per_volume) int64 and offsets (N + 1) int32 (the ssd3d_match_priors input),
@@ -607,6 +645,11 @@ int ssd3d_augment_elastic_batch(const void* src, int src_is_bf16, const uint8_t*
                                 float shift, float affine_prob, const float* rotate_range, const float* zoom_range,
                                 float elastic_prob, const int32_t* elastic_points, const float* elastic_magnitude,
                                 void* out, uint8_t* out_mask, int32_t* record, void* stream);
+int64_t ssd3d_augment_intensity_workspace_bytes(int N, int C, int d, int h, int w);
+int ssd3d_augment_intensity_batch(void* image, int N, int C, int d, int h, int w, const int64_t* state,
+                                  float bias_prob, float bias_coefficient, float gamma_prob, float gamma_log_range,
+                                  float noise_prob, float noise_std, int32_t* record, void* workspace,
+                                  int64_t workspace_bytes, void* stream);
 int ssd3d_gt_pack(const float* boxes, const int64_t* labels, const int32_t* counts, const int32_t* n_components,
                   int N, int max_boxes, int per_volume, float* gt_boxes, int64_t* gt_labels, int32_t* offsets,
                   int32_t* status, void* stream);

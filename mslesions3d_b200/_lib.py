@@ -128,6 +128,9 @@ SIGNATURES = {
     "ssd3d_augment_elastic_batch": (c_int, [P, c_int, P, c_int, c_int, c_int, c_int, c_int, P, P, P, P, c_int, c_int,
                                             c_int, c_int, c_float, c_float, c_float, c_int, c_int, c_float, c_float,
                                             c_float, P, P, c_float, P, P, P, P, P, P]),
+    "ssd3d_augment_intensity_workspace_bytes": (c_int64, [c_int, c_int, c_int, c_int, c_int]),
+    "ssd3d_augment_intensity_batch": (c_int, [P, c_int, c_int, c_int, c_int, c_int, P, c_float, c_float, c_float,
+                                              c_float, c_float, c_float, P, P, c_int64, P]),
     "ssd3d_gt_pack": (c_int, [P, P, P, P, c_int, c_int, c_int, P, P, P, P, P]),
     # ---- sliding-window inference ----
     "ssd3d_window_gather": (c_int, [P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int,

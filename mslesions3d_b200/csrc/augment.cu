@@ -527,6 +527,228 @@ __global__ void __launch_bounds__(32 * AFF_WARPS, ELASTIC ? 6 : 0) augment_affin
   if (tid == 0) aug_advance_state(state);
 }
 
+// MR intensity augmentation (ssd3d_augment_intensity_batch): gamma, bias field and Gaussian noise, a point-wise pass
+// in place over the bf16 batch the augment kernels above have written.  Two launches: intensity_slot_kernel draws
+// every slot's values into the record and, when gamma_prob > 0, the per-(slot, chunk) min / max partials of the
+// slots that draw gamma; intensity_voxel_kernel reduces those partials per block in a fixed order and streams 16-byte
+// bf16 vectors.  Every draw is a pure function of (seed, draw counter, global slot, voxel index).
+constexpr int INT_WORDS = 27;                   // record words per slot (layout in include/ssd3d_b200.h)
+constexpr int INT_NCOEF = 20;                   // monomials u_d^i u_h^j u_w^k, i + j + k <= 3
+constexpr uint32_t INT_CALL_SLOT = 1u << 16;    // per-slot draws: Philox calls 2^16 + j
+constexpr uint32_t INT_CALL_NOISE = 1u << 24;   // noise: call 2^24 + q for the voxel quad q of the slot
+constexpr int INT_CHUNK = 16384;                // bf16 values per min / max partial: 256 threads x 8 16-byte vectors
+constexpr int INT_VPT = 4;                      // 8-voxel vectors per thread of the per-voxel pass
+
+struct IntArgs {
+  int N, C, d, h, w, chunks;                    // chunks: partials per slot, 0 when gamma_prob == 0
+  float bias_prob, bias_coef, gamma_prob, gamma_log_range, noise_prob, noise_std;
+  float su[2], ou[2];                           // u = fp32_rn(fp32_rn(p * su) - ou) on d and h (su = ou = 0: n = 1)
+  float sw;                                     // the same on w (w >= 16)
+};
+
+// Philox4x32-10 of global slot g at the draw counter the preceding augment launch consumed (state[1] - 1)
+__device__ __forceinline__ Philox4 int_philox(const long long* __restrict__ state, uint32_t g, uint32_t call) {
+  const unsigned long long seed = (unsigned long long)state[0], ctr = (unsigned long long)state[1] - 1ull;
+  return philox4x32_10(g, (uint32_t)ctr, (uint32_t)(ctr >> 32), call, (uint32_t)seed, (uint32_t)(seed >> 32));
+}
+
+__device__ __forceinline__ uint32_t int_slot(const IntArgs& a, const long long* __restrict__ state, int b) {
+  return (uint32_t)(state[3] * a.N + b);
+}
+
+// the draws of slot b into rec[INT_WORDS]; lo and hi (words 4, 5) are left 0 for the per-voxel pass
+__device__ void intensity_draw(const IntArgs& a, const long long* __restrict__ state, int b, int* rec) {
+  const uint32_t g = int_slot(a, state, b);
+  const Philox4 r0 = int_philox(state, g, INT_CALL_SLOT), r1 = int_philox(state, g, INT_CALL_SLOT + 1u);
+  const bool gon = u01(r0.v[0]) < a.gamma_prob, bon = u01(r0.v[1]) < a.bias_prob, non = u01(r0.v[2]) < a.noise_prob;
+  float gamma = 1.f, sigma = 0.f;
+  if (gon) gamma = expf(__fmul_rn(a.gamma_log_range, __fsub_rn(__fmul_rn(2.f, u01(r0.v[3])), 1.f)));
+  if (non) sigma = __fmul_rn(a.noise_std, u01(r1.v[0]));
+  rec[0] = gon ? 1 : 0;
+  rec[1] = bon ? 1 : 0;
+  rec[2] = non ? 1 : 0;
+  rec[3] = __float_as_int(gamma);
+  rec[4] = 0;
+  rec[5] = 0;
+  rec[6] = __float_as_int(sigma);
+  for (int q = 0; q < INT_NCOEF / 4; ++q) {
+    const Philox4 rc = int_philox(state, g, INT_CALL_SLOT + 2u + (uint32_t)q);
+#pragma unroll
+    for (int e = 0; e < 4; ++e)
+      rec[7 + q * 4 + e] =
+          __float_as_int(bon ? __fmul_rn(a.bias_coef, __fsub_rn(__fmul_rn(2.f, u01(rc.v[e])), 1.f)) : 0.f);
+  }
+}
+
+// grid: (max(chunks, 1), N); 256 threads.  Block (0, b) writes slot b's record; with chunks > 0 block (k, b) of a
+// slot that draws gamma writes the min and max of the slot's bf16 values [k, k + 1) * INT_CHUNK (all channels)
+__global__ void __launch_bounds__(256) intensity_slot_kernel(IntArgs a, const __nv_bfloat16* __restrict__ img,
+                                                             const long long* __restrict__ state,
+                                                             int* __restrict__ record, float2* __restrict__ partial) {
+  __shared__ float s_lo[8], s_hi[8];
+  const int b = blockIdx.y, tid = threadIdx.x;
+  if (blockIdx.x == 0 && tid == 0) {
+    int rec[INT_WORDS];
+    intensity_draw(a, state, b, rec);
+    for (int i = 0; i < INT_WORDS; ++i) record[b * INT_WORDS + i] = rec[i];
+  }
+  if (a.chunks == 0 || !(u01(int_philox(state, int_slot(a, state, b), INT_CALL_SLOT).v[0]) < a.gamma_prob)) return;
+  const long long n = (long long)a.C * a.d * a.h * a.w;
+  const uint4* src = reinterpret_cast<const uint4*>(img + (long long)b * n);
+  const long long v1 = min((long long)(blockIdx.x + 1) * (INT_CHUNK / 8), n / 8);
+  const __nv_bfloat162 inf2 = __floats2bfloat162_rn(INFINITY, INFINITY);
+  __nv_bfloat162 lo2 = inf2, hi2 = __hneg2(inf2);
+  for (long long v = (long long)blockIdx.x * (INT_CHUNK / 8) + tid; v < v1; v += 256) {
+    const uint4 q = src[v];
+    const uint32_t u[4] = {q.x, q.y, q.z, q.w};
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const __nv_bfloat162 p = *reinterpret_cast<const __nv_bfloat162*>(&u[j]);
+      lo2 = __hmin2(lo2, p);
+      hi2 = __hmax2(hi2, p);
+    }
+  }
+  float lo = fminf(__low2float(lo2), __high2float(lo2)), hi = fmaxf(__low2float(hi2), __high2float(hi2));
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    lo = fminf(lo, __shfl_xor_sync(0xffffffffu, lo, o));
+    hi = fmaxf(hi, __shfl_xor_sync(0xffffffffu, hi, o));
+  }
+  if ((tid & 31) == 0) { s_lo[tid >> 5] = lo; s_hi[tid >> 5] = hi; }
+  __syncthreads();
+  if (tid == 0) {
+    for (int i = 1; i < 8; ++i) { lo = fminf(lo, s_lo[i]); hi = fmaxf(hi, s_hi[i]); }
+    partial[(long long)b * a.chunks + blockIdx.x] = make_float2(lo, hi);
+  }
+}
+
+// the standard normals of the 8 voxels [i, i + 8) of a slot (i = c * d * h * w + 8 * vector, a multiple of 8): voxel
+// quad q takes Philox call 2^24 + q, and Box-Muller on words (0, 1) and (2, 3) gives its voxels {r cos, r sin} each
+__device__ __forceinline__ void int_normals(const long long* __restrict__ state, uint32_t g, uint32_t quad, float* n) {
+#pragma unroll
+  for (int h = 0; h < 2; ++h) {
+    const Philox4 r = int_philox(state, g, INT_CALL_NOISE + quad + (uint32_t)h);
+#pragma unroll
+    for (int p = 0; p < 2; ++p) {
+      const float u1 = (float)((r.v[2 * p] >> 8) + 1u) * (1.f / 16777216.f);     // (0, 1]: the log is finite
+      const float u2 = u01(r.v[2 * p + 1]);                                       // [0, 1)
+      const float rad = sqrtf(__fmul_rn(-2.f, logf(u1)));
+      float s, c;
+      sincospif(__fmul_rn(2.f, u2), &s, &c);
+      n[h * 4 + p * 2] = __fmul_rn(rad, c);
+      n[h * 4 + p * 2 + 1] = __fmul_rn(rad, s);
+    }
+  }
+}
+
+// grid: (ceil(d * h * w / 8 / (256 * INT_VPT)), N); 256 threads, each INT_VPT vectors of 8 W voxels, every channel
+__global__ void __launch_bounds__(256) intensity_voxel_kernel(IntArgs a, __nv_bfloat16* __restrict__ img,
+                                                              const long long* __restrict__ state,
+                                                              int* __restrict__ record,
+                                                              const float2* __restrict__ partial) {
+  __shared__ int s_rec[INT_WORDS];
+  __shared__ float s_lohi[2];
+  const int b = blockIdx.y, tid = threadIdx.x;
+  if (tid < INT_WORDS) s_rec[tid] = record[b * INT_WORDS + tid];
+  __syncthreads();
+  const bool gon = s_rec[0] != 0, bon = s_rec[1] != 0, non = s_rec[2] != 0;
+  if (!gon && !bon && !non) return;                                       // block-uniform: the slot draws nothing
+  if (gon) {                                                              // lo, hi: min / max of the partials
+    if (tid < 32) {
+      float lo = INFINITY, hi = -INFINITY;
+      for (int i = tid; i < a.chunks; i += 32) {
+        const float2 p = partial[(long long)b * a.chunks + i];
+        lo = fminf(lo, p.x);
+        hi = fmaxf(hi, p.y);
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+        lo = fminf(lo, __shfl_xor_sync(0xffffffffu, lo, o));
+        hi = fmaxf(hi, __shfl_xor_sync(0xffffffffu, hi, o));
+      }
+      if (tid == 0) {
+        s_lohi[0] = lo;
+        s_lohi[1] = hi;
+        if (blockIdx.x == 0) {
+          record[b * INT_WORDS + 4] = __float_as_int(lo);
+          record[b * INT_WORDS + 5] = __float_as_int(hi);
+        }
+      }
+    }
+    __syncthreads();
+  }
+  const float gamma = __int_as_float(s_rec[3]), sigma = __int_as_float(s_rec[6]);
+  const float lo = gon ? s_lohi[0] : 0.f, hi = gon ? s_lohi[1] : 0.f;
+  const bool g_act = gon && gamma != 1.f && hi != lo, n_act = non && sigma != 0.f;
+  if (!g_act && !bon && !n_act) return;                                   // zero strengths: the identity
+  const float r = __fsub_rn(hi, lo), rinv = g_act ? __frcp_rn(r) : 0.f;
+  float cf[INT_NCOEF];
+#pragma unroll
+  for (int i = 0; i < INT_NCOEF; ++i) cf[i] = __int_as_float(s_rec[7 + i]);
+  const uint32_t g = int_slot(a, state, b);
+  const int wv = a.w / 8;
+  const long long vox = (long long)a.d * a.h * a.w, nvec = vox / 8;
+  __nv_bfloat16* base = img + (long long)b * a.C * vox;
+  // 32-bit index arithmetic: d h w / 8 < 2^31 (the entry point bounds C d h w / 4 by 2^32)
+  const unsigned nvec32 = (unsigned)nvec, hh = (unsigned)a.h;
+#pragma unroll 1
+  for (int k = 0; k < INT_VPT; ++k) {
+    const unsigned v = (blockIdx.x * INT_VPT + k) * 256u + tid;
+    if (v >= nvec32) break;
+    const unsigned row = v / (unsigned)wv, zz = row / hh;
+    const int x0 = (int)(v - row * wv) * 8, z = (int)zz, y = (int)(row - zz * hh);
+    float field[8];
+    if (bon) {
+      // the row's cubic in u_w: a_k = sum over (i, j) in coefficient order of c_ijk * (u_d^i u_h^j)
+      const float ud = __fsub_rn(__fmul_rn((float)z, a.su[0]), a.ou[0]);
+      const float uh = __fsub_rn(__fmul_rn((float)y, a.su[1]), a.ou[1]);
+      const float pd[4] = {1.f, ud, __fmul_rn(ud, ud), __fmul_rn(__fmul_rn(ud, ud), ud)};
+      const float ph[4] = {1.f, uh, __fmul_rn(uh, uh), __fmul_rn(__fmul_rn(uh, uh), uh)};
+      float ak[4] = {0.f, 0.f, 0.f, 0.f};
+      int idx = 0;
+#pragma unroll
+      for (int i = 0; i < 4; ++i)
+#pragma unroll
+        for (int j = 0; j < 4 - i; ++j)
+#pragma unroll
+          for (int kk = 0; kk < 4 - i - j; ++kk)
+            ak[kk] = __fadd_rn(ak[kk], __fmul_rn(cf[idx++], __fmul_rn(pd[i], ph[j])));
+#pragma unroll
+      for (int e = 0; e < 8; ++e) {
+        const float uw = __fsub_rn(__fmul_rn((float)(x0 + e), a.sw), 1.f);
+        const float p = __fadd_rn(__fmul_rn(__fadd_rn(__fmul_rn(__fadd_rn(__fmul_rn(ak[3], uw), ak[2]), uw), ak[1]),
+                                            uw), ak[0]);
+        field[e] = __expf(p);
+      }
+    }
+#pragma unroll 1
+    for (int c = 0; c < a.C; ++c) {
+      uint4* ptr = reinterpret_cast<uint4*>(base + (long long)c * vox) + v;
+      const uint4 q = *ptr;
+      uint32_t u[4] = {q.x, q.y, q.z, q.w};
+      float nz[8];
+      if (n_act) int_normals(state, g, (uint32_t)(((long long)c * vox + (long long)v * 8) >> 2), nz);
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const float2 f = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&u[j]));
+        float x[2] = {f.x, f.y};
+#pragma unroll
+        for (int e = 0; e < 2; ++e) {
+          if (g_act) {
+            const float t = fminf(__fmul_rn(__fsub_rn(x[e], lo), rinv), 1.f);
+            x[e] = __fadd_rn(lo, __fmul_rn(r, exp2f(__fmul_rn(gamma, __log2f(t)))));
+          }
+          if (bon) x[e] = __fmul_rn(x[e], field[2 * j + e]);
+          if (n_act) x[e] = __fadd_rn(x[e], __fmul_rn(sigma, nz[2 * j + e]));
+        }
+        const __nv_bfloat162 o = __floats2bfloat162_rn(x[0], x[1]);
+        u[j] = *reinterpret_cast<const uint32_t*>(&o);
+      }
+      *ptr = make_uint4(u[0], u[1], u[2], u[3]);
+    }
+  }
+}
+
 // one block: per-volume overflow test, offsets (exclusive scan of the counts) and the row copy
 __global__ void __launch_bounds__(256) gt_pack_kernel(const float* __restrict__ boxes, const long long* __restrict__ labels,
                                                       const int* __restrict__ counts, const int* __restrict__ n_comp,
@@ -690,6 +912,51 @@ extern "C" int ssd3d_augment_batch(const void* src, int src_is_bf16, const uint8
   else
     augment_kernel<float><<<grid, 256, 0, st>>>(a, static_cast<const float*>(src), masks, order, reinterpret_cast<long long*>(state), boxes,
                                                 box_offsets, static_cast<__nv_bfloat16*>(out), out_mask, record);
+  SSD3D_CHECK_LAUNCH();
+  return SSD3D_OK;
+}
+
+static long long int_chunks(int C, int d, int h, int w) {
+  return ((long long)C * d * h * w + INT_CHUNK - 1) / INT_CHUNK;
+}
+
+extern "C" int64_t ssd3d_augment_intensity_workspace_bytes(int N, int C, int d, int h, int w) {
+  if (N <= 0 || C <= 0 || d <= 0 || h <= 0 || w <= 0) return 0;
+  return (int64_t)N * int_chunks(C, d, h, w) * (int64_t)sizeof(float2);
+}
+
+extern "C" int ssd3d_augment_intensity_batch(void* image, int N, int C, int d, int h, int w, const int64_t* state,
+                                             float bias_prob, float bias_coefficient, float gamma_prob,
+                                             float gamma_log_range, float noise_prob, float noise_std,
+                                             int32_t* record, void* workspace, int64_t workspace_bytes,
+                                             void* stream) {
+  if (!image || !state || !record) return SSD3D_ERR_ARG;
+  if (N <= 0 || C <= 0 || d <= 0 || h <= 0 || w <= 0 || w % 16 != 0) return SSD3D_ERR_ARG;
+  // the negated comparisons also refuse NaN
+  if (!(bias_prob >= 0.f && bias_prob <= 1.f) || !(gamma_prob >= 0.f && gamma_prob <= 1.f) ||
+      !(noise_prob >= 0.f && noise_prob <= 1.f) || !(bias_coefficient >= 0.f && bias_coefficient <= 1.f) ||
+      !(gamma_log_range >= 0.f && gamma_log_range < 1.f) || !(noise_std >= 0.f && noise_std <= 3.40282347e38f))
+    return SSD3D_ERR_ARG;
+  const long long chunks = int_chunks(C, d, h, w);
+  if (gamma_prob > 0.f && (!workspace || workspace_bytes < (int64_t)N * chunks * (int64_t)sizeof(float2)))
+    return SSD3D_ERR_ARG;
+  // noise call numbers 2^24 + quad stay below 2^32; N is the grid's y extent
+  const long long vox = (long long)d * h * w;
+  if (N > 65535 || (long long)C * vox / 4 > (1ll << 32) - (1ll << 24)) return SSD3D_ERR_UNSUPPORTED;
+  IntArgs a{N, C, d, h, w, gamma_prob > 0.f ? (int)chunks : 0, bias_prob, bias_coefficient, gamma_prob,
+            gamma_log_range, noise_prob, noise_std, {0.f, 0.f}, {0.f, 0.f}, 2.f / (float)(w - 1)};
+  const int ext[2] = {d, h};
+  for (int i = 0; i < 2; ++i)
+    if (ext[i] > 1) { a.su[i] = 2.f / (float)(ext[i] - 1); a.ou[i] = 1.f; }    // one correctly rounded division
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  intensity_slot_kernel<<<dim3((unsigned)(a.chunks > 0 ? a.chunks : 1), (unsigned)N), 256, 0, st>>>(
+      a, static_cast<const __nv_bfloat16*>(image), reinterpret_cast<const long long*>(state), record,
+      static_cast<float2*>(workspace));
+  SSD3D_CHECK_LAUNCH();
+  const long long blocks = (vox / 8 + 256 * INT_VPT - 1) / (256 * INT_VPT);
+  intensity_voxel_kernel<<<dim3((unsigned)blocks, (unsigned)N), 256, 0, st>>>(
+      a, static_cast<__nv_bfloat16*>(image), reinterpret_cast<const long long*>(state), record,
+      static_cast<const float2*>(workspace));
   SSD3D_CHECK_LAUNCH();
   return SSD3D_OK;
 }

@@ -37,7 +37,16 @@ class Augment:
       semantics: ``ssd3d_augment_elastic_batch``);
     * ``np.rot90(x, k, axes=rot90_axes)``, k uniform in {1, 2, 3}, with probability ``rot90_prob``;
     * ``np.flip`` of each spatial axis with probability ``flip_prob``;
-    * ``x * (1 + f) + o`` with ``f ~ U(-scale, scale)``, ``o ~ U(-shift, shift)`` per volume (shared by its channels).
+    * ``x * (1 + f) + o`` with ``f ~ U(-scale, scale)``, ``o ~ U(-shift, shift)`` per volume (shared by its channels);
+    * the MR intensity set, a separate pass over the batch (exact semantics: ``ssd3d_augment_intensity_batch``):
+      with probability ``gamma_prob``, a contrast change ``lo + (hi - lo) * ((x - lo) / (hi - lo)) ** gamma`` with
+      ``log(gamma) ~ U(-gamma_log_range, gamma_log_range)`` and ``lo``, ``hi`` the volume's minimum and maximum (MONAI
+      ``RandAdjustContrast``, TorchIO ``RandomGamma``); with probability ``bias_prob``, a smooth multiplicative bias
+      field ``exp(sum c_ijk u_d^i u_h^j u_w^k)`` over the 20 monomials of degree <= 3 of the coordinates scaled to
+      [-1, 1], ``c_ijk ~ U(-bias_coefficient, bias_coefficient)`` (TorchIO ``RandomBiasField``, MONAI
+      ``RandBiasField``); with probability ``noise_prob``, additive Gaussian noise of ``sigma ~ U(0, noise_std)``
+      per voxel and channel (MONAI ``RandGaussianNoise``, TorchIO ``RandomNoise``).  One field and one gamma per
+      volume, shared by its channels; the masks, and so the ground truth, are unchanged.
 
     The corners of a rotated crop hold source data wherever the source extends past the crop (MONAI's crop-then-
     rotate pads them); zeros appear only outside the source.  A positive crop is chosen to hold the lesion box before
@@ -50,7 +59,8 @@ class Augment:
 
     ``Augment()`` on a data set of ``input_size`` volumes is the identity (up to the bf16 rounding of the input);
     without the affine and the field (``affine_prob == 0``, ``elastic_prob == 0``) the batches are those of
-    ``ssd3d_augment_batch``, and without the field those of ``ssd3d_augment_affine_batch``."""
+    ``ssd3d_augment_batch``, and without the field those of ``ssd3d_augment_affine_batch``; with ``bias_prob``,
+    ``gamma_prob`` and ``noise_prob`` all 0 the intensity pass does not run."""
     pos_ratio: float = 0.0
     flip_prob: float = 0.0
     rot90_prob: float = 0.0
@@ -64,10 +74,32 @@ class Augment:
     elastic_prob: float = 0.0
     elastic_points: Tuple[int, int, int] = (7, 7, 7)
     elastic_magnitude: Tuple[float, float, float] = (0.0, 0.0, 0.0)
+    bias_prob: float = 0.0
+    bias_coefficient: float = 0.0
+    gamma_prob: float = 0.0
+    gamma_log_range: float = 0.0
+    noise_prob: float = 0.0
+    noise_std: float = 0.0
+
+    @property
+    def intensity(self) -> bool:
+        """Whether the MR intensity pass runs (``bias_prob``, ``gamma_prob`` or ``noise_prob`` > 0)."""
+        return self.bias_prob > 0 or self.gamma_prob > 0 or self.noise_prob > 0
 
     def validate(self, input_size: Sequence[int], source_size: Sequence[int]) -> None:
         """Raise ValueError unless this augmentation can turn ``source_size`` volumes into ``input_size`` ones."""
         out, src = tuple(int(v) for v in input_size), tuple(int(v) for v in source_size)
+        # the intensity fields first: a non-number must not reach the comparisons below (and the Augment is hashed)
+        for name, hi, closed in (("bias_prob", 1.0, True), ("gamma_prob", 1.0, True), ("noise_prob", 1.0, True),
+                                 ("bias_coefficient", 1.0, True), ("gamma_log_range", 1.0, False),
+                                 ("noise_std", 3.4028234663852886e38, True)):
+            v = getattr(self, name)
+            if not isinstance(v, (int, float)) or isinstance(v, bool) or not math.isfinite(v):
+                raise ValueError("%s must be a finite number, got %r" % (name, v))
+            # checked as the fp32 the kernel receives
+            v32 = float(np.float32(v)) if abs(v) <= hi else math.inf
+            if not (0.0 <= v32 and (v32 <= hi if closed else v32 < hi)):
+                raise ValueError("%s=%r must lie in [0, %g%s" % (name, v, hi, "]" if closed else ")"))
         for name in ("pos_ratio", "flip_prob", "rot90_prob", "affine_prob", "elastic_prob"):
             p = getattr(self, name)
             if not 0.0 <= p <= 1.0:

@@ -1212,6 +1212,42 @@ def augment_elastic_batch(src: torch.Tensor, masks: torch.Tensor, order: torch.T
     return out
 
 
+def augment_intensity_batch(images: torch.Tensor, state: torch.Tensor, batch_size: int, bias_prob: float = 0.0,
+                            bias_coefficient: float = 0.0, gamma_prob: float = 0.0, gamma_log_range: float = 0.0,
+                            noise_prob: float = 0.0, noise_std: float = 0.0, out_record=None, workspace=None):
+    """MR intensity augmentation in place on a batch an augment launch has just written (see
+    ``ssd3d_augment_intensity_batch`` in the header): per slot, with their probabilities, gamma = exp(U(-r, r)) on the
+    slot's [min, max], an order-3 polynomial bias field exp(sum c u_d^i u_h^j u_w^k) with c ~ U(-bias_coefficient,
+    bias_coefficient), and Gaussian noise of sigma ~ U(0, noise_std); ``state`` is read, not advanced.  images
+    (N, C, d, h, w) bf16 -> record (N, 27) int32: gamma / bias / noise drawn, gamma, lo, hi, sigma, the 20
+    coefficients (fp32 bits).  ``workspace``: ``augment_intensity_workspace_bytes`` bytes (allocated if None)."""
+    _need_cuda(images, state)
+    if images.dim() != 5 or images.dtype != BF16 or not images.is_contiguous():
+        raise RuntimeError("expected contiguous bf16 images (N, C, d, h, w)")
+    if state.dtype != torch.int64 or not state.is_contiguous():
+        raise RuntimeError("state must be contiguous int64")
+    n, c, d, h, w = images.shape
+    if n != int(batch_size):
+        raise RuntimeError("images hold %d volumes, batch_size is %d" % (n, int(batch_size)))
+    lib = _lib.load()
+    if out_record is None:
+        out_record = torch.empty((n, 27), dtype=torch.int32, device=images.device)
+    if workspace is None:
+        workspace = torch.empty((max(1, augment_intensity_workspace_bytes(n, c, d, h, w)),), dtype=torch.uint8,
+                                device=images.device)
+    rc = lib.ssd3d_augment_intensity_batch(images.data_ptr(), n, c, d, h, w, state.data_ptr(), float(bias_prob),
+                                           float(bias_coefficient), float(gamma_prob), float(gamma_log_range),
+                                           float(noise_prob), float(noise_std), out_record.data_ptr(),
+                                           workspace.data_ptr(), workspace.numel(), _stream())
+    _lib.check(rc, "ssd3d_augment_intensity_batch")
+    LAUNCHES[0] += 2
+    return out_record
+
+
+def augment_intensity_workspace_bytes(n: int, c: int, d: int, h: int, w: int) -> int:
+    return int(_lib.load().ssd3d_augment_intensity_workspace_bytes(int(n), int(c), int(d), int(h), int(w)))
+
+
 def _augment_args(src, masks, order, state, boxes, box_offsets, batch_size, out_size, pos_ratio, flip_prob,
                   rot90_prob, rot90_axes, scale, shift, record_words, out):
     """The checked leading arguments shared by ssd3d_augment_batch, ssd3d_augment_affine_batch and

@@ -696,9 +696,10 @@ def fit_step(model, batch, world_size: int = 1, allreduce=None):
 class _EpochPlan(_TrainPlan):
     """The fused step fed from a ``DeviceDataset``: the captured graph also samples and augments the batch straight
     into the static image buffer (``ssd3d_augment_batch``; ``ssd3d_augment_affine_batch`` when the augmentation
-    draws a rotation and zoom; ``ssd3d_augment_elastic_batch`` when it draws an elastic deformation), extracts the ground truth of the augmented masks
-    (``ssd3d_gt_boxes_from_segmentation``) and packs it into the static GT buffers (``ssd3d_gt_pack``).  The draw
-    state advances inside the graph, so every replay is the next step of the epoch with no host copy or sync."""
+    draws a rotation and zoom; ``ssd3d_augment_elastic_batch`` when it draws an elastic deformation), then, when the
+    augmentation draws MR intensity changes, applies them in place (``ssd3d_augment_intensity_batch``), extracts the
+    ground truth of the augmented masks (``ssd3d_gt_boxes_from_segmentation``) and packs it into the static GT
+    buffers (``ssd3d_gt_pack``).  The draw state advances inside the graph, so every replay is the next step of the epoch with no host copy or sync."""
 
     def __init__(self, model, dataset, augment, n: int, per_volume: int, world_size: int, allreduce):
         dev = model.device
@@ -719,6 +720,10 @@ class _EpochPlan(_TrainPlan):
         lib = _lib.load()
         self.gt_ws = torch.empty((lib.ssd3d_gt_boxes_workspace_bytes(n, d, h, w, per_volume),), dtype=torch.uint8,
                                  device=dev)
+        if augment.intensity:
+            self.intensity_record = torch.empty((n, 27), dtype=torch.int32, device=dev)
+            self.intensity_ws = torch.empty((max(1, ops.augment_intensity_workspace_bytes(n, c, d, h, w)),),
+                                            dtype=torch.uint8, device=dev)
         self.extra_state = [self.state, self.pack_status]
 
     def _prepare(self, model):
@@ -733,6 +738,10 @@ class _EpochPlan(_TrainPlan):
                                      out=(self.image, self.mask, self.record))
         else:
             ops.augment_batch(*args, out=(self.image, self.mask, self.record))
+        if a.intensity:
+            ops.augment_intensity_batch(self.image, self.state, self.n, a.bias_prob, a.bias_coefficient, a.gamma_prob,
+                                        a.gamma_log_range, a.noise_prob, a.noise_std,
+                                        out_record=self.intensity_record, workspace=self.intensity_ws)
         boxes, labels, meta = ops.gt_boxes_padded(self.mask, ds.n_classes, self.per_volume, out=self.gt_out,
                                                   workspace=self.gt_ws)
         ops.gt_pack(boxes, labels, meta, self.per_volume, out=(self.gt_boxes, self.gt_labels, self.offsets),
